@@ -23,6 +23,8 @@
 // memory and the rest comes from L2 with per-thread loads; above that every warp streams its own contiguous segment
 // through a private ring of bulk copies (the TMA engine runs ahead of the arithmetic; each pass arms the next pass's
 // first copies before the grid reduction; the head of an HBM-sized vector is kept in L2 by cache hints).
+// Series passes (STANDARD): once rho dominates max e, a pass takes its two sums from power sums of e built once per call
+// (series_sums) and reads no e at all; only the passes before that switch, and the final pass, stream the vector.
 // RLVI_FP_TRACE=1 prints the per-round timeline of a call (profiles/r02_fixed_point_trace.txt).
 #include <math.h>
 #include <stdlib.h>
@@ -35,6 +37,10 @@ constexpr int kFpThreads = 256;
 constexpr int kFpUnroll = 8;            // independent 128-bit loads in flight per thread
 constexpr int kFpCacheSlots = 24;       // whole trips: 24 x 256 x 16 B = 96 KiB of e[] per CTA stay in shared memory (2 CTAs/SM)
 constexpr unsigned long long kSpinTimeoutNs = 20ull * 1000ull * 1000ull * 1000ull;
+// Series passes (STANDARD, VEC): power sums P_j = sum z^j, z = e / 2^E, j = 1..kFpSeriesJ, built once per call.  They
+// travel through the grid reduction as (kFpSeriesJ + 1) / 3 rounds of three values: the power sums and, last, min z.
+constexpr int kFpSeriesJ = 17;
+static_assert(kFpSeriesJ % 3 == 2, "the power sums and min z fill whole reduction rounds");
 
 enum ReduceOp { OP_SUM = 0, OP_MIN = 1, OP_MAX = 2 };
 
@@ -59,6 +65,7 @@ struct FpParams {
   int cache_slots;        // FP64 VEC kernels: chunks per thread kept in shared memory
   int l2_head;            // ring mode: keep the head of the vector L2-resident across passes (cache-hinted bulk copies)
   double pi0;             // initial posterior; 0 = the variant's constant (0.95 / 0.5)
+  int series;             // STANDARD, VEC: allow series passes (RLVI_FP_SERIES=0 forces streaming)
   unsigned long long* trace;   // bring-up only (RLVI_FP_TRACE=1): [round][grid][4] globaltimer stamps, else NULL
 };
 constexpr int kFpTraceRounds = 64;
@@ -464,12 +471,90 @@ __device__ __forceinline__ bool finite_f64(double x) {
   return (((unsigned int)__double2hiint(x) >> 20) & 0x7ffu) != 0x7ffu;
 }
 
+// ---- series passes (STANDARD; DESIGN.md section 4, "Series passes") ------------------------------------------------
+// Once rho dominates max e, both sums of a pass follow from the power sums P_j = sum z^j of z = e / 2^E (2^E = the
+// smallest power of two >= max e, so z is in [0, 1] and the scaling is exact).  With a = 2^E / rho', b = 2^E / rho:
+//   sum pi'   = sum_{k >= 1} (-1)^(k-1) a^k P_k
+//   sum t^2   = (a b / 2^E)^2 sum_{m >= 0} (-1)^m c_m P_{m+2},   c_m = sum_{i=0..m} (i+1)(m-i+1) a^i b^(m-i)
+//             ((-1)^m c_m: the coefficients of 1 / ((1 + a x)^2 (1 + b x)^2))
+// (t = (pi' - pi) / (rho - rho'), as in trip_fast).  The build pass accumulates them next to its ordinary sums.
+__device__ __forceinline__ void trip_powers(const double2 (&v)[kFpUnroll], double zs, double (&P)[kFpSeriesJ], double& zmin) {
+#pragma unroll
+  for (int u = 0; u < kFpUnroll; ++u) {
+    const double za = v[u].x * zs, zb = v[u].y * zs;
+    zmin = fmin(zmin, fmin(za, zb));
+    double pa = za, pb = zb;
+#pragma unroll
+    for (int j = 0; j < kFpSeriesJ; ++j) {
+      P[j] += pa + pb;
+      if (j + 1 < kFpSeriesJ) {
+        pa *= za;
+        pb *= zb;
+      }
+    }
+  }
+}
+
+// The a-priori truncation bounds of both series after kFpSeriesJ power sums, relative to the sums themselves, at
+// q = 2^E / min(rho', rho) >= a, b (derivation: DESIGN.md section 4).  A pass is evaluated from the series only when
+// both are <= 2^-60, i.e. well below the rounding of the direct sums.
+__device__ __forceinline__ bool series_admits(double q) {
+  constexpr int J = kFpSeriesJ;
+  const double r = q * double(J + 3) / double(J);
+  if (!(q > 0.0 && r < 1.0)) return false;           // also rejects NaN
+  double qm = 1.0;                                    // q^(J-1)
+  for (int j = 0; j < J - 1; ++j) qm *= q;
+  const double b1 = qm * q * (1.0 + q) / (1.0 - q);  // sum pi':  q^J (1 + q) / (1 - q)
+  const double q1 = (1.0 + q) * (1.0 + q);
+  const double b2 = q1 * q1 * (double(J + 2) * double(J + 1) * double(J) / 6.0) * qm / (1.0 - r);   // sum t^2
+  constexpr double kTol = 8.673617379884035e-19;     // 2^-60
+  return b1 <= kTol && b2 <= kTol;
+}
+
+// Evaluates both series from the published power sums P (shared memory, P[j] = P_{j+1}) in a fixed order: every
+// thread of every block (of every rank) computes the same bits.  s2 = sum (pi' - pi)^2 as the streamed pass forms it.
+__device__ __forceinline__ void series_sums(const double* P, double two_e, double zs, double rho_new, double rho_old,
+                                            double& s1, double& s2) {
+  constexpr int J = kFpSeriesJ;
+  const double a = two_e / rho_new, b = two_e / rho_old;
+  double h = P[J - 1];
+#pragma unroll
+  for (int j = J - 2; j >= 0; --j) h = fma(-a, h, P[j]);
+  s1 = a * h;
+  // sum_{m=0..J-2} g_m P_{m+2} with g_m = (-1)^m c_m, the coefficients of 1 / D(x), D(x) = (1 + a x)^2 (1 + b x)^2 =
+  // 1 + d1 x + d2 x^2 + d3 x^3 + d4 x^4: g_0 = 1, g_m = -(d1 g_{m-1} + d2 g_{m-2} + d3 g_{m-3} + d4 g_{m-4}).  O(J) and a
+  // short dependency chain, instead of the O(J^2) double sum (a series pass is on the critical path of every block).
+  const double ab = a * b;
+  const double d1 = 2.0 * (a + b), d2 = fma(a, a, fma(b, b, 4.0 * ab)), d3 = 2.0 * ab * (a + b), d4 = ab * ab;
+  double g0 = 1.0, g1 = 0.0, g2 = 0.0, g3 = 0.0, acc = P[1];
+#pragma unroll
+  for (int m = 1; m <= J - 2; ++m) {
+    const double g = -fma(d1, g0, fma(d2, g1, fma(d3, g2, d4 * g3)));
+    g3 = g2;
+    g2 = g1;
+    g1 = g0;
+    g0 = g;
+    acc = fma(g, P[m + 1], acc);
+  }
+  const double w = a * b * zs, drho = rho_old - rho_new;
+  s2 = (drho * drho) * ((w * w) * acc);
+}
+
 // SUM_ONLY (STANDARD): accumulate sum pi' only (s2 comes back 0); the IEEE / remainder paths still form (pi' - pi)^2 but
-// their sum is discarded.
-template <int VARIANT, bool SUM_ONLY>
+// their sum is discarded.  POW (STANDARD): the build pass of the series -- also accumulate this thread's power sums P and
+// min z of z = e zs (trip_powers; zero-filled lanes add nothing).
+template <int VARIANT, bool SUM_ONLY, bool POW = false>
 __device__ __forceinline__ void stream_pass_vec(const double* e, ECache& ec, int64_t n, double rho_new,
-                                                double rho_old, double& s1, double& s2) {
+                                                double rho_old, double& s1, double& s2, double zs = 0.0,
+                                                double* P = nullptr, double* zmin = nullptr) {
   static_assert(!SUM_ONLY || VARIANT == RLVI_FP_STANDARD, "the sum-only pass exists for the STANDARD variant");
+  static_assert(!POW || VARIANT == RLVI_FP_STANDARD, "the series exists for the STANDARD variant");
+  double pw[kFpSeriesJ], zm = 0.0;
+  if (POW) {
+#pragma unroll
+    for (int j = 0; j < kFpSeriesJ; ++j) pw[j] = 0.0;
+    zm = INFINITY;
+  }
   const double2* ev = reinterpret_cast<const double2*>(e);
   const int64_t nvec = n >> 1;
   const int64_t stride = int64_t(gridDim.x) * blockDim.x;
@@ -559,6 +644,7 @@ __device__ __forceinline__ void stream_pass_vec(const double* e, ECache& ec, int
         for (int u = 0; u < kFpUnroll; ++u) v[u] = (u * 32 + lane < rem) ? lds2(src + uint32_t(u) * 512u) : make_double2(0.0, 0.0);
       }
       __syncwarp();                              // every lane has its data: the slot may be re-armed next trip
+      if (POW) trip_powers(v, zs, pw, zm);
       if (SUM_ONLY) trip_sum_only(v, rho_new, s1a, s1b);
       else trip_fast<VARIANT>(v, rho_new, rho_old, s1a, s1b, q2sa, q2sb);
       rd = (rd + 1 == kFpRingDepth) ? 0 : rd + 1;
@@ -600,6 +686,7 @@ __device__ __forceinline__ void stream_pass_vec(const double* e, ECache& ec, int
 #pragma unroll
       for (int u = 0; u < kFpUnroll; ++u) v[u] = ld_e2(ev + c + u * stride);
     }
+    if (POW) trip_powers(v, zs, pw, zm);
     double t1a = 0.0, t1b = 0.0, q2a = 0.0, q2b = 0.0;
     if (SUM_ONLY) trip_sum_only(v, rho_new, t1a, t1b);
     else trip_fast<VARIANT>(v, rho_new, rho_old, t1a, t1b, q2a, q2b);
@@ -633,6 +720,7 @@ __device__ __forceinline__ void stream_pass_vec(const double* e, ECache& ec, int
       const int64_t i = c + u * stride;
       v[u] = (i < nvec) ? ld_e2c(ec, slot0 + u, ev + i) : make_double2(0.0, 0.0);
     }
+    if (POW) trip_powers(v, zs, pw, zm);
     double t1a = 0.0, t1b = 0.0, q2a = 0.0, q2b = 0.0;
     if (SUM_ONLY) trip_sum_only(v, rho_new, t1a, t1b);
     else trip_fast<VARIANT>(v, rho_new, rho_old, t1a, t1b, q2a, q2b);
@@ -662,6 +750,21 @@ __device__ __forceinline__ void stream_pass_vec(const double* e, ECache& ec, int
     post_pair_f64<VARIANT>(e[n - 1], rho_new, rho_old, pn, d);
     s1a += pn;
     s2a = fma(d, d, s2a);
+    if (POW) {
+      const double z = e[n - 1] * zs;
+      double pz = z;
+      zm = fmin(zm, z);
+#pragma unroll
+      for (int j = 0; j < kFpSeriesJ; ++j) {
+        pw[j] += pz;
+        pz *= z;
+      }
+    }
+  }
+  if (POW) {
+#pragma unroll
+    for (int j = 0; j < kFpSeriesJ; ++j) P[j] = pw[j];
+    *zmin = zm;
   }
   s1 = s1a + s1b;
   s2 = SUM_ONLY ? 0.0 : (s2a + s2b) + ((VARIANT == RLVI_FP_STANDARD) ? (drho * drho) * (q2sa + q2sb) : (q2sa + q2sb));
@@ -763,6 +866,34 @@ __device__ __forceinline__ void final_pass_vec(const double* e, const ECache& ec
   if ((n & 1) && blockIdx.x == 0 && threadIdx.x == 0) out[n - 1] = one(e[n - 1]);
 }
 
+// The build pass of the series (STANDARD, VEC): a sum-only streamed pass that also accumulates the
+// power sums, then the pass's own sums reduced as usual, then the power sums and min z in (kFpSeriesJ + 1) / 3 further
+// rounds of the same fixed-order reduction, so every block of every rank holds the same P_j.  They are kept in
+// shared memory (`pw`, block-wide) rather than in registers across the later passes.
+template <int VARIANT>
+__device__ __forceinline__ void build_power_sums(const FpParams<double>& p, FpShared& sh, ECache& ec, const double* e,
+                                              double rho_new, double rho_old, double zs, double* pw,
+                                              double& s1, double& s2, int& pw_state, bool& ok, unsigned int& round) {
+  double P[kFpSeriesJ], zmin = 0.0;
+  stream_pass_vec<VARIANT, true, true>(e, ec, p.n, rho_new, rho_old, s1, s2, zs, P, &zmin);
+  double z = 0.0;
+  ok = grid_allreduce3<double, OP_SUM, false>(p, sh, s1, s2, z, round);
+  bool fin = true;
+#pragma unroll
+  for (int j = 0; j + 2 < kFpSeriesJ; j += 3) {
+    ok = ok && grid_allreduce3<double, OP_SUM, false>(p, sh, P[j], P[j + 1], P[j + 2], round);
+    fin = fin && finite_f64(P[j]) && finite_f64(P[j + 1]) && finite_f64(P[j + 2]);
+  }
+  ok = ok && grid_allreduce3<double, OP_MIN, false>(p, sh, P[kFpSeriesJ - 2], P[kFpSeriesJ - 1], zmin, round);
+  fin = fin && finite_f64(P[kFpSeriesJ - 2]) && finite_f64(P[kFpSeriesJ - 1]);
+  if (threadIdx.x == 0) {
+#pragma unroll
+    for (int j = 0; j < kFpSeriesJ; ++j) pw[j] = P[j];
+  }
+  __syncthreads();
+  pw_state = (fin && zmin >= 0.0) ? 1 : -1;
+}
+
 // =================================================================================================
 // FP64 kernel: STANDARD and ONLINE
 // =================================================================================================
@@ -818,10 +949,23 @@ __global__ void __launch_bounds__(kFpThreads) fp_kernel_f64(const FpParams<doubl
   double bound_prev = 0.0, bound_prev2 = 0.0;
   int k = 1, converged = 0;
   bool ok = true;
+  // series passes: the power sums (block-wide copy), 2^E and 2^-E; pw_state 0 = not built, 1 = usable, -1 = built, unusable
+  constexpr bool kSeries = VEC && VARIANT == RLVI_FP_STANDARD;
+  __shared__ double fp_pw[kFpSeriesJ];
+  double two_e = 0.0, zs = 0.0;
+  int pw_state = 0;
   for (;; ++k) {
     double s1 = 0.0, s2 = 0.0, mx = 0.0;
-    bool sum_only = false;
-    if (k == 1 && VEC && !have_losses) {
+    bool sum_only = false, series = false, build = false;
+    if (kSeries && k >= 2 && pw_state == 1 && series_admits(two_e / fmin(rho_new, rho_old))) {
+      // a series pass: no stream, no grid barrier.  An err within 2^-40 tol of tol is re-taken from the streamed sums,
+      // so a stop decision never rests on the series' rounding.
+      series_sums(fp_pw, two_e, zs, rho_new, rho_old, s1, s2);
+      series = !(fabs(sqrt(s2) - p.tol) <= 0x1p-40 * fabs(p.tol));
+    }
+    if (series) {
+      // s1, s2 came from the series
+    } else if (k == 1 && VEC && !have_losses) {
       first_pass_vec<VARIANT>(e, ec, p.n, rho_new, pi0, s1, s2, mx);
     } else if (k == 1) {
       for_each_chunk<double, VEC>(p.n, [&](int64_t c, int) {
@@ -859,8 +1003,20 @@ __global__ void __launch_bounds__(kFpThreads) fp_kernel_f64(const FpParams<doubl
       // sum-only and whose bound then fails to prove anything is repeated in full, so every decision is the exact one.
       sum_only = (VARIANT == RLVI_FP_STANDARD) && k < p.maxiter && bound_prev2 > 0.0 &&
                  bound_prev * fmin(1.0, bound_prev / bound_prev2) > 2.0 * p.tol;
-      if (sum_only) stream_pass_vec<VARIANT, VARIANT == RLVI_FP_STANDARD>(e, ec, p.n, rho_new, rho_old, s1, s2);
-      else stream_pass_vec<VARIANT, false>(e, ec, p.n, rho_new, rho_old, s1, s2);
+      // Build the power sums (once per call) in a sum-only pass whose last two ratios predict that the series will be
+      // admitted two passes on: rho grows by r = rho' / rho per pass, so q falls to q / r^2.  Data that never nears
+      // the switch (r ~ 1, q >= 1) never builds them.  Only the sum-only trip has the registers to spare for them.
+      if (kSeries && p.series && sum_only && pw_state == 0 && rho_old > 0.0) {
+        const double r = rho_new / rho_old;
+        build = series_admits(two_e / fmin(rho_new, rho_old) / (r * r));
+      }
+      if constexpr (kSeries) {
+        if (build) build_power_sums<VARIANT>(p, sh, ec, e, rho_new, rho_old, zs, fp_pw, s1, s2, pw_state, ok, round);
+      }
+      if (!build) {
+        if (sum_only) stream_pass_vec<VARIANT, VARIANT == RLVI_FP_STANDARD>(e, ec, p.n, rho_new, rho_old, s1, s2);
+        else stream_pass_vec<VARIANT, false>(e, ec, p.n, rho_new, rho_old, s1, s2);
+      }
     } else {
       for_each_chunk<double, VEC>(p.n, [&](int64_t c, int) {
         const int64_t i = c * W;
@@ -883,6 +1039,16 @@ __global__ void __launch_bounds__(kFpThreads) fp_kernel_f64(const FpParams<doubl
       if (ec.ring && have_losses) asm volatile("fence.proxy.async;" ::: "memory");
       ok = grid_allreduce3<double, OP_MAX, true>(p, sh, s1, s2, mx, round);
       emax = mx;
+      if (kSeries && emax > 0x1p-1000 && emax < 0x1p1000) {     // normal and finite: 2^E and 2^-E are exact
+        int ex;
+        const double m = frexp(emax, &ex);                     // emax = m 2^ex, m in [0.5, 1)
+        two_e = (m == 0.5) ? emax : ldexp(1.0, ex);
+        zs = 1.0 / two_e;
+      } else {
+        pw_state = -1;
+      }
+    } else if (series || build) {
+      // the sums are complete (series) or were reduced with the power sums
     } else {
       double z = 0.0;
       ok = grid_allreduce3<double, OP_SUM, false>(p, sh, s1, s2, z, round);
@@ -1399,6 +1565,13 @@ static int fp_cache_slots(int64_t n) {
   return n <= (int64_t(1) << 22) ? kFpCacheSlots : -1;
 }
 
+// Series passes of the STANDARD kernel (on by default; the kernel switches from the data).  RLVI_FP_SERIES=0 streams
+// every pass (A/B comparisons, tests); read per call.
+static int fp_series_enabled() {
+  const char* env = getenv("RLVI_FP_SERIES");
+  return (env && *env && atoi(env) == 0) ? 0 : 1;
+}
+
 extern "C" int rlvi_fixed_point_f64(rlvi_ctx* ctx, int variant, const double* losses, const double* scale,
                                     double* e_work, int64_t n, double tol, int maxiter, double* pi_out,
                                     rlvi_fp_result* result, const rlvi_fp_dist* dist, void* stream) {
@@ -1435,6 +1608,7 @@ static int fixed_point_f64_impl(rlvi_ctx* ctx, int variant, const double* losses
   int rc = fill_dist(p, dist, n);
   if (rc != RLVI_OK) return rc;
   p.pi0 = pi0;
+  p.series = fp_series_enabled();
   const bool vec = rlvi_aligned16(e_work) && rlvi_aligned16(pi_out) && (!losses || rlvi_aligned16(losses));
   const int64_t chunks = vec ? (n + 1) / 2 : n;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
