@@ -286,6 +286,42 @@ int rlvi_wce_fwd_bwd_f32(rlvi_ctx* ctx, const float* logits, const int64_t* labe
 int rlvi_fn_threshold_f32(rlvi_ctx* ctx, float* weights, int64_t n, float alpha, float prev_threshold,
                           int truncate, float* out_threshold, void* stream);
 
+/* ---- batched small problems (many independent fits in one launch) ----------------------------- */
+/* `nprob` problems packed back to back: problem b owns rows [offsets[b], offsets[b+1]) of every per-row array (X [rows][d]
+ * row-major, y, losses, pi_out); `offsets` is a DEVICE int64[nprob + 1].  One warp runs one problem entirely on chip
+ * (per-row vector, d x d statistics and Cholesky factor in shared memory), so a problem's bits depend only on its own rows,
+ * never on its place in the batch or on the batch size.  Every segment is checked on the device: a segment that breaks
+ * 0 <= offsets[b] < offsets[b+1] <= n_rows or is longer than the cap gets NaN outputs and status -1, and none of its rows
+ * is read or written. */
+enum rlvi_batched_model {
+  RLVI_BATCHED_MEAN = 0,   /* standard-learning/rlvi.py:46-65  mean              */
+  RLVI_BATCHED_LINREG = 1  /* standard-learning/rlvi.py:68-89  linear_regression */
+};
+
+/* Rows one problem may have at `d` features (1 <= d <= 64; 0 outside): the shared-memory budget of one warp.  At least
+ * 1024 at every d.  rlvi_batched_fixed_point_f64 admits rlvi_batched_max_rows(1) rows per problem. */
+int rlvi_batched_max_rows(int d);
+
+/* standard-learning/rlvi.py:8-20 update_weights on every segment of `losses` (the RLVI_FP_STANDARD iteration of
+ * rlvi_fixed_point_f64, same operation order): pi_out [n_rows], results [nprob] (a rejected segment: NaN fields,
+ * iters = converged = -1, its pi rows untouched). */
+int rlvi_batched_fixed_point_f64(rlvi_ctx* ctx, const double* losses, const int64_t* offsets, int nprob,
+                                 int64_t n_rows, double tol, int maxiter, double* pi_out,
+                                 rlvi_fp_result* results, void* stream);
+
+/* The whole EM loop of standard-learning/rlvi.py:46-65 (MEAN) or :68-89 (LINREG) per problem, following the drop-in
+ * rlvi_b200/rlvi.py: pi = 1; M-step (MEAN theta = S1/S0, r^2 = ||theta - x||^2; LINREG the normal equations
+ * G theta = b with G = X^T Pi X, b = X^T Pi y by Cholesky, r^2 = (y - x.theta)^2); then up to `maxiter` times the E-step
+ * (the update_weights fixed point, tol 1e-3, maxiter 100, on the losses 0.5 r^2 / sigma2) and the M-step, stopping at
+ * the first theta with ||theta - prev|| / ||prev|| <= tol.  y is NULL for MEAN.  Outputs: theta_out [nprob][d],
+ * iters_out [nprob] (EM iterations), status_out [nprob]: 0 stop test met, 1 maxiter reached, 2 the LINREG Cholesky
+ * failed the drop-in's pivot test (min L_ii^2 / G_ii > 2^-52 (d + sqrt(n)); rank-deficient or ill-conditioned design,
+ * n < d included) at some iteration: theta is NaN and the problem needs the drop-in's minimum-norm solve; -1 rejected
+ * segment.  RLVI_ERR_UNSUPPORTED for d outside 1..64. */
+int rlvi_batched_em_f64(rlvi_ctx* ctx, int model, const double* X, const double* y, const int64_t* offsets, int nprob,
+                        int64_t n_rows, int d, double tol, int maxiter, double* theta_out, int32_t* iters_out,
+                        int32_t* status_out, void* stream);
+
 /* ---- host-buffer convenience (the drop-in's NumPy route; bench.py's `e2e`) ------------------- */
 /* One E+M step of the logistic model on HOST buffers (pinned or pageable): chunks of X/y are copied
  * H2D on a copy stream while the loss kernel consumes the previous chunk; then the fixed point and

@@ -12,13 +12,14 @@ import numpy as np
 import torch
 
 from . import _lib
-from ._lib import (FP_DEEP, FP_ONLINE, FP_STANDARD, LOSS_GAUSSIAN, LOSS_LOGISTIC_CE, LOSS_PCA, LOSS_SOFTPLUS,
-                   LOSS_SQDIST, LOSS_SQRES, TF32X1, TF32X3)
+from ._lib import (BATCHED_LINREG, BATCHED_MEAN, FP_DEEP, FP_ONLINE, FP_STANDARD, LOSS_GAUSSIAN, LOSS_LOGISTIC_CE,
+                   LOSS_PCA, LOSS_SOFTPLUS, LOSS_SQDIST, LOSS_SQRES, TF32X1, TF32X3)
 
 __all__ = ["FP_STANDARD", "FP_ONLINE", "FP_DEEP", "LOSS_LOGISTIC_CE", "LOSS_SOFTPLUS", "LOSS_SQRES",
            "LOSS_SQDIST", "LOSS_PCA", "LOSS_GAUSSIAN", "fixed_point", "fixed_point_deep", "shift_sum", "shift_sum_e", "loss",
            "weighted_moments", "split_moments", "logistic_grad", "wce_fwd_bwd", "fn_threshold", "read_result",
-           "em_step_logistic_host", "launch_count", "TF32X3", "TF32X1", "sigmoid", "online_ce", "irls_weights", "rrm_sum"]
+           "em_step_logistic_host", "launch_count", "TF32X3", "TF32X1", "sigmoid", "online_ce", "irls_weights", "rrm_sum",
+           "BATCHED_MEAN", "BATCHED_LINREG", "batched_max_rows", "batched_fixed_point", "batched_results", "batched_em"]
 
 _RESULT_DTYPE = np.dtype([("eps", "<f8"), ("rho", "<f8"), ("sum_pi", "<f8"), ("err", "<f8"), ("iters", "<i4"),
                           ("converged", "<i4")])
@@ -348,6 +349,98 @@ def rrm_sum(losses, inv_alpha, cutoff=1e-16, *, norm=0.0, w_out=None, out=None):
                                   _p(w_out), _p(out), _stream(dev))
     _lib.check(rc, "rlvi_rrm_sum_f64")
     return out
+
+
+def batched_max_rows(d) -> int:
+    """rlvi_batched_max_rows: rows one problem of a batched call may have at `d` features (0 outside 1..64)."""
+    return int(_lib.load().rlvi_batched_max_rows(int(d)))
+
+
+def _batched_offsets(offsets, rows, cap, ref):
+    """Checks the caller's problem boundaries on the host (the kernels index X, y and pi with them) and uploads them once:
+    offsets[0] == 0, strictly increasing, offsets[-1] == rows, every length <= cap.  Returns (device int64 tensor, nprob)."""
+    if isinstance(offsets, torch.Tensor):
+        if offsets.is_cuda:
+            raise TypeError("offsets must be a host array (they are checked on the host before any launch)")
+        offsets = offsets.numpy()
+    off = np.asarray(offsets)
+    if off.ndim != 1 or off.size < 2 or not np.issubdtype(off.dtype, np.integer):
+        raise TypeError("offsets must be a 1-D integer array of nprob + 1 row boundaries")
+    off = np.ascontiguousarray(off, dtype=np.int64)
+    lengths = np.diff(off)
+    if off[0] != 0 or off[-1] != rows:
+        raise ValueError(f"offsets must start at 0 and end at the number of rows ({rows}); got {off[0]} .. {off[-1]}")
+    if np.any(lengths <= 0):
+        raise ValueError("offsets must be strictly increasing (every problem needs at least one row)")
+    if int(lengths.max()) > cap:
+        raise ValueError(f"a problem has {int(lengths.max())} rows; batched calls admit at most {cap} at this d")
+    return torch.from_numpy(off).to(ref.device), off.size - 1
+
+
+def batched_fixed_point(losses, offsets, *, tol=1e-3, maxiter=100, out=None, results=None):
+    """rlvi_batched_fixed_point_f64: update_weights (rlvi.py:8-20) on every segment [offsets[b], offsets[b+1]) of `losses`.
+    `offsets` is a host integer array.  Returns (pi, results): `results` is a device float64 [nprob, 5] buffer holding one
+    rlvi_fp_result per problem (`batched_results` decodes it)."""
+    dev = _dev(losses)
+    f64 = torch.float64
+    _chk(losses, f64, "losses")
+    if losses.dim() != 1:
+        raise ValueError("losses must be 1-D (the problems packed back to back)")
+    n = losses.numel()
+    ctx = _ctx(dev)
+    offs, nprob = _batched_offsets(offsets, n, ctx.lib.rlvi_batched_max_rows(1), losses)
+    if out is None:
+        out = torch.empty(n, dtype=f64, device=losses.device)
+    _len(_chk(out, f64, "out"), n, "out")
+    if results is None:
+        results = torch.empty(nprob, 5, dtype=f64, device=losses.device)
+    _len(_chk(results, f64, "results"), 5 * nprob, "results")
+    _same_device(losses, out, results)
+    rc = ctx.lib.rlvi_batched_fixed_point_f64(ctx.handle, _p(losses), _p(offs), nprob, n, float(tol), int(maxiter),
+                                              _p(out), _p(results), _stream(dev))
+    _lib.check(rc, "rlvi_batched_fixed_point_f64")
+    return out, results
+
+
+def batched_results(results):
+    """The [nprob, 5] device buffer of batched_fixed_point as a NumPy structured array (fields of rlvi_fp_result)."""
+    return results.cpu().numpy().reshape(-1).view(_RESULT_DTYPE).copy()
+
+
+def batched_em(model, X, y, offsets, *, tol=1e-3, maxiter=100):
+    """rlvi_batched_em_f64: the EM loop of rlvi.mean (model BATCHED_MEAN, y None) or rlvi.linear_regression
+    (BATCHED_LINREG) on every segment of the rows of X [rows, d] (and y [rows]).  `offsets` is a host integer array.
+    Returns device tensors (theta [nprob, d] float64, iters [nprob] int32, status [nprob] int32); status 0 = stop test met,
+    1 = maxiter reached, 2 = the normal equations failed the pivot test: theta is NaN, solve that problem with
+    rlvi.linear_regression."""
+    dev = _dev(X)
+    f64 = torch.float64
+    _chk(X, f64, "X")
+    if model not in (BATCHED_MEAN, BATCHED_LINREG):
+        raise ValueError("model must be BATCHED_MEAN or BATCHED_LINREG")
+    if X.dim() != 2:
+        raise ValueError("X must be [rows, d]")
+    rows, d = X.shape
+    if not 1 <= d <= 64:
+        raise ValueError(f"batched calls support 1 <= d <= 64 (got d = {d})")
+    if model == BATCHED_MEAN and y is not None:
+        raise ValueError("the mean model takes no y")
+    if model == BATCHED_LINREG:
+        if y is None:
+            raise ValueError("linear regression needs y")
+        _len(_chk(y, f64, "y"), rows, "y")
+    _same_device(X, y)
+    if int(maxiter) < 0:
+        raise ValueError("maxiter must be >= 0")
+    ctx = _ctx(dev)
+    offs, nprob = _batched_offsets(offsets, rows, ctx.lib.rlvi_batched_max_rows(d), X)
+    theta = torch.empty(nprob, d, dtype=f64, device=X.device)
+    iters = torch.empty(nprob, dtype=torch.int32, device=X.device)
+    status = torch.empty(nprob, dtype=torch.int32, device=X.device)
+    rc = ctx.lib.rlvi_batched_em_f64(ctx.handle, int(model), _p(X), _p(y), _p(offs), nprob, rows, d, float(tol),
+                                     int(maxiter), _p(theta), _p(iters), _p(status), _stream(dev))
+    _lib.check(rc, "rlvi_batched_em_f64")
+    return theta, iters, status
 
 
 def sever_pass(X, u, op, scalar, *, a=None, b=None, active=None, out0=None, out1=None, out2=None):
