@@ -5,37 +5,36 @@
 //   standard-learning/rlvi.py:70-71    sqrt(pi)-scaled least squares (power = 1:  G = sum pi_i x_i x_i^T)
 //   standard-learning/utils.py:36-38,103-105                         (power = 1)
 //
-// Formulation.  With s_i = pi_i (power 2) or sqrt(pi_i) (power 1) and z_i = s_i x_i -- the very rows the reference
-// forms -- G = Z^T Z.  The d features are cut into nb = ceil(d/128) blocks.  A GROUP computes one 128 x 256 strip
-// D = Z[A]^T [Z[B0] Z[B0+1]] of G (one M = 128, N = 256 instruction per K step: N = 128 instructions run at half
-// rate because the shared-memory read of A is exposed, measured); row A of the block matrix needs the strips
-// B0 = A, A+2, ..., the last one shifted back to nb-2 when the count is odd (a redundant block instead of a
-// half-rate one): 1 / 2 / 4 / 6 groups for nb = 1 .. 4.  CTA c (persistent, one per SM) serves group c % ngroups on
-// the row tiles c / ngroups, + nslots, + 2 nslots, ... (16 rows each), so the CTAs of the different groups sweep
-// the same rows at about the same time and part of X comes from L2 (42 % of the sectors, ncu).  Keeping them in
-// lockstep with progress counters in global memory (RLVI_TF32_WINDOW=<tiles>) was measured and is OFF: the
-// producer's polling costs more than the extra L2 hits return (2.05 -> 2.5 k clk per tile).
+// Routes.  rlvi_weighted_moments_f32 (at the end of this file) picks exactly one per call, before anything is queued:
+//   d > 512, d % 4 != 0, unaligned X, n >= 2^31 - 16, no tensor-map entry point: X is converted to FP64 chunk by chunk
+//               and handed to rlvi_weighted_moments_f64;
+//   d = 129..512  CTA pairs, cta_group::2 (gram_tf32_pair.cu);
+//   d <= 128      the single-CTA kernel below.
 //
-// Per CTA, warp-specialised (16 warps = 4 warpgroups with their own register budgets, setmaxnreg 40/88/192/192):
-//   warp 0      TMA producer: per tile and loaded feature block ONE cp.async.bulk.tensor.3d box (32 floats x 16 rows
-//               x 4 column groups; four 2-D boxes when d % 32 != 0), CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B -> exactly
-//               the one canonical MN-major layout tcgen05 accepts for 32-bit operands, SWIZZLE_128B_BASE32B
-//               (Swizzle<2,5,2>: atoms of 128 B x 4 rows, the 32-byte unit index XORed with row mod 4), LBO = 2048 B
-//               (next 32 features), SBO = 512 B (next 4 rows).  The plain SWIZZLE_128B / no-swizzle MN-major layouts
-//               silently give zeros for kind::tf32 (tools/tf32_debug.cu, profiles/r02_tf32_descriptor_probe.txt);
+// Formulation.  With s_i = pi_i (power 2) or sqrt(pi_i) (power 1) and z_i = s_i x_i -- the very rows the reference
+// forms -- G = Z^T Z.  For d <= 128 the features are ONE 128-feature block (zero-filled past d by the TMA), so G is one
+// M = 128, N = 128 product whose A and B are the same shared-memory block.  CTA c (persistent, one per SM) takes the
+// row tiles c, c + nslots, c + 2 nslots, ... (16 rows each).
+//
+// Per CTA, warp-specialised (16 warps = 4 warpgroups with their own register budgets, setmaxnreg 40/88/192/88):
+//   warp 0      TMA producer: per tile ONE cp.async.bulk.tensor.3d box (32 floats x 16 rows x 4 column groups; four 2-D
+//               boxes when d % 32 != 0), CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B -> exactly the one canonical MN-major
+//               layout tcgen05 accepts for 32-bit operands, SWIZZLE_128B_BASE32B (Swizzle<2,5,2>: atoms of 128 B x 4
+//               rows, the 32-byte unit index XORed with row mod 4), LBO = 2048 B (next 32 features), SBO = 512 B (next
+//               4 rows).  The plain SWIZZLE_128B / no-swizzle MN-major layouts silently give zeros for kind::tf32
+//               (tools/tf32_debug.cu, profiles/r02_tf32_descriptor_probe.txt);
 //   warps 4-15  three transform TEAMS of four warps; team t takes the CTA's tiles t, t + 3, ... (CUDA cores, in
 //               place on the landed tile): z = s_i x rounded to TF32 (round-to-nearest on the bit pattern) = Z_hi,
 //               and for the 3xTF32 mode the remainder Z_lo = tf32(z - Z_hi) into a second buffer; the column
 //               sums S1 = X^T pi, Sy = X^T (w y), S0, sum w y ride along; fence.proxy.async, mbarrier arrive;
-//   warp 1      MMA issuer (one thread): D += Z_hi[A]^T Z_hi[B] (+ Z_lo[A]^T Z_hi[B] + Z_hi[A]^T Z_lo[B]), K = 8
-//               per instruction, both operands MN-major straight from shared memory; tcgen05.commit frees the
-//               stage / publishes the chunk;
-//   warps 8-15  (teams 1 and 2) are also the accumulators: the tensor core adds in FP32 (round-toward-zero inside
-//               the datapath), so a TMEM accumulator only lives for 8 tiles (128 rows); it is then read back
-//               (tcgen05.ld 32x32b) and added, round-to-nearest, into 128 FP32 registers per thread, which are
-//               themselves flushed into this CTA's FP64 partial in global memory every `chunks_per_flush` chunks.
-//               Two TMEM buffers (2 x 256 columns) alternate so the read-back overlaps the next chunk's MMAs; a
-//               team drains chunk c - 2 just before it transforms its first tile of chunk c (complete by then).
+//   warp 1      MMA issuer (one thread): D += Z_hi^T Z_hi (+ Z_lo^T Z_hi + Z_hi^T Z_lo), K = 8 per instruction, both
+//               operands MN-major straight from shared memory; tcgen05.commit frees the stage / publishes the chunk;
+//   warps 8-11  (team 1) are also the accumulator: the tensor core adds in FP32 (round-toward-zero inside the
+//               datapath), so a TMEM accumulator only lives for 8 tiles (128 rows); it is then read back (tcgen05.ld
+//               32x32b) and added, round-to-nearest, into 128 FP32 registers per thread, which are themselves flushed
+//               into this CTA's FP64 partial in global memory every `chunks_per_flush` chunks.  Two TMEM buffers
+//               (2 x 128 columns) alternate so the read-back overlaps the next chunk's MMAs; team 1 drains chunk c - 2
+//               just before it transforms its first tile of chunk c (complete by then).
 // A finalize kernel adds the per-CTA partials in slot order (deterministic) and mirrors the upper triangle.
 // The weights are normalised by a power of two (max pi <= 2^e) so that the collapse regime (pi ~ 1e-7 .. 1e-20,
 // SURVEY.md H1) stays inside the FP32 range; the statistics are scaled back exactly.
@@ -43,94 +42,50 @@
 // Accuracy: 3xTF32 keeps ~2^-21 per product, the three-level accumulation keeps the sums at FP32 level over
 // any N -> statistics agree with the FP64 oracle on the same float32 samples to ~1e-6 (tested at 1e-5);
 // single-pass TF32 (precision = RLVI_TF32X1) rounds operands to 11 bits (zero-mean error): ~1e-3/sqrt(rows).
-//
-// Shapes outside the tensor path (d > 512, d % 4 != 0, unaligned X) are converted to FP64 chunk by chunk and
-// handed to rlvi_weighted_moments_f64.
 #include "tf32.cuh"
 
 namespace {
 
 using namespace tf32;
 
-// ---- the strips ------------------------------------------------------------------------------------------------
-__host__ __device__ __forceinline__ int strips_of_row(int a, int nb) { return (nb - a + 1) / 2; }
-__host__ __device__ __forceinline__ int strip_count(int nb) {
-  int c = 0;
-  for (int a = 0; a < nb; ++a) c += strips_of_row(a, nb);
-  return c;
-}
-// first B block of strip j of row a: a + 2j, shifted back to nb - 2 when the strip would stick out (nb >= 2)
-__host__ __device__ __forceinline__ int strip_b0(int a, int j, int nb) {
-  const int b0 = a + 2 * j;
-  return (nb >= 2 && b0 + 1 > nb - 1) ? nb - 2 : b0;
-}
-__host__ __device__ __forceinline__ int group_of(int a, int j, int nb) {
-  int g = 0;
-  for (int r = 0; r < a; ++r) g += strips_of_row(r, nb);
-  return g + j;
-}
+constexpr int kTeams = 3;
+constexpr int kStages = 8;                   // 8 KiB (TF32X1) or 16 KiB (3xTF32: Z_hi + Z_lo) each
+static_assert(kStages * 2 * kBlkBytes <= kSmemBudget, "stages exceed the shared-memory budget");
 
-// What one group works on: A operand block `a`, B operand blocks b0 (and b0 + 1 when nbk == 2); the distinct
-// feature blocks it loads (`fb`, A first unless it is one of the B blocks, B blocks adjacent and ascending) and the
-// operands' slots in that list; `oslot` = slot of the block whose column sums this group owns (first strip of row a).
-struct GroupPlan {
-  int a, b0, nbk;
-  int nfb;
-  int fb[kMaxFb];
-  int ia, ib;
-  int oslot;
+struct CtaParams {
+  Tf32Params b;           // gpart64: [grid][128][128]; spart: [grid][kTeams][2][128] (S1, Sy)
+  int nslots;             // = grid
+  double* s0part;         // [grid][kTeams][2]   S0, Swy
 };
 
-__host__ __device__ inline GroupPlan make_plan(int g, int nb) {
-  GroupPlan pl;
-  int a = 0, j = g;
-  while (j >= strips_of_row(a, nb)) {
-    j -= strips_of_row(a, nb);
-    ++a;
-  }
-  pl.a = a;
-  pl.b0 = strip_b0(a, j, nb);
-  pl.nbk = (nb >= 2) ? 2 : 1;
-  pl.nfb = 0;
-  const bool a_is_b = (a == pl.b0) || (pl.nbk == 2 && a == pl.b0 + 1);
-  if (!a_is_b) pl.fb[pl.nfb++] = a;
-  pl.ib = pl.nfb;
-  pl.fb[pl.nfb++] = pl.b0;
-  if (pl.nbk == 2) pl.fb[pl.nfb++] = pl.b0 + 1;
-  pl.ia = a_is_b ? pl.ib + (a - pl.b0) : 0;
-  for (int k = pl.nfb; k < kMaxFb; ++k) pl.fb[k] = 0;
-  pl.oslot = (j == 0) ? pl.ia : -1;
-  return pl;
-}
-
-// One transform team (four warps): tiles team, team + 3, ... of the CTA.  IS_ACC teams (1, 2) also own the level-2
-// accumulators of B block team - 1 of the strip.  A separate instantiation per register budget (setmaxnreg 88 / 192).
+// One transform team (four warps): tiles team, team + 3, ... of the CTA.  The IS_ACC team (1) also owns the level-2
+// accumulator.  A separate instantiation per register budget (setmaxnreg 88 / 192).
 struct TeamCtx {
   unsigned char* smem;
   uint64_t *full_bar, *ready_bar, *empty_bar, *tfull_bar, *tempty_bar;
   float* red_all;
   double* dred_all;
   uint32_t tmem_base;
-  int stage_bytes, nst, group, slot, team;
+  int slot, team;
   int my_tiles, my_chunks;
 };
 
 template <int NSPLIT, bool HAS_Y, bool IS_ACC>
-__device__ __forceinline__ void team_body(const Tf32Params& p, const TeamCtx& cx, const int nfb, const int oslot,
-                                          const int nbk) {
+__device__ __forceinline__ void team_body(const CtaParams& cp, const TeamCtx& cx) {
+  const Tf32Params& p = cp.b;
+  constexpr int kStageBytes = kBlkBytes * (NSPLIT == 3 ? 2 : 1);
   unsigned char* smem = cx.smem;
   uint64_t *full_bar = cx.full_bar, *ready_bar = cx.ready_bar, *tfull_bar = cx.tfull_bar, *tempty_bar = cx.tempty_bar;
   uint64_t* empty_bar = cx.empty_bar;
   const uint32_t tmem_base = cx.tmem_base;
-  const int stage_bytes = cx.stage_bytes, nst = cx.nst, group = cx.group, slot = cx.slot, team = cx.team;
+  const int slot = cx.slot, team = cx.team;
   const int my_tiles = cx.my_tiles, my_chunks = cx.my_chunks;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int tt = threadIdx.x & 127;                      // thread of the team
   const int q = tt & 7, rr = tt >> 3;                    // logical 16-byte unit, row of the tile
   // SWIZZLE_128B_ATOM_32B: the 32-byte unit q >> 1 of row rr sits at unit (q >> 1) ^ (rr & 3)
   const uint32_t off = uint32_t(rr * 128 + (((((q >> 1) ^ (rr & 3)) << 1) | (q & 1)) << 4));
-  const uint32_t lo_off = uint32_t(nfb * kBlkBytes);
-  const bool own_s0 = (group == 0) && (q == 0);
+  const bool own_s0 = (q == 0);
   float* red = cx.red_all + team * 1024;
   double* dred = cx.dred_all + team * 32;
   const int bar_id = 1 + team;
@@ -142,32 +97,28 @@ __device__ __forceinline__ void team_body(const Tf32Params& p, const TeamCtx& cx
   double s1d = 0.0, syd = 0.0, s0 = 0.0, swy = 0.0;
   const double wscale = ldexp(1.0, -weight_exponent(p.wmax));      // exact power of two
 
-  // ---- accumulator state (teams 1, 2: B block h = team - 1 of the strip; thread = TMEM lane quarter * 32 + lane) ----
-  const int h = team - 1;
+  // ---- accumulator state (team 1 only; thread = TMEM lane quarter * 32 + lane) ----
   const int quarter = warp & 3;                          // hardware: a warp reaches TMEM lanes 32 (warp id % 4) ..
-  const bool active = IS_ACC && h < nbk;
-  float acc[IS_ACC ? 128 : 2];
+  float acc[128];
 #pragma unroll
-  for (int i = 0; i < (IS_ACC ? 128 : 2); ++i) acc[i] = 0.f;
-  double* gp = p.gpart64 + ((size_t(blockIdx.x) * 2 + (IS_ACC ? h : 0)) * 128 + size_t(quarter * 32 + lane)) * 128;
+  for (int i = 0; i < 128; ++i) acc[i] = 0.f;
+  double* gp = p.gpart64 + (size_t(blockIdx.x) * 128 + size_t(quarter * 32 + lane)) * 128;
   bool flushed = false;
   int next_drain = 0;
   bool ok = true;
 
   auto flush_acc = [&]() {
-    if (IS_ACC && active) {
 #pragma unroll
-      for (int i = 0; i < (IS_ACC ? 128 : 2); i += 2) {
-        double2 v = make_double2(double(acc[i]), double(acc[i + 1]));
-        if (flushed) {
-          const double2 o = *reinterpret_cast<const double2*>(gp + i);
-          v.x += o.x;
-          v.y += o.y;
-        }
-        *reinterpret_cast<double2*>(gp + i) = v;
-        acc[i] = 0.f;
-        acc[i + 1] = 0.f;
+    for (int i = 0; i < 128; i += 2) {
+      double2 v = make_double2(double(acc[i]), double(acc[i + 1]));
+      if (flushed) {
+        const double2 o = *reinterpret_cast<const double2*>(gp + i);
+        v.x += o.x;
+        v.y += o.y;
       }
+      *reinterpret_cast<double2*>(gp + i) = v;
+      acc[i] = 0.f;
+      acc[i + 1] = 0.f;
     }
     flushed = true;
   };
@@ -175,15 +126,13 @@ __device__ __forceinline__ void team_body(const Tf32Params& p, const TeamCtx& cx
     const int buf = ch & 1;
     if (!wait_or_abort(&tfull_bar[buf], uint32_t(ch >> 1) & 1u, p.err)) return false;
     tc_fence_after();
-    if (IS_ACC && active) {
-      const uint32_t taddr = tmem_base + (uint32_t(quarter * 32) << 16) + uint32_t(buf * 256 + h * 128);
+    const uint32_t taddr = tmem_base + (uint32_t(quarter * 32) << 16) + uint32_t(buf * kMB);
 #pragma unroll
-      for (int c = 0; c < (IS_ACC ? 8 : 0); ++c) {
-        float v[16];
-        tc_ld16(taddr + uint32_t(c * 16), v);
+    for (int c = 0; c < 8; ++c) {
+      float v[16];
+      tc_ld16(taddr + uint32_t(c * 16), v);
 #pragma unroll
-        for (int j = 0; j < 16; ++j) acc[(c * 16 + j) % (IS_ACC ? 128 : 2)] += v[j];
-      }
+      for (int j = 0; j < 16; ++j) acc[c * 16 + j] += v[j];
     }
     tc_fence_before();
     mbar_arrive(&tempty_bar[buf]);
@@ -192,36 +141,32 @@ __device__ __forceinline__ void team_body(const Tf32Params& p, const TeamCtx& cx
   };
 
   auto flush_sums = [&]() {
-    if (oslot >= 0) {
-      const int wq = tt >> 5;
+    const int wq = tt >> 5;
 #pragma unroll
-      for (int c = 0; c < 4; ++c)
+    for (int c = 0; c < 4; ++c)
 #pragma unroll
-        for (int k = 0; k < 4; ++k) {
-          float v = s1acc[c][k];
-          v += __shfl_xor_sync(0xffffffffu, v, 8);
-          v += __shfl_xor_sync(0xffffffffu, v, 16);
-          if (lane < 8) red[(wq * 2 + 0) * 128 + c * 32 + lane * 4 + k] = v;
-          s1acc[c][k] = 0.f;
-          if (HAS_Y) {
-            float u = syacc[c][k];
-            u += __shfl_xor_sync(0xffffffffu, u, 8);
-            u += __shfl_xor_sync(0xffffffffu, u, 16);
-            if (lane < 8) red[(wq * 2 + 1) * 128 + c * 32 + lane * 4 + k] = u;
-            syacc[c][k] = 0.f;
-          }
+      for (int k = 0; k < 4; ++k) {
+        float v = s1acc[c][k];
+        v += __shfl_xor_sync(0xffffffffu, v, 8);
+        v += __shfl_xor_sync(0xffffffffu, v, 16);
+        if (lane < 8) red[(wq * 2 + 0) * 128 + c * 32 + lane * 4 + k] = v;
+        s1acc[c][k] = 0.f;
+        if (HAS_Y) {
+          float u = syacc[c][k];
+          u += __shfl_xor_sync(0xffffffffu, u, 8);
+          u += __shfl_xor_sync(0xffffffffu, u, 16);
+          if (lane < 8) red[(wq * 2 + 1) * 128 + c * 32 + lane * 4 + k] = u;
+          syacc[c][k] = 0.f;
         }
-    }
+      }
     asm volatile("bar.sync %0, 128;" ::"r"(bar_id) : "memory");
-    if (oslot >= 0) {
-      s1d += double((red[0 * 128 + tt] + red[2 * 128 + tt]) + (red[4 * 128 + tt] + red[6 * 128 + tt]));
-      if (HAS_Y) syd += double((red[1 * 128 + tt] + red[3 * 128 + tt]) + (red[5 * 128 + tt] + red[7 * 128 + tt]));
-    }
+    s1d += double((red[0 * 128 + tt] + red[2 * 128 + tt]) + (red[4 * 128 + tt] + red[6 * 128 + tt]));
+    if (HAS_Y) syd += double((red[1 * 128 + tt] + red[3 * 128 + tt]) + (red[5 * 128 + tt] + red[7 * 128 + tt]));
     asm volatile("bar.sync %0, 128;" ::"r"(bar_id) : "memory");
   };
 
   auto load_row = [&](int it, double& pid, double& yd) {
-    const int64_t row = (int64_t(slot) + int64_t(it) * p.nslots) * kR + rr;
+    const int64_t row = (int64_t(slot) + int64_t(it) * cp.nslots) * kR + rr;
     pid = (it < my_tiles && row < p.n) ? p.w[row] : 0.0;
     yd = (HAS_Y && it < my_tiles && row < p.n) ? p.y[row] : 0.0;
   };
@@ -229,19 +174,16 @@ __device__ __forceinline__ void team_body(const Tf32Params& p, const TeamCtx& cx
   double pid, yd;
   load_row(team, pid, yd);
   int done = 0;
-  long long t_full = 0, t_busy = 0, t_drain = 0;
-  int s = team % nst;
-  uint32_t ph = uint32_t(team / nst) & 1u;
+  int s = team;                                          // team < kStages
+  uint32_t ph = 0;
   for (int it = team; it < my_tiles; it += kTeams) {
     double pid_n, yd_n;
     load_row(it + kTeams, pid_n, yd_n);                  // prefetch the row coefficients of the team's next tile
-    const long long k0 = clock64();
-    if (IS_ACC) {                                        // chunk c - 2 is complete by now: drain it before chunk c
+    if constexpr (IS_ACC) {                              // chunk c - 2 is complete by now: drain it before chunk c
       const int ch = it / kTpc;
       while (ok && next_drain + 2 <= ch) ok = drain(next_drain++);
       if (!ok) break;
     }
-    const long long k1 = clock64();
     const double wd = (p.power == 2) ? pid * pid : pid;
     const double pis = pid * wscale;                       // normalised weight, <= 1
     const float sc = (p.power == 2) ? float(pis) : float(sqrt(pis));
@@ -256,39 +198,28 @@ __device__ __forceinline__ void team_body(const Tf32Params& p, const TeamCtx& cx
     // (`empty`, one phase back) implies that phase of `full` is over, so wait for that first.
     ok = wait_or_abort(&empty_bar[s], ph ^ 1u, p.err) && wait_or_abort(&full_bar[s], ph, p.err);
     if (!ok) break;
-    const long long k2 = clock64();
-    t_drain += k1 - k0;
-    t_full += k2 - k1;
-    unsigned char* sb = smem + size_t(s) * stage_bytes;
+    unsigned char* sb = smem + size_t(s) * kStageBytes;
 #pragma unroll
-    for (int i = 0; i < kMaxFb; ++i) {
-      if (i < nfb) {
-        const bool sums = (i == oslot);
-#pragma unroll
-        for (int c = 0; c < 4; ++c) {
-          float4* ptr = reinterpret_cast<float4*>(sb + i * kBlkBytes + c * kChunkBytes + off);
-          const float4 x = *ptr;
-          if (sums) {
-            s1acc[c][0] = fmaf(c1, x.x, s1acc[c][0]);
-            s1acc[c][1] = fmaf(c1, x.y, s1acc[c][1]);
-            s1acc[c][2] = fmaf(c1, x.z, s1acc[c][2]);
-            s1acc[c][3] = fmaf(c1, x.w, s1acc[c][3]);
-            if (HAS_Y) {
-              syacc[c][0] = fmaf(cy, x.x, syacc[c][0]);
-              syacc[c][1] = fmaf(cy, x.y, syacc[c][1]);
-              syacc[c][2] = fmaf(cy, x.z, syacc[c][2]);
-              syacc[c][3] = fmaf(cy, x.w, syacc[c][3]);
-            }
-          }
-          const float z0 = sc * x.x, z1 = sc * x.y, z2 = sc * x.z, z3 = sc * x.w;
-          const uint32_t h0 = to_tf32(z0), h1 = to_tf32(z1), h2 = to_tf32(z2), h3 = to_tf32(z3);
-          *reinterpret_cast<uint4*>(ptr) = make_uint4(h0, h1, h2, h3);
-          if (NSPLIT == 3) {
-            const uint32_t l0 = to_tf32(z0 - __uint_as_float(h0)), l1 = to_tf32(z1 - __uint_as_float(h1)),
-                           l2 = to_tf32(z2 - __uint_as_float(h2)), l3 = to_tf32(z3 - __uint_as_float(h3));
-            *reinterpret_cast<uint4*>(reinterpret_cast<unsigned char*>(ptr) + lo_off) = make_uint4(l0, l1, l2, l3);
-          }
-        }
+    for (int c = 0; c < 4; ++c) {
+      float4* ptr = reinterpret_cast<float4*>(sb + c * kChunkBytes + off);
+      const float4 x = *ptr;
+      s1acc[c][0] = fmaf(c1, x.x, s1acc[c][0]);
+      s1acc[c][1] = fmaf(c1, x.y, s1acc[c][1]);
+      s1acc[c][2] = fmaf(c1, x.z, s1acc[c][2]);
+      s1acc[c][3] = fmaf(c1, x.w, s1acc[c][3]);
+      if (HAS_Y) {
+        syacc[c][0] = fmaf(cy, x.x, syacc[c][0]);
+        syacc[c][1] = fmaf(cy, x.y, syacc[c][1]);
+        syacc[c][2] = fmaf(cy, x.z, syacc[c][2]);
+        syacc[c][3] = fmaf(cy, x.w, syacc[c][3]);
+      }
+      const float z0 = sc * x.x, z1 = sc * x.y, z2 = sc * x.z, z3 = sc * x.w;
+      const uint32_t h0 = to_tf32(z0), h1 = to_tf32(z1), h2 = to_tf32(z2), h3 = to_tf32(z3);
+      *reinterpret_cast<uint4*>(ptr) = make_uint4(h0, h1, h2, h3);
+      if (NSPLIT == 3) {                                   // Z_lo: the block behind Z_hi in the stage
+        const uint32_t l0 = to_tf32(z0 - __uint_as_float(h0)), l1 = to_tf32(z1 - __uint_as_float(h1)),
+                       l2 = to_tf32(z2 - __uint_as_float(h2)), l3 = to_tf32(z3 - __uint_as_float(h3));
+        *reinterpret_cast<uint4*>(reinterpret_cast<unsigned char*>(ptr) + kBlkBytes) = make_uint4(l0, l1, l2, l3);
       }
     }
     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // generic writes -> visible to the tensor core
@@ -296,40 +227,31 @@ __device__ __forceinline__ void team_body(const Tf32Params& p, const TeamCtx& cx
     if ((++done % kFlushTiles) == 0) flush_sums();
     pid = pid_n;
     yd = yd_n;
-    s += kTeams;                                           // nst >= 4 > kTeams: at most one wrap
-    if (s >= nst) {
-      s -= nst;
+    s += kTeams;                                           // kStages > kTeams: at most one wrap
+    if (s >= kStages) {
+      s -= kStages;
       ph ^= 1u;
     }
-    t_busy += clock64() - k2;
-  }
-  if (p.stats && tt == 0 && team < 2) {
-    p.stats[size_t(blockIdx.x) * 8 + (team == 0 ? 1 : 6)] = (team == 0) ? t_full : t_drain;
-    if (team == 0) p.stats[size_t(blockIdx.x) * 8 + 2] = t_busy;
   }
   if (ok) {
     flush_sums();
-    if (oslot >= 0) {
-      p.spart[((size_t(blockIdx.x) * kTeams + team) * 2 + 0) * 128 + tt] = s1d;
-      p.spart[((size_t(blockIdx.x) * kTeams + team) * 2 + 1) * 128 + tt] = syd;
+    p.spart[((size_t(blockIdx.x) * kTeams + team) * 2 + 0) * 128 + tt] = s1d;
+    p.spart[((size_t(blockIdx.x) * kTeams + team) * 2 + 1) * 128 + tt] = syd;
+    if (q == 0) {
+      dred[rr * 2 + 0] = s0;
+      dred[rr * 2 + 1] = swy;
     }
-    if (group == 0) {
-      if (q == 0) {
-        dred[rr * 2 + 0] = s0;
-        dred[rr * 2 + 1] = swy;
+    asm volatile("bar.sync %0, 128;" ::"r"(bar_id) : "memory");
+    if (tt == 0) {
+      double a = 0.0, b = 0.0;
+      for (int r = 0; r < kR; ++r) {
+        a += dred[r * 2 + 0];
+        b += dred[r * 2 + 1];
       }
-      asm volatile("bar.sync %0, 128;" ::"r"(bar_id) : "memory");
-      if (tt == 0) {
-        double a = 0.0, b = 0.0;
-        for (int r = 0; r < kR; ++r) {
-          a += dred[r * 2 + 0];
-          b += dred[r * 2 + 1];
-        }
-        p.s0part[(size_t(blockIdx.x) * kTeams + team) * 2 + 0] = a;
-        p.s0part[(size_t(blockIdx.x) * kTeams + team) * 2 + 1] = b;
-      }
+      cp.s0part[(size_t(blockIdx.x) * kTeams + team) * 2 + 0] = a;
+      cp.s0part[(size_t(blockIdx.x) * kTeams + team) * 2 + 1] = b;
     }
-    if (IS_ACC) {
+    if constexpr (IS_ACC) {
       while (ok && next_drain < my_chunks) ok = drain(next_drain++);
       if (ok) flush_acc();
     }
@@ -338,59 +260,43 @@ __device__ __forceinline__ void team_body(const Tf32Params& p, const TeamCtx& cx
 
 template <int NSPLIT, bool HAS_Y>
 __global__ void __launch_bounds__(kThreads, 1)
-    gram_tf32_kernel(const __grid_constant__ CUtensorMap tmap2, const __grid_constant__ CUtensorMap tmap3, const Tf32Params p) {
+    gram_tf32_kernel(const __grid_constant__ CUtensorMap tmap2, const __grid_constant__ CUtensorMap tmap3, const CtaParams cp) {
+  const Tf32Params& p = cp.b;
+  constexpr int kStageBytes = kBlkBytes * (NSPLIT == 3 ? 2 : 1);
   extern __shared__ unsigned char smem_raw[];
   const uint32_t raw = smem_u32(smem_raw);
   unsigned char* smem = smem_raw + ((1024u - (raw & 1023u)) & 1023u);
   const uint32_t smem_base = smem_u32(smem);
   unsigned char* tail = smem + kSmemBudget;
-  uint64_t* full_bar = reinterpret_cast<uint64_t*>(tail);          // [kMaxStages] TMA -> transform
-  uint64_t* ready_bar = full_bar + kMaxStages;                      // [kMaxStages] transform -> MMA
-  uint64_t* empty_bar = ready_bar + kMaxStages;                     // [kMaxStages] MMA -> TMA
-  uint64_t* tfull_bar = empty_bar + kMaxStages;                     // [2] MMA -> accumulator warps
-  uint64_t* tempty_bar = tfull_bar + 2;                             // [2] accumulator warps -> MMA
+  uint64_t* full_bar = reinterpret_cast<uint64_t*>(tail);          // [kStages] TMA -> transform
+  uint64_t* ready_bar = full_bar + kStages;                         // [kStages] transform -> MMA
+  uint64_t* empty_bar = ready_bar + kStages;                        // [kStages] MMA -> TMA
+  uint64_t* tfull_bar = empty_bar + kStages;                        // [2] MMA -> accumulator team
+  uint64_t* tempty_bar = tfull_bar + 2;                             // [2] accumulator team -> MMA
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tempty_bar + 2);
   float* red_all = reinterpret_cast<float*>(tail + 512);            // [kTeams][4 warps][2][128] column-sum exchange
   double* dred_all = reinterpret_cast<double*>(tail + 512 + kTeams * 4096);   // [kTeams][16][2] S0 / Swy exchange
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int group = blockIdx.x % p.ngroups, slot = blockIdx.x / p.ngroups;
-  // the plan as scalars: a struct indexed at run time would live in local memory, and every asm("memory")
-  // statement forces its reload (~100 clk per MMA, measured)
-  int nfb, nbk, oslot, fb0, fb1, fb2;
-  uint32_t a_off, b_off;
-  {
-    const GroupPlan pl = make_plan(group, p.nb);
-    nfb = pl.nfb;
-    nbk = pl.nbk;
-    oslot = pl.oslot;
-    fb0 = pl.fb[0];
-    fb1 = pl.fb[1];
-    fb2 = pl.fb[2];
-    a_off = uint32_t(pl.ia * kBlkBytes);
-    b_off = uint32_t(pl.ib * kBlkBytes);
-  }
-  const int stage_bytes = nfb * kBlkBytes * (NSPLIT == 3 ? 2 : 1);
-  int nst = kSmemBudget / stage_bytes;
-  if (nst > kMaxStages) nst = kMaxStages;
+  const int slot = blockIdx.x;
   const int ntiles = int((p.n + kR - 1) / kR);
-  const int my_tiles = (ntiles > slot) ? (ntiles - slot + p.nslots - 1) / p.nslots : 0;
+  const int my_tiles = (ntiles > slot) ? (ntiles - slot + cp.nslots - 1) / cp.nslots : 0;
   const int my_chunks = (my_tiles + kTpc - 1) / kTpc;
 
   if (threadIdx.x == 0) {
-    for (int s = 0; s < kMaxStages; ++s) {
+    for (int s = 0; s < kStages; ++s) {
       mbar_init(&full_bar[s], 1);
       mbar_init(&ready_bar[s], 128);
       mbar_init(&empty_bar[s], 1);
     }
     for (int b = 0; b < 2; ++b) {
       mbar_init(&tfull_bar[b], 1);
-      mbar_init(&tempty_bar[b], 256);
+      mbar_init(&tempty_bar[b], 128);   // team 1
     }
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
-  if (warp == 1) {   // TMEM: all 512 columns (two 256-column accumulator buffers); one CTA per SM
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(512)
+  if (warp == 1) {   // TMEM: two 128-column accumulator buffers
+    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(2 * kMB)
                  : "memory");
     asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
   }
@@ -405,111 +311,66 @@ __global__ void __launch_bounds__(kThreads, 1)
     if (warp == 0 && lane == 0) {
       int s = 0;
       uint32_t ph = 0;
-      long long t_wait = 0;
-      const long long t_begin = clock64();
-      volatile unsigned int* prog = p.progress + size_t(slot) * p.ngroups;
       for (int it = 0; it < my_tiles; ++it) {
-        if (p.window > 0 && (it & 3) == 0 && it >= p.window && p.ngroups > 1) {
-          // L2-sharing hint: do not run more than kWindow tiles ahead of the slowest group of this slot (bounded:
-          // the other CTAs are normally co-resident, but nothing here may depend on it)
-          const long long h0 = clock64();
-          for (;;) {
-            unsigned int m = 0xffffffffu;
-            for (int g = 0; g < p.ngroups; ++g) {
-              const unsigned int v = prog[g];
-              m = v < m ? v : m;
-            }
-            if (m + unsigned(p.window) >= unsigned(it) || clock64() - h0 > 40000) break;
-          }
-        }
-        const long long c0 = clock64();
         if (!wait_or_abort(&empty_bar[s], ph ^ 1u, p.err)) break;
-        t_wait += clock64() - c0;
-        const int row0 = (slot + it * p.nslots) * kR;
-        const uint32_t sb = smem_base + uint32_t(s) * uint32_t(stage_bytes);
-        mbar_arrive_expect_tx(&full_bar[s], uint32_t(nfb * kBlkBytes));
+        const int row0 = (slot + it * cp.nslots) * kR;
+        const uint32_t sb = smem_base + uint32_t(s) * uint32_t(kStageBytes);
+        mbar_arrive_expect_tx(&full_bar[s], uint32_t(kBlkBytes));
+        if (p.box3d) {       // one box: 32 floats x 16 rows x 4 column groups
+          tma_load_3d_f32(sb, &tmap3, 0, row0, 0, &full_bar[s]);
+        } else {
 #pragma unroll
-        for (int i = 0; i < kMaxFb; ++i) {
-          if (i < nfb) {
-            const int fbi = (i == 0) ? fb0 : (i == 1 ? fb1 : fb2);
-            if (p.box3d) {       // one box: 32 floats x 16 rows x 4 column groups
-              tma_load_3d_f32(sb + uint32_t(i * kBlkBytes), &tmap3, 0, row0, fbi * 4, &full_bar[s]);
-            } else {
-#pragma unroll
-              for (int c = 0; c < 4; ++c)
-                tma_load_2d_f32(sb + uint32_t(i * kBlkBytes + c * kChunkBytes), &tmap2, fbi * kMB + c * 32, row0,
-                                &full_bar[s]);
-            }
-          }
+          for (int c = 0; c < 4; ++c) tma_load_2d_f32(sb + uint32_t(c * kChunkBytes), &tmap2, c * 32, row0, &full_bar[s]);
         }
-        if (++s == nst) {
+        if (++s == kStages) {
           s = 0;
           ph ^= 1u;
         }
       }
-      if (p.stats) {
-        p.stats[size_t(blockIdx.x) * 8 + 0] = t_wait;
-        p.stats[size_t(blockIdx.x) * 8 + 7] = clock64() - t_begin;
-      }
     } else if (warp == 1 && lane == 0) {
-      const uint32_t idesc = umma_idesc(nbk == 2 ? 256 : 128);
-      const uint32_t lo_off = uint32_t(nfb * kBlkBytes);   // Z_lo blocks follow the Z_hi blocks of a stage
+      const uint32_t idesc = umma_idesc(kMB);
       // descriptor = constant | (address >> 4): only the low 14 bits change
       const uint64_t dconst = umma_desc(0);
       auto desc = [&](uint32_t addr) { return dconst | uint64_t((addr & 0x3FFFFu) >> 4); };
-      unsigned int* prog = p.progress + size_t(slot) * p.ngroups + group;
       int s = 0;
       uint32_t ph = 0;
       bool ok = true;
-      long long t_ready = 0, t_tempty = 0, t_issue = 0;
       for (int it = 0; it < my_tiles && ok; ++it) {
         const int ch = it / kTpc;
         const int tin = it - ch * kTpc;
         const int buf = ch & 1;
-        const long long c0 = clock64();
         if (tin == 0) {
           ok = wait_or_abort(&tempty_bar[buf], (uint32_t(ch >> 1) & 1u) ^ 1u, p.err);
           if (!ok) break;
           tc_fence_after();
         }
-        const long long c1 = clock64();
         ok = wait_or_abort(&ready_bar[s], ph, p.err);
         if (!ok) break;
         tc_fence_after();
-        const long long c2 = clock64();
-        t_tempty += c1 - c0;
-        t_ready += c2 - c1;
-        const uint32_t sb = smem_base + uint32_t(s) * uint32_t(stage_bytes);
-        const uint32_t dcol = tmem_base + uint32_t(buf * 256);
+        const uint32_t sb = smem_base + uint32_t(s) * uint32_t(kStageBytes);
+        const uint32_t dcol = tmem_base + uint32_t(buf * kMB);
 #pragma unroll
         for (int ks = 0; ks < kR / 8; ++ks) {
           const uint32_t first = (tin == 0 && ks == 0) ? 0u : 1u;
           const uint32_t kb = sb + uint32_t(ks * 1024);
-          const uint64_t a_hi = desc(kb + a_off), b_hi = desc(kb + b_off);
-          tc_mma_tf32(dcol, a_hi, b_hi, idesc, first);
+          const uint64_t hi = desc(kb);
+          tc_mma_tf32(dcol, hi, hi, idesc, first);
           if (NSPLIT == 3) {
-            tc_mma_tf32(dcol, desc(kb + lo_off + a_off), b_hi, idesc, 1u);
-            tc_mma_tf32(dcol, a_hi, desc(kb + lo_off + b_off), idesc, 1u);
+            const uint64_t lo = desc(kb + kBlkBytes);
+            tc_mma_tf32(dcol, lo, hi, idesc, 1u);
+            tc_mma_tf32(dcol, hi, lo, idesc, 1u);
           }
         }
         tc_commit(&empty_bar[s]);                                        // stage free once these MMAs have read it
         if (tin == kTpc - 1 || it == my_tiles - 1) tc_commit(&tfull_bar[buf]);   // chunk complete in TMEM
-        if ((it & 3) == 3 || it == my_tiles - 1) *reinterpret_cast<volatile unsigned int*>(prog) = unsigned(it + 1);
-        t_issue += clock64() - c2;
-        if (++s == nst) {
+        if (++s == kStages) {
           s = 0;
           ph ^= 1u;
         }
       }
-      if (ok) *reinterpret_cast<volatile unsigned int*>(prog) = 0x7fffffffu;     // done: never hold the others back
-      if (p.stats) {
-        p.stats[size_t(blockIdx.x) * 8 + 3] = t_ready;
-        p.stats[size_t(blockIdx.x) * 8 + 4] = t_tempty;
-        p.stats[size_t(blockIdx.x) * 8 + 5] = t_issue;
-      }
     }
   } else {
-    // ===== warpgroups 1-3: the transform teams; teams 1 and 2 also hold the level-2 accumulators ================
+    // ===== warpgroups 1-3: the transform teams; team 1 also holds the level-2 accumulator =========================
     TeamCtx cx;
     cx.smem = smem;
     cx.full_bar = full_bar;
@@ -520,83 +381,63 @@ __global__ void __launch_bounds__(kThreads, 1)
     cx.red_all = red_all;
     cx.dred_all = dred_all;
     cx.tmem_base = tmem_base;
-    cx.stage_bytes = stage_bytes;
-    cx.nst = nst;
-    cx.group = group;
     cx.slot = slot;
     cx.team = (warp >> 2) - 1;
     cx.my_tiles = my_tiles;
     cx.my_chunks = my_chunks;
-    if (cx.team == 0) {
-      asm volatile("setmaxnreg.dec.sync.aligned.u32 88;");
-      team_body<NSPLIT, HAS_Y, false>(p, cx, nfb, oslot, nbk);
-    } else {
+    if (cx.team == 1) {
       asm volatile("setmaxnreg.inc.sync.aligned.u32 192;");
-      team_body<NSPLIT, HAS_Y, true>(p, cx, nfb, oslot, nbk);
+      team_body<NSPLIT, HAS_Y, true>(cp, cx);
+    } else {
+      asm volatile("setmaxnreg.dec.sync.aligned.u32 88;");
+      team_body<NSPLIT, HAS_Y, false>(cp, cx);
     }
   }
 
   tc_fence_before();
   __syncthreads();
   if (warp == 1) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512) : "memory");
+    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(2 * kMB) : "memory");
   }
 }
 
 // Sum the per-CTA partials in slot order, mirror the upper triangle, write [S0, Swy, S1, Sy, G] (FP64).
-__global__ void __launch_bounds__(256) gram_tf32_finalize_kernel(const Tf32Params p, int has_y, int want_gram, double* out) {
-  const int d = p.d, nb = p.nb;
-  const int npairs = nb * (nb + 1) / 2;
-  const int64_t gtotal = int64_t(npairs) * kMB * kMB;
+__global__ void __launch_bounds__(256) gram_tf32_finalize_kernel(const CtaParams cp, int has_y, int want_gram, double* out) {
+  const Tf32Params& p = cp.b;
+  const int d = p.d;
+  const int64_t gtotal = int64_t(kMB) * kMB;
   const int64_t idx = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
   const bool bad = *p.err != 0u;
   const int wexp = weight_exponent(p.wmax);
   const double up1 = ldexp(1.0, wexp), upw = ldexp(1.0, wexp * p.power);   // undo the weight normalisation
   if (idx < gtotal) {
     if (!want_gram) return;
-    int pidx = int(idx / (kMB * kMB));
-    const int i = int((idx / kMB) % kMB), j = int(idx % kMB);     // G block (a, b), a <= b, element (i, j)
-    int a = 0;
-    while (pidx >= nb - a) {
-      pidx -= nb - a;
-      ++a;
-    }
-    const int b = a + pidx;
-    const int fi = a * kMB + i, fj = b * kMB + j;
-    if (fi >= d || fj >= d) return;
-    if (a == b && i > j) return;
-    // the strip of row a that holds block b: strip js with b0 <= b <= b0 + 1 (the first one that does)
-    int js = (b - a) / 2;
-    if (js >= strips_of_row(a, nb)) js = strips_of_row(a, nb) - 1;
-    const int b0 = strip_b0(a, js, nb);
-    const int g = group_of(a, js, nb), h = b - b0;
+    const int i = int(idx / kMB), j = int(idx % kMB);
+    if (j >= d || i > j) return;                                   // upper triangle, i <= j < d
     double s = 0.0;
-    for (int sl = 0; sl < p.nslots; ++sl)
-      s += p.gpart64[((size_t(sl) * p.ngroups + g) * 2 + h) * (kMB * kMB) + size_t(i) * kMB + j];
+    for (int sl = 0; sl < cp.nslots; ++sl) s += p.gpart64[size_t(sl) * (kMB * kMB) + size_t(i) * kMB + j];
     s *= upw;
     if (bad) s = nan("");
     double* G = out + 2 + 2 * d;
-    G[size_t(fi) * d + fj] = s;
-    G[size_t(fj) * d + fi] = s;
+    G[size_t(i) * d + j] = s;
+    G[size_t(j) * d + i] = s;
     return;
   }
   const int64_t k = idx - gtotal;
-  if (k < 2) {          // S0, Swy: group 0
+  if (k < 2) {          // S0, Swy
     double s = 0.0;
-    for (int sl = 0; sl < p.nslots; ++sl)
-      for (int t = 0; t < kTeams; ++t) s += p.s0part[((size_t(sl) * p.ngroups) * kTeams + t) * 2 + k];
+    for (int sl = 0; sl < cp.nslots; ++sl)
+      for (int t = 0; t < kTeams; ++t) s += cp.s0part[(size_t(sl) * kTeams + t) * 2 + k];
     out[k] = bad ? nan("") : ((k == 1 && !has_y) ? 0.0 : s);
     return;
   }
   const int64_t f2 = k - 2;
   if (f2 < 2 * int64_t(d)) {
     const int which = int(f2 / d), f = int(f2 % d);
-    const int blk = f / kMB, fin = f % kMB;
-    const int g = group_of(blk, 0, nb);
     double s = 0.0;
     if (which == 0 || has_y)
-      for (int sl = 0; sl < p.nslots; ++sl)
-        for (int t = 0; t < kTeams; ++t) s += p.spart[(((size_t(sl) * p.ngroups + g) * kTeams + t) * 2 + which) * 128 + fin];
+      for (int sl = 0; sl < cp.nslots; ++sl)
+        for (int t = 0; t < kTeams; ++t) s += p.spart[((size_t(sl) * kTeams + t) * 2 + which) * 128 + f];
     out[2 + which * d + f] = bad ? nan("") : s * (which == 0 ? up1 : upw);
   }
 }
@@ -619,10 +460,6 @@ __global__ void __launch_bounds__(256) add_f64_kernel(double* __restrict__ dst, 
 }
 
 }  // namespace
-
-size_t rlvi_tf32_pair_scratch_bytes(int sm_count, int64_t n, int power, bool has_y);   // gram_tf32_pair.cu
-int rlvi_tf32_pair_moments(rlvi_ctx* ctx, const CUtensorMap& tmap, const CUtensorMap& tmap3, tf32::Tf32Params p, int precision,
-                           int want_gram, double* out, cudaStream_t st);   // gram_tf32_pair.cu
 
 // Shapes the tensor path does not cover: convert row chunks to FP64 and reuse the FP64 statistics kernels.
 static int moments_f32_via_f64(rlvi_ctx* ctx, const float* X, const double* y, const double* weights, int64_t n, int d,
@@ -676,6 +513,25 @@ extern "C" int rlvi_weighted_moments_f32(rlvi_ctx* ctx, const float* X, const do
   if (!encode || d > 4 * kMB || d % 4 != 0 || n >= (int64_t(1) << 31) - kR || !rlvi_aligned16(X))
     return moments_f32_via_f64(ctx, X, y, weights, n, d, power, want_gram, out, st);
 
+  // The route and its partials (behind the 4 KiB scratch header), decided before anything is queued.  d = 129..512 runs
+  // on CTA pairs when the device can co-schedule one pair per pair type, and otherwise takes the FP64 route; a B200
+  // always can (148 SMs hold up to 74 pairs, at most 3 are needed).
+  const bool pairs = d > kMB;
+  PairPlan plan;
+  CtaParams cp;
+  memset(&cp, 0, sizeof(cp));
+  size_t part_bytes = 0;
+  if (pairs) {
+    const int rc = rlvi_tf32_pair_plan(ctx, n, d, power, y != nullptr, precision, &plan);
+    if (rc != RLVI_OK) return rc;
+    if (plan.first[plan.ntypes] == 0) return moments_f32_via_f64(ctx, X, y, weights, n, d, power, want_gram, out, st);
+    part_bytes = plan.part_bytes;
+  } else {
+    const int64_t ntiles = (n + kR - 1) / kR;
+    cp.nslots = int(ntiles < ctx->sm_count ? ntiles : ctx->sm_count);
+    part_bytes = size_t(cp.nslots) * (size_t(kMB) * kMB + kTeams * 2 * 128 + kTeams * 2) * sizeof(double);
+  }
+
   CUtensorMap tmap, tmap3;
   const cuuint64_t gdim[2] = {cuuint64_t(d), cuuint64_t(n)};
   const cuuint64_t gstride[1] = {cuuint64_t(d) * 4};
@@ -688,8 +544,7 @@ extern "C" int rlvi_weighted_moments_f32(rlvi_ctx* ctx, const float* X, const do
     rlvi_set_error("cuTensorMapEncodeTiled (FP32) failed (%d)", int(cr));
     return RLVI_ERR_CUDA;
   }
-  Tf32Params p;
-  memset(&p, 0, sizeof(p));
+  Tf32Params& p = cp.b;
   // d % 32 == 0: view X as [d/32 column groups][n rows][32 floats] so ONE box (32 x 16 x 4) fetches a whole
   // 128-feature block of a tile (TMA instructions issue at ~60 clk each); column groups past d/32 are zero-filled
   tmap3 = tmap;
@@ -708,64 +563,33 @@ extern "C" int rlvi_weighted_moments_f32(rlvi_ctx* ctx, const float* X, const do
   p.n = n;
   p.d = d;
   p.power = power;
-  p.nb = (d + kMB - 1) / kMB;
-  p.ngroups = strip_count(p.nb);
-  const int64_t ntiles = (n + kR - 1) / kR;
-  int nslots = ctx->sm_count / p.ngroups;
-  if (nslots > ntiles) nslots = int(ntiles);
-  if (nslots < 1) nslots = 1;
-  p.nslots = nslots;
   p.chunks_per_flush = 256;     // 32 Ki rows per register accumulation
-  p.window = kWindow;
-  if (const char* e = getenv("RLVI_TF32_WINDOW")) p.window = atoi(e);
-  const int grid = p.ngroups * p.nslots;
-  const size_t gbytes = size_t(grid) * 2 * kMB * kMB * sizeof(double);
-  const size_t sbytes = size_t(grid) * kTeams * 2 * 128 * sizeof(double);
-  const size_t s0bytes = size_t(grid) * kTeams * 2 * sizeof(double);
-  const size_t pbytes = size_t(grid) * sizeof(unsigned int);
-  // sized for one CTA per SM whichever kernel runs (the pair path lays its own partials out in the same scratch, and
-  // the scratch must not move once the weight-maximum kernel below has been queued)
-  const size_t per_cta = size_t(2) * kMB * kMB * sizeof(double) + size_t(8) * 2 * 128 * sizeof(double) +
-                         size_t(8) * 2 * sizeof(double) + sizeof(unsigned int);      // up to 8 column-sum workers per CTA
-  size_t need = 4096 + gbytes + sbytes + s0bytes + pbytes;
-  if (need < 4096 + per_cta * size_t(ctx->sm_count)) need = 4096 + per_cta * size_t(ctx->sm_count);
-  {
-    const size_t pair_need = rlvi_tf32_pair_scratch_bytes(ctx->sm_count, n, power, y != nullptr);
-    if (p.nb >= 2 && need < pair_need) need = pair_need;
-  }
+
   void* scratch = nullptr;
-  const int rc = rlvi_scratch(ctx, need, &scratch);
+  const int rc = rlvi_scratch(ctx, 4096 + part_bytes, &scratch);
   if (rc != RLVI_OK) return rc;
   char* base = static_cast<char*>(scratch);
+  char* part = base + 4096;
   p.err = reinterpret_cast<unsigned int*>(base + 2048);
-  p.gpart64 = reinterpret_cast<double*>(base + 4096);
-  p.spart = reinterpret_cast<double*>(base + 4096 + gbytes);
-  p.s0part = reinterpret_cast<double*>(base + 4096 + gbytes + sbytes);
-  p.progress = reinterpret_cast<unsigned int*>(base + 4096 + gbytes + sbytes + s0bytes);
-  RLVI_CUDA(cudaMemsetAsync(p.progress, 0, pbytes, st));
-  RLVI_CUDA(cudaMemsetAsync(p.err, 0, 16, st));          // error flag + the weight maximum
   unsigned long long* wmax = reinterpret_cast<unsigned long long*>(base + 2048 + 8);
   p.wmax = wmax;
+  RLVI_CUDA(cudaMemsetAsync(p.err, 0, 16, st));          // error flag + the weight maximum
   {
     int64_t want = (n + 256 * 8 - 1) / (256 * 8);
     const int64_t cap = int64_t(ctx->sm_count) * 8;
     wmax_kernel<<<int(want < 1 ? 1 : (want > cap ? cap : want)), 256, 0, st>>>(weights, n, wmax);
     RLVI_LAUNCH_CHECK(ctx);
   }
+  if (pairs) return rlvi_tf32_pair_moments(ctx, tmap, tmap3, p, plan, part, want_gram, out, st);
 
-  {   // d = 129..512: CTA pairs (gram_tf32_pair.cu); d <= 128, or a device that cannot co-schedule pairs: below
-    const int prc = rlvi_tf32_pair_moments(ctx, tmap, tmap3, p, precision, want_gram, out, st);
-    if (prc != RLVI_ERR_UNSUPPORTED) return prc;
-  }
-  if (getenv("RLVI_TF32_STATS")) {
-    RLVI_CUDA(cudaMalloc(&p.stats, size_t(grid) * 64));
-    RLVI_CUDA(cudaMemset(p.stats, 0, size_t(grid) * 64));
-  }
-
+  const int grid = cp.nslots;
+  p.gpart64 = reinterpret_cast<double*>(part);
+  p.spart = p.gpart64 + size_t(grid) * kMB * kMB;
+  cp.s0part = p.spart + size_t(grid) * kTeams * 2 * 128;
 #define RLVI_TF32_LAUNCH(NS, HY)                                                                                   \
   {                                                                                                                \
     RLVI_CUDA(cudaFuncSetAttribute(gram_tf32_kernel<NS, HY>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemTotal)); \
-    gram_tf32_kernel<NS, HY><<<grid, kThreads, kSmemTotal, st>>>(tmap, tmap3, p);                                         \
+    gram_tf32_kernel<NS, HY><<<grid, kThreads, kSmemTotal, st>>>(tmap, tmap3, cp);                                        \
   }
   if (precision == RLVI_TF32X1) {
     if (y) RLVI_TF32_LAUNCH(1, true) else RLVI_TF32_LAUNCH(1, false)
@@ -774,26 +598,8 @@ extern "C" int rlvi_weighted_moments_f32(rlvi_ctx* ctx, const float* X, const do
   }
 #undef RLVI_TF32_LAUNCH
   RLVI_LAUNCH_CHECK(ctx);
-  if (p.stats) {     // bring-up only: synchronise and print the per-role cycle counters (mean over CTAs)
-    RLVI_CUDA(cudaStreamSynchronize(st));
-    long long* h = static_cast<long long*>(malloc(size_t(grid) * 64));
-    cudaMemcpy(h, p.stats, size_t(grid) * 64, cudaMemcpyDeviceToHost);
-    const char* names[8] = {"producer wait empty", "team0 wait full", "team0 busy", "mma wait ready", "mma wait tempty",
-                            "mma issue", "team1 drain", "producer total"};
-    for (int g = 0; g < p.ngroups; ++g) {
-      double acc[8] = {0, 0, 0, 0, 0, 0, 0, 0};
-      for (int sl = 0; sl < p.nslots; ++sl)
-        for (int k = 0; k < 8; ++k) acc[k] += double(h[(size_t(sl) * p.ngroups + g) * 8 + k]) / p.nslots;
-      const double tiles = double((n + kR - 1) / kR) / p.nslots;
-      fprintf(stderr, "[tf32 stats] group %d (%.0f tiles/CTA), cycles per tile:", g, tiles);
-      for (int k = 0; k < 8; ++k) fprintf(stderr, " %s=%.0f", names[k], acc[k] / tiles);
-      fprintf(stderr, "\n");
-    }
-    free(h);
-    cudaFree(p.stats);
-  }
-  const int64_t total = int64_t(p.nb) * (p.nb + 1) / 2 * kMB * kMB + 2 + 2 * int64_t(d);
-  gram_tf32_finalize_kernel<<<int((total + 255) / 256), 256, 0, st>>>(p, y ? 1 : 0, want_gram, out);
+  const int64_t total = int64_t(kMB) * kMB + 2 + 2 * int64_t(d);
+  gram_tf32_finalize_kernel<<<int((total + 255) / 256), 256, 0, st>>>(cp, y ? 1 : 0, want_gram, out);
   RLVI_LAUNCH_CHECK(ctx);
   return RLVI_OK;
 }

@@ -1,5 +1,6 @@
 // gram_tf32_pair.cu -- the TF32 weighted Gram of FP32-stored samples on CTA PAIRS (tcgen05.mma.cta_group::2, M = 256):
-// the d = 129..256 and d = 385..512 shapes of rlvi_weighted_moments_f32 (config C3: N = 2^24, d = 512).  Same
+// the d = 129..512 shapes of rlvi_weighted_moments_f32 (config C3: N = 2^24, d = 512; d = 257..384 runs as 512 with the
+// fourth 128-feature block zero-filled by the TMA).  Same
 // statistics, same three-level accumulation and the same operand layout as gram_tf32.cu (read its header first);
 // what changes is who computes what:
 //
@@ -42,18 +43,12 @@ namespace {
 using namespace tf32;
 
 constexpr int kPairStages = 12;             // upper bound; the ring uses min(kPairStages, budget / stage bytes)
-constexpr int kPairTypes = 3;
-constexpr int kWorkers = 6;                 // transform warps per CTA: warps 2-7
-#ifndef RLVI_PAIR_WARPS_PER_TILE
-#define RLVI_PAIR_WARPS_PER_TILE 1
-#endif
-constexpr int kWarpsPerTile = RLVI_PAIR_WARPS_PER_TILE;   // 1: a warp transforms a whole 16-row tile; 2: two warps share it (8 rows each)
-constexpr int kTeams = kWorkers / kWarpsPerTile;
+constexpr int kWorkers = 6;                 // transform warps per CTA (warps 2-7), one whole 16-row tile each
 constexpr int kCoefBytes = 256;             // per stage: s, c1, cy of the tile's 16 rows (64 B each)
 constexpr int kCoefThreads = 256;
 
 struct PairParams {
-  Tf32Params b;                 // w, y, n, d, power, chunks_per_flush, box3d, partials, err, wmax, stats
+  Tf32Params b;                 // gpart64: [grid][2][128][128]; spart: [grid][kWorkers][2][128] (diagonal pairs)
   int nbp;                      // 256-feature pair blocks: 1 or 2
   int ntypes;                   // 1 or 3
   int first[kPairTypes + 1];    // first pair of each type; first[ntypes] = number of pairs (grid = 2 x that)
@@ -63,6 +58,7 @@ struct PairParams {
   const float* coef_cy;         // the X^T (w y) coefficient, or null
   double* s0blocks;             // [coef_blocks][2] partial S0 / Swy of the coefficient kernel
   int coef_blocks;
+  long long* stats;             // optional [grid][8] per-role cycle counters (RLVI_TF32_STATS=1)
 };
 
 __host__ __device__ __forceinline__ void pair_type(int t, int nbp, int& pa, int& pb) {
@@ -194,7 +190,8 @@ struct PairCtx {
 // is a chain of dependent shared-memory round trips whose latency triples under load, so what counts is how many
 // tiles are in flight, and a warp needs no barrier but __syncwarp.
 template <int NSPLIT, bool HAS_Y, bool HAS_SUMS>
-__device__ __forceinline__ void pair_transform_warp(const Tf32Params& p, const PairCtx& cx, const int worker) {
+__device__ __forceinline__ void pair_transform_warp(const PairParams& pp, const PairCtx& cx, const int worker) {
+  const Tf32Params& p = pp.b;
   unsigned char* smem = cx.smem;
   uint64_t *full_bar = cx.full_bar, *empty_bar = cx.empty_bar;
   const int stage_bytes = cx.stage_bytes, nst = cx.nst, nfb = cx.nfb, slot = cx.slot;
@@ -262,24 +259,21 @@ __device__ __forceinline__ void pair_transform_warp(const Tf32Params& p, const P
 
   int done = 0;
   long long t_full = 0, t_busy = 0;
-  const int team = worker / kWarpsPerTile, half = worker % kWarpsPerTile;
-  constexpr int kPassesPerWarp = (kR / 4) / kWarpsPerTile;
-  int s = team % nst;
-  uint32_t ph = uint32_t(team / nst) & 1u;
-  for (int it = team; it < my_tiles; it += kTeams) {
-    const long long k1 = p.stats ? clock64() : 0;
+  int s = worker % nst;
+  uint32_t ph = uint32_t(worker / nst) & 1u;
+  for (int it = worker; it < my_tiles; it += kWorkers) {
+    const long long k1 = pp.stats ? clock64() : 0;
     // see gram_tf32.cu: `empty` one phase back first, so that `full` cannot be mistaken for the previous phase
     ok = wait_or_abort(&empty_bar[s], ph ^ 1u, p.err) && wait_or_abort(&full_bar[s], ph, p.err);
     if (!ok) break;
-    const long long k2 = p.stats ? clock64() : 0;
+    const long long k2 = pp.stats ? clock64() : 0;
     t_full += k2 - k1;
     unsigned char* sb = smem + size_t(s) * stage_bytes;
     // the tile's row coefficients arrived with it (FP32, from pair_coef_kernel): no FP64 and no global load in this loop --
     // FP64 instructions issued while the tensor pipe is busy wait for it (stall_math was 47 % of these warps' time)
     const float* cf = reinterpret_cast<const float*>(smem + cx.coef_off + uint32_t(s) * kCoefBytes);
 #pragma unroll
-    for (int pp = 0; pp < kPassesPerWarp; ++pp) {
-      const int pass = half * kPassesPerWarp + pp;
+    for (int pass = 0; pass < kR / 4; ++pass) {
       const int rr = pass * 4 + r4;
       const float sc = cf[rr];
       const float c1 = cx.c1_is_sc ? sc : cf[kR + rr];
@@ -332,16 +326,16 @@ __device__ __forceinline__ void pair_transform_warp(const Tf32Params& p, const P
     __syncwarp();
     if (lane == 0) mbar_arrive_cluster(cx.ready_remote + uint32_t(s) * 8u);   // the leader's barrier: 1 + 1 warps per tile
     if ((++done % kFlushTiles) == 0) flush_sums();
-    s += kTeams;
+    s += kWorkers;
     while (s >= nst) {
       s -= nst;
       ph ^= 1u;
     }
-    if (p.stats) t_busy += clock64() - k2;
+    if (pp.stats) t_busy += clock64() - k2;
   }
-  if (p.stats && lane == 0 && worker == 0) {
-    p.stats[size_t(blockIdx.x) * 8 + 1] = t_full * kTeams;      // scaled to "per tile of the CTA" like the other roles
-    p.stats[size_t(blockIdx.x) * 8 + 2] = t_busy * kTeams;
+  if (pp.stats && lane == 0 && worker == 0) {
+    pp.stats[size_t(blockIdx.x) * 8 + 1] = t_full * kWorkers;   // scaled to "per tile of the CTA" like the other roles
+    pp.stats[size_t(blockIdx.x) * 8 + 2] = t_busy * kWorkers;
   }
   if (ok) {
     flush_sums();
@@ -359,7 +353,8 @@ __device__ __forceinline__ void pair_transform_warp(const Tf32Params& p, const P
 // adds in FP32 with truncation, so a TMEM accumulator only lives for kTpc tiles; it is read back (tcgen05.ld) and
 // added, round-to-nearest, into 128 FP32 registers, themselves flushed into the CTA's FP64 partial every
 // `chunks_per_flush` chunks.  Two TMEM buffers alternate, so chunk c is drained while chunk c + 1 accumulates.
-__device__ __forceinline__ void pair_acc_warp(const Tf32Params& p, const PairCtx& cx) {
+__device__ __forceinline__ void pair_acc_warp(const PairParams& pp, const PairCtx& cx) {
+  const Tf32Params& p = pp.b;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int h = (warp - 8) >> 2, quarter = warp & 3;
   float acc[128];
@@ -390,7 +385,7 @@ __device__ __forceinline__ void pair_acc_warp(const Tf32Params& p, const PairCtx
       ok = false;
       break;
     }
-    const long long k0 = p.stats ? clock64() : 0;
+    const long long k0 = pp.stats ? clock64() : 0;
     tc_fence_after();
     {
       const uint32_t taddr = cx.tmem_base + (uint32_t(quarter * 32) << 16) + uint32_t(buf * 256 + h * 128);
@@ -406,9 +401,9 @@ __device__ __forceinline__ void pair_acc_warp(const Tf32Params& p, const PairCtx
     __syncwarp();
     if (lane == 0) mbar_arrive_cluster(cx.tempty_remote + uint32_t(buf) * 8u);
     if (((ch + 1) % p.chunks_per_flush) == 0) flush_acc();
-    if (p.stats) t_drain += clock64() - k0;
+    if (pp.stats) t_drain += clock64() - k0;
   }
-  if (p.stats && lane == 0 && warp == 8) p.stats[size_t(blockIdx.x) * 8 + 6] = t_drain * kTpc;   // per chunk -> per 8 tiles
+  if (pp.stats && lane == 0 && warp == 8) pp.stats[size_t(blockIdx.x) * 8 + 6] = t_drain * kTpc;   // per chunk -> per 8 tiles
   if (ok) flush_acc();
 }
 
@@ -454,7 +449,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1)
   if (threadIdx.x == 0) {
     for (int s = 0; s < kPairStages; ++s) {
       mbar_init(&full_bar[s], 1);
-      mbar_init(&ready_bar[s], 2 * kWarpsPerTile);      // the tile's transform warp(s) of each CTA
+      mbar_init(&ready_bar[s], 2);      // the tile's transform warp of each CTA
       mbar_init(&empty_bar[s], 1);
     }
     for (int b = 0; b < 2; ++b) {
@@ -503,12 +498,12 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1)
       const long long t_begin = clock64();
       bool ok = true;
       for (int it = 0; it < my_tiles; ++it) {
-        const long long c0 = p.stats ? clock64() : 0;
+        const long long c0 = pp.stats ? clock64() : 0;
         if (!wait_or_abort(&empty_bar[s], ph ^ 1u, p.err)) {
           ok = false;
           break;
         }
-        if (p.stats) t_wait += clock64() - c0;
+        if (pp.stats) t_wait += clock64() - c0;
         const int row0 = (slot + it * nslots) * kR;
         const uint32_t sb = smem_base + uint32_t(s) * uint32_t(stage_bytes);
         const bool c1_sep = (pp.coef_c1 != pp.coef_sc);
@@ -548,9 +543,9 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1)
           ph ^= 1u;
         }
       }
-      if (p.stats) {
-        p.stats[size_t(blockIdx.x) * 8 + 0] = t_wait;
-        p.stats[size_t(blockIdx.x) * 8 + 7] = clock64() - t_begin;
+      if (pp.stats) {
+        pp.stats[size_t(blockIdx.x) * 8 + 0] = t_wait;
+        pp.stats[size_t(blockIdx.x) * 8 + 7] = clock64() - t_begin;
       }
     } else if (warp == 1 && lane == 0 && rank == 0) {
       const uint32_t idesc = umma_idesc_pair(256);
@@ -566,17 +561,17 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1)
         const int ch = it / kTpc;
         const int tin = it - ch * kTpc;
         const int buf = ch & 1;
-        const long long c0 = p.stats ? clock64() : 0;      // (the issuer's loop is on the critical path: no clock reads unless asked)
+        const long long c0 = pp.stats ? clock64() : 0;     // (the issuer's loop is on the critical path: no clock reads unless asked)
         if (tin == 0) {
           ok = wait_or_abort_cluster(&tempty_bar[buf], (uint32_t(ch >> 1) & 1u) ^ 1u, p.err);
           if (!ok) break;
           tc_fence_after();
         }
-        const long long c1 = p.stats ? clock64() : 0;
+        const long long c1 = pp.stats ? clock64() : 0;
         ok = wait_or_abort_cluster(&ready_bar[s], ph, p.err);
         if (!ok) break;
         tc_fence_after();
-        const long long c2 = p.stats ? clock64() : 0;
+        const long long c2 = pp.stats ? clock64() : 0;
         t_tempty += c1 - c0;
         t_ready += c2 - c1;
         const uint32_t sb = smem_base + uint32_t(s) * uint32_t(stage_bytes);
@@ -600,25 +595,25 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1)
         }
         tc2_commit_both(&empty_bar[s]);                                        // stage free in both CTAs
         if (tin == kTpc - 1 || it == my_tiles - 1) tc2_commit_both(&tfull_bar[buf]);   // chunk complete in both TMEMs
-        if (p.stats) t_issue += clock64() - c2;
+        if (pp.stats) t_issue += clock64() - c2;
         if (++s == nst) {
           s = 0;
           ph ^= 1u;
         }
       }
-      if (p.stats) {
-        p.stats[size_t(blockIdx.x) * 8 + 3] = t_ready;
-        p.stats[size_t(blockIdx.x) * 8 + 4] = t_tempty;
-        p.stats[size_t(blockIdx.x) * 8 + 5] = t_issue;
+      if (pp.stats) {
+        pp.stats[size_t(blockIdx.x) * 8 + 3] = t_ready;
+        pp.stats[size_t(blockIdx.x) * 8 + 4] = t_tempty;
+        pp.stats[size_t(blockIdx.x) * 8 + 5] = t_issue;
       }
     } else if (warp >= 2) {
-      if (diag) pair_transform_warp<NSPLIT, HAS_Y, true>(p, cx, warp - 2);
-      else pair_transform_warp<NSPLIT, HAS_Y, false>(p, cx, warp - 2);
+      if (diag) pair_transform_warp<NSPLIT, HAS_Y, true>(pp, cx, warp - 2);
+      else pair_transform_warp<NSPLIT, HAS_Y, false>(pp, cx, warp - 2);
     }
   } else {
     // ===== warpgroups 2, 3: the accumulator warps (TMEM -> FP32 registers -> FP64 partials) ===========================
     asm volatile("setmaxnreg.inc.sync.aligned.u32 160;");
-    pair_acc_warp(p, cx);
+    pair_acc_warp(pp, cx);
   }
 
   tc_fence_before();
@@ -726,39 +721,37 @@ __global__ void __launch_bounds__(256) gram_tf32_pair_finalize_kernel(const Pair
   }
 }
 
-}  // namespace
-
-// Scratch the pair path needs for n rows (partials for one CTA per SM + the FP32 row coefficients): asked for by
-// rlvi_weighted_moments_f32 BEFORE it queues the weight-maximum kernel, because the scratch must not move afterwards.
-size_t rlvi_tf32_pair_scratch_bytes(int sm_count, int64_t n, int power, bool has_y) {
-  const size_t grid = size_t(sm_count);
-  const size_t gbytes = grid * 2 * kMB * kMB * sizeof(double);
-  const size_t sbytes = grid * kWorkers * 2 * 128 * sizeof(double);
-  const int64_t npad = (n + kR - 1) / kR * kR;
-  const int ncoef = 1 + (power == 1 ? 1 : 0) + (has_y ? 1 : 0);
-  const size_t cbytes = (size_t(npad) * 4 + 255) / 256 * 256;
-  const size_t s0bytes = (size_t(sm_count) * 8 * 2 * sizeof(double) + 255) / 256 * 256;
-  return 4096 + gbytes + sbytes + s0bytes + cbytes * size_t(ncoef) + 4096;
+// The partials and row coefficients of a pair grid, in scratch order behind the header.
+struct PairLayout {
+  size_t gbytes, sbytes, s0bytes, cbytes;
+  int ncoef;
+  size_t total() const { return gbytes + sbytes + s0bytes + cbytes * size_t(ncoef); }
+};
+PairLayout pair_layout(int grid, int64_t npad, int coef_blocks, int power, bool has_y) {
+  PairLayout l;
+  l.gbytes = size_t(grid) * 2 * kMB * kMB * sizeof(double);
+  l.sbytes = size_t(grid) * kWorkers * 2 * 128 * sizeof(double);
+  l.s0bytes = (size_t(coef_blocks) * 2 * sizeof(double) + 255) / 256 * 256;
+  l.cbytes = (size_t(npad) * 4 + 255) / 256 * 256;
+  l.ncoef = 1 + (power == 1 ? 1 : 0) + (has_y ? 1 : 0);
+  return l;
 }
 
-// Host side of the pair path.  `p` arrives with w, y, n, d, power, box3d, err, wmax filled in by
-// rlvi_weighted_moments_f32 (which also ran the weight-maximum kernel); returns RLVI_ERR_UNSUPPORTED when the shape or
-// the device does not take pairs (the caller then runs the single-CTA kernel).
-int rlvi_tf32_pair_moments(rlvi_ctx* ctx, const CUtensorMap& tmap, const CUtensorMap& tmap3, tf32::Tf32Params p,
-                           int precision, int want_gram, double* out, cudaStream_t st) {
-  const int nb = (p.d + kMB - 1) / kMB;
-  if (nb < 2 || nb > 4) return RLVI_ERR_UNSUPPORTED;     // d <= 128: the single-CTA kernel
-  if (getenv("RLVI_TF32_NO_PAIR")) return RLVI_ERR_UNSUPPORTED;
-  PairParams pp;
-  memset(&pp, 0, sizeof(pp));
-  pp.nbp = (nb + 1) / 2;                                // d = 257..384: the fourth block is zero-filled by the TMA
-  pp.ntypes = (pp.nbp == 1) ? 1 : 3;
+}  // namespace
+
+// Host-side queries only: which kernel, how many pairs of each type, how much scratch.  The caller guarantees
+// d = 129..512.  first[ntypes] == 0 when the device cannot co-schedule one pair per type.
+int rlvi_tf32_pair_plan(rlvi_ctx* ctx, int64_t n, int d, int power, bool has_y, int precision, PairPlan* plan) {
+  memset(plan, 0, sizeof(*plan));
+  const int nb = (d + kMB - 1) / kMB;
+  const int nbp = (nb + 1) / 2;                         // d = 257..384: the fourth block is zero-filled by the TMA
+  plan->ntypes = (nbp == 1) ? 1 : 3;
 
   // RLVI_TF32X3 = the ~1e-6 mode: TF32 hi.hi + the two correction products.  By default the corrections run as BF16
   // (NSPLIT = 2: a third less tensor time); RLVI_TF32_PURE3=1 keeps all three passes in TF32 (NSPLIT = 3).
   const char* pure_env = getenv("RLVI_TF32_PURE3");      // read per call: tests switch it
-  const int nsplit = (precision == RLVI_TF32X1) ? 1 : ((pure_env && atoi(pure_env) != 0) ? 3 : 2);
-  const int variant = (nsplit == 1 ? 0 : (nsplit == 3 ? 2 : 4)) + (p.y ? 1 : 0);
+  plan->nsplit = (precision == RLVI_TF32X1) ? 1 : ((pure_env && atoi(pure_env) != 0) ? 3 : 2);
+  const int variant = (plan->nsplit == 1 ? 0 : (plan->nsplit == 3 ? 2 : 4)) + (has_y ? 1 : 0);
   const void* fns[6] = {(const void*)gram_tf32_pair_kernel<1, false>, (const void*)gram_tf32_pair_kernel<1, true>,
                         (const void*)gram_tf32_pair_kernel<3, false>, (const void*)gram_tf32_pair_kernel<3, true>,
                         (const void*)gram_tf32_pair_kernel<2, false>, (const void*)gram_tf32_pair_kernel<2, true>};
@@ -791,86 +784,71 @@ int rlvi_tf32_pair_moments(rlvi_ctx* ctx, const CUtensorMap& tmap, const CUtenso
   }
   if (max_pairs > ctx->sm_count / 2) max_pairs = ctx->sm_count / 2;
   if (getenv("RLVI_TF32_STATS")) fprintf(stderr, "[tf32 pair] resident pairs: %d\n", max_pairs);
-  if (const char* e = getenv("RLVI_TF32_PAIRS")) {
-    const int v = atoi(e);
-    if (v > 0 && v < max_pairs) max_pairs = v;
-  }
-  const int64_t ntiles = (p.n + kR - 1) / kR;
-  if (max_pairs < pp.ntypes) return RLVI_ERR_UNSUPPORTED;
+  if (max_pairs < plan->ntypes) return RLVI_OK;
+  const int64_t ntiles = (n + kR - 1) / kR;
 
   // pairs per type: in proportion to the per-tile cost (off-diagonal pairs load and transform two blocks per tile)
   int count[kPairTypes] = {0, 0, 0};
-  if (pp.ntypes == 1) {
+  if (plan->ntypes == 1) {
     count[0] = int(ntiles < max_pairs ? ntiles : max_pairs);
   } else {
     // measured per-tile cost (profiles/r02_tf32_pair_stats.txt): the tensor pipe bounds both kinds of pair alike
     // ... except in the mixed mode, where the stages of an off-diagonal pair are twice as large and half as many, and the
     // pair is bound by the round trip of a stage instead (986 vs 738 clk per tile): 28.2 -> 26.9 ms at config 3 with 1.25
-    double wdiag = 1.0, woff = (nsplit == 2) ? 1.25 : 1.0;
-    if (const char* e = getenv("RLVI_TF32_PAIR_OFFDIAG")) woff = atof(e);
+    const double wdiag = 1.0, woff = (plan->nsplit == 2) ? 1.25 : 1.0;
     int total = max_pairs;
     if (ntiles * 3 < total) total = int(ntiles) * 3;
     int off = int(double(total) * woff / (2.0 * wdiag + woff) + 0.5);
     if (off < 1) off = 1;
     int dg = (total - off) / 2;
     if (dg < 1) dg = 1;
-    off = total - 2 * dg;
-    if (off < 1) return RLVI_ERR_UNSUPPORTED;
+    off = total - 2 * dg;                               // >= 1: total >= 3
     count[0] = dg;
     count[1] = off;
     count[2] = dg;
   }
-  pp.first[0] = 0;
-  for (int t = 0; t < pp.ntypes; ++t) pp.first[t + 1] = pp.first[t] + count[t];
-  for (int t = pp.ntypes; t < kPairTypes; ++t) pp.first[t + 1] = pp.first[pp.ntypes];
-  const int npairs = pp.first[pp.ntypes];
-  const int grid = 2 * npairs;
-
-  p.nb = 2 * pp.nbp;
-  p.ngroups = 0;
-  p.nslots = 0;
-  p.chunks_per_flush = 256;
-  p.window = 0;                 // (single-CTA kernel only)
-  const size_t gbytes = size_t(grid) * 2 * kMB * kMB * sizeof(double);
-  const size_t sbytes = size_t(grid) * kWorkers * 2 * 128 * sizeof(double);
+  for (int t = 0; t < plan->ntypes; ++t) plan->first[t + 1] = plan->first[t] + count[t];
+  for (int t = plan->ntypes; t < kPairTypes; ++t) plan->first[t + 1] = plan->first[plan->ntypes];
   const int64_t npad = ntiles * kR;
-  const int ncoef = 1 + (p.power == 1 ? 1 : 0) + (p.y ? 1 : 0);
-  const size_t cbytes = (size_t(npad) * 4 + 255) / 256 * 256;
-  int coef_blocks = int((npad + kCoefThreads * 4 - 1) / (kCoefThreads * 4));
-  if (coef_blocks > ctx->sm_count * 8) coef_blocks = ctx->sm_count * 8;
-  const size_t s0bytes = (size_t(coef_blocks) * 2 * sizeof(double) + 255) / 256 * 256;
-  void* scratch = nullptr;
-  const int rc = rlvi_scratch(ctx, rlvi_tf32_pair_scratch_bytes(ctx->sm_count, p.n, p.power, p.y != nullptr), &scratch);
-  if (rc != RLVI_OK) return rc;
-  char* base = static_cast<char*>(scratch);
-  if (reinterpret_cast<unsigned int*>(base + 2048) != p.err) {
-    rlvi_set_error("rlvi_tf32_pair_moments: the scratch moved after the weight-maximum kernel was queued");
-    return RLVI_ERR_CUDA;
-  }
-  p.gpart64 = reinterpret_cast<double*>(base + 4096);
-  p.spart = reinterpret_cast<double*>(base + 4096 + gbytes);
-  p.s0part = nullptr;
-  pp.s0blocks = reinterpret_cast<double*>(base + 4096 + gbytes + sbytes);
-  pp.coef_blocks = coef_blocks;
+  plan->coef_blocks = int((npad + kCoefThreads * 4 - 1) / (kCoefThreads * 4));
+  if (plan->coef_blocks > ctx->sm_count * 8) plan->coef_blocks = ctx->sm_count * 8;
+  plan->part_bytes = pair_layout(2 * plan->first[plan->ntypes], npad, plan->coef_blocks, power, has_y).total();
+  return RLVI_OK;
+}
+
+int rlvi_tf32_pair_moments(rlvi_ctx* ctx, const CUtensorMap& tmap, const CUtensorMap& tmap3, const Tf32Params& p,
+                           const PairPlan& plan, char* part, int want_gram, double* out, cudaStream_t st) {
+  PairParams pp;
+  memset(&pp, 0, sizeof(pp));
+  pp.b = p;
+  pp.nbp = (plan.ntypes == 1) ? 1 : 2;
+  pp.ntypes = plan.ntypes;
+  for (int t = 0; t <= kPairTypes; ++t) pp.first[t] = plan.first[t];
+  const int grid = 2 * plan.first[plan.ntypes];
+  const int64_t ntiles = (p.n + kR - 1) / kR;
+  const int64_t npad = ntiles * kR;
+  const PairLayout l = pair_layout(grid, npad, plan.coef_blocks, p.power, p.y != nullptr);
+  pp.b.gpart64 = reinterpret_cast<double*>(part);
+  pp.b.spart = reinterpret_cast<double*>(part + l.gbytes);
+  pp.s0blocks = reinterpret_cast<double*>(part + l.gbytes + l.sbytes);
+  pp.coef_blocks = plan.coef_blocks;
   {
-    float* c0 = reinterpret_cast<float*>(base + 4096 + gbytes + sbytes + s0bytes);
-    float* c1 = (p.power == 1) ? reinterpret_cast<float*>(reinterpret_cast<char*>(c0) + cbytes) : c0;
-    float* c2 = p.y ? reinterpret_cast<float*>(reinterpret_cast<char*>(c0) + cbytes * size_t(ncoef - 1)) : nullptr;
+    float* c0 = reinterpret_cast<float*>(part + l.gbytes + l.sbytes + l.s0bytes);
+    float* c1 = (p.power == 1) ? reinterpret_cast<float*>(reinterpret_cast<char*>(c0) + l.cbytes) : c0;
+    float* c2 = p.y ? reinterpret_cast<float*>(reinterpret_cast<char*>(c0) + l.cbytes * size_t(l.ncoef - 1)) : nullptr;
     pp.coef_sc = c0;
     pp.coef_c1 = c1;
     pp.coef_cy = c2;
-    pair_coef_kernel<<<coef_blocks, kCoefThreads, 0, st>>>(p.w, p.y, p.n, npad, p.power, p.wmax, c0, c1, c2, pp.s0blocks);
+    pair_coef_kernel<<<plan.coef_blocks, kCoefThreads, 0, st>>>(p.w, p.y, p.n, npad, p.power, p.wmax, c0, c1, c2, pp.s0blocks);
     RLVI_LAUNCH_CHECK(ctx);
   }
-  p.progress = nullptr;
-  p.stats = nullptr;
+  const size_t stats_bytes = size_t(grid) * 8 * sizeof(long long);
   if (getenv("RLVI_TF32_STATS")) {
-    RLVI_CUDA(cudaMalloc(&p.stats, size_t(grid) * 128));
-    RLVI_CUDA(cudaMemset(p.stats, 0, size_t(grid) * 128));
+    RLVI_CUDA(cudaMalloc(&pp.stats, stats_bytes));
+    RLVI_CUDA(cudaMemset(pp.stats, 0, stats_bytes));
   }
-  pp.b = p;
 
-  switch (variant) {
+  switch ((plan.nsplit == 1 ? 0 : (plan.nsplit == 3 ? 2 : 4)) + (p.y ? 1 : 0)) {
     case 0: gram_tf32_pair_kernel<1, false><<<grid, kThreads, kSmemTotal, st>>>(tmap, tmap3, pp); break;
     case 1: gram_tf32_pair_kernel<1, true><<<grid, kThreads, kSmemTotal, st>>>(tmap, tmap3, pp); break;
     case 2: gram_tf32_pair_kernel<3, false><<<grid, kThreads, kSmemTotal, st>>>(tmap, tmap3, pp); break;
@@ -879,10 +857,10 @@ int rlvi_tf32_pair_moments(rlvi_ctx* ctx, const CUtensorMap& tmap, const CUtenso
     default: gram_tf32_pair_kernel<2, true><<<grid, kThreads, kSmemTotal, st>>>(tmap, tmap3, pp); break;
   }
   RLVI_LAUNCH_CHECK(ctx);
-  if (p.stats) {     // bring-up only: synchronise and print the per-role cycle counters (mean over the CTAs of a type)
+  if (pp.stats) {    // bring-up only: synchronise and print the per-role cycle counters (mean over the CTAs of a type)
     RLVI_CUDA(cudaStreamSynchronize(st));
-    long long* hst = static_cast<long long*>(malloc(size_t(grid) * 128));
-    cudaMemcpy(hst, p.stats, size_t(grid) * 128, cudaMemcpyDeviceToHost);
+    long long* hst = static_cast<long long*>(malloc(stats_bytes));
+    cudaMemcpy(hst, pp.stats, stats_bytes, cudaMemcpyDeviceToHost);
     const char* names[8] = {"producer wait empty", "worker0 wait full (x6)", "worker0 busy (x6)", "mma wait ready", "mma wait tempty",
                             "mma issue", "acc warp drain (x8)", "producer total"};
     for (int t = 0; t < pp.ntypes; ++t) {
@@ -898,9 +876,11 @@ int rlvi_tf32_pair_moments(rlvi_ctx* ctx, const CUtensorMap& tmap, const CUtenso
       }
     }
     free(hst);
-    cudaFree(p.stats);
+    cudaFree(pp.stats);
+    pp.stats = nullptr;
   }
-  const int64_t total = int64_t(p.nb) * (p.nb + 1) / 2 * kMB * kMB + 2 + 2 * int64_t(p.d);
+  const int nb = 2 * pp.nbp;
+  const int64_t total = int64_t(nb) * (nb + 1) / 2 * kMB * kMB + 2 + 2 * int64_t(p.d);
   gram_tf32_pair_finalize_kernel<<<int((total + 255) / 256), 256, 0, st>>>(pp, p.y ? 1 : 0, want_gram, out);
   RLVI_LAUNCH_CHECK(ctx);
   return RLVI_OK;

@@ -1,5 +1,6 @@
-// tf32.cuh -- shared by the TF32 weighted-Gram kernels (gram_tf32.cu: one CTA per strip; gram_tf32_pair.cu: CTA pairs,
-// cta_group::2): tensor-map encode entry point, tile constants, launch parameters, tcgen05 / TMA PTX wrappers.
+// tf32.cuh -- shared by the TF32 weighted-Gram kernels (gram_tf32.cu: one CTA per SM, d <= 128; gram_tf32_pair.cu: CTA
+// pairs, cta_group::2, d = 129..512): tensor-map encode entry point, tile constants, launch parameters, the cross-file
+// host entry points, tcgen05 / TMA PTX wrappers.
 #pragma once
 
 #include <cuda.h>
@@ -31,37 +32,37 @@ constexpr int kMB = 128;                     // feature block edge = UMMA M
 constexpr int kR = 16;                       // rows per tile (two K = 8 steps)
 constexpr int kChunkBytes = kR * 128;        // 32 floats x 16 rows
 constexpr int kBlkBytes = 4 * kChunkBytes;   // one 128-feature block of one tile: 8 KiB
-constexpr int kMaxStages = 8;
-constexpr int kMaxFb = 3;                    // distinct feature blocks a group can touch
 constexpr int kThreads = 512;
-constexpr int kTeams = 3;
 constexpr int kTpc = 8;                      // tiles per TMEM accumulation (128 rows)
 constexpr int kSmemBudget = 200 * 1024;      // stages
 constexpr int kTailBytes = 16 * 1024;        // barriers, TMEM slot, per-team reduction scratch
 constexpr int kSmemTotal = kSmemBudget + kTailBytes + 1024;   // + alignment slack
 constexpr int kFlushTiles = 16;              // column sums: FP32 per thread for 16 of the team's tiles, then FP64
-constexpr int kWindow = 0;                   // progress-window throttle between the CTAs of one slot: off (see header)
-constexpr int kMaxGroups = 6;
+constexpr int kPairTypes = 3;                // CTA-pair types (0,0), (0,1), (1,1) over 256-feature blocks
 
+// What both routes read.  rlvi_weighted_moments_f32 fills the inputs and the scratch header (err, wmax); each route lays
+// out its own G / column-sum partials behind the header (their shapes are in CtaParams / PairParams).
 struct Tf32Params {
   const double* w;        // pi [n]
   const double* y;        // [n] or null
   int64_t n;
   int d;
   int power;
-  int nb;                 // feature blocks
-  int ngroups;            // strips (1, 2, 4, 6 for nb = 1 .. 4)
-  int nslots;             // CTAs per group; grid = ngroups * nslots
   int chunks_per_flush;   // register (level 2) accumulation length, in chunks
   int box3d;              // 1: one 3-D TMA box per feature block (d % 32 == 0); 0: four 2-D boxes
-  int window;             // > 0: producers of one slot stay within this many tiles of each other (L2-sharing hint)
-  double* gpart64;        // [grid][2][128][128]
-  double* spart;          // [grid][kTeams][2][128]   S1, Sy of the block this group owns
-  double* s0part;         // [grid][kTeams][2]        S0, Swy (group 0 only)
+  double* gpart64;        // per-CTA FP64 partials of G
+  double* spart;          // per-CTA FP64 partials of S1, Sy
   unsigned int* err;      // device flag: a bounded wait expired
   const unsigned long long* wmax;   // bits of max_i pi_i (device): the weights are normalised by a power of two
-  unsigned int* progress; // [nslots][ngroups] tiles committed (L2-sharing hint)
-  long long* stats;       // optional [grid][8] cycle counters (RLVI_TF32_STATS=1; bring-up only)
+};
+
+// The CTA-pair route of one call (gram_tf32_pair.cu), fixed before anything is queued.
+struct PairPlan {
+  int nsplit;                  // 1: TF32X1; 2: TF32X3 with BF16 corrections; 3: TF32X3 in TF32 (RLVI_TF32_PURE3=1)
+  int ntypes;                  // 1 (d <= 256) or 3
+  int first[kPairTypes + 1];   // first pair of each type; first[ntypes] = pairs, 0 when the device cannot hold ntypes
+  int coef_blocks;             // blocks of the row-coefficient kernel
+  size_t part_bytes;           // partials and row coefficients, behind the scratch header
 };
 
 // The even exponent e with max pi <= 2^e (0 when max pi is 0 or not finite): rows are scaled by pi 2^-e so that
@@ -180,3 +181,10 @@ __device__ __forceinline__ bool wait_or_abort(uint64_t* bar, uint32_t parity, un
 }
 
 }  // namespace tf32
+
+// gram_tf32_pair.cu.  rlvi_tf32_pair_plan: host-side queries only (d = 129..512).  rlvi_tf32_pair_moments: queues the
+// route; `p` has the inputs and the scratch header filled in and the weight-maximum kernel queued, `part` is plan.part_bytes
+// of scratch behind the header.
+int rlvi_tf32_pair_plan(rlvi_ctx* ctx, int64_t n, int d, int power, bool has_y, int precision, tf32::PairPlan* plan);
+int rlvi_tf32_pair_moments(rlvi_ctx* ctx, const CUtensorMap& tmap, const CUtensorMap& tmap3, const tf32::Tf32Params& p,
+                           const tf32::PairPlan& plan, char* part, int want_gram, double* out, cudaStream_t st);

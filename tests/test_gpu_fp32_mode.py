@@ -96,12 +96,13 @@ def test_moments_f32_fallback_shapes():
 
 
 def test_moments_f32_single_pass_tf32_is_bounded():
-    rng = np.random.default_rng(9)
-    X = rng.normal(size=(50000, 256)).astype(np.float32)
-    w = rng.random(50000)
-    m1 = gpu_moments(X, w, None, 2, precision=1)
-    r = oracle_moments(X, w, None, 2)
-    assert rel(m1["G"], r["G"]) < 2e-4            # 2^-11 operand rounding, zero-mean: ~1e-3 / sqrt(rows)
+    for d in (256, 128):                          # CTA pairs / the single-CTA kernel
+        rng = np.random.default_rng(9)
+        X = rng.normal(size=(50000, d)).astype(np.float32)
+        w = rng.random(50000)
+        m1 = gpu_moments(X, w, None, 2, precision=1)
+        r = oracle_moments(X, w, None, 2)
+        assert rel(m1["G"], r["G"]) < 2e-4, d     # 2^-11 operand rounding, zero-mean: ~1e-3 / sqrt(rows)
 
 
 @pytest.mark.parametrize("n,d,power,with_y", [(30000, 512, 2, False), (9000, 256, 1, True), (5000, 388, 2, True)])
@@ -131,14 +132,15 @@ def test_moments_f32_correction_modes_agree(n, d, power, with_y, monkeypatch):
 
 
 def test_moments_f32_deterministic_and_linear():
-    rng = np.random.default_rng(11)
-    X = rng.normal(size=(70001, 512)).astype(np.float32)
-    w = rng.random(70001)
-    a = gpu_moments(X, w, None, 1)
-    b = gpu_moments(X, w, None, 1)
-    assert np.array_equal(a["G"], b["G"]) and np.array_equal(a["S1"], b["S1"])
-    c = gpu_moments(X, 4.0 * w, None, 1)                         # exact power-of-two scaling of every product
-    assert rel(c["G"], 4.0 * a["G"]) < 1e-6
+    for d in (512, 128):                                         # CTA pairs / the single-CTA kernel
+        rng = np.random.default_rng(11)
+        X = rng.normal(size=(70001, d)).astype(np.float32)
+        w = rng.random(70001)
+        a = gpu_moments(X, w, None, 1)
+        b = gpu_moments(X, w, None, 1)
+        assert np.array_equal(a["G"], b["G"]) and np.array_equal(a["S1"], b["S1"]), d
+        c = gpu_moments(X, 4.0 * w, None, 1)                     # exact power-of-two scaling of every product
+        assert rel(c["G"], 4.0 * a["G"]) < 1e-6, d
 
 
 def test_moments_f32_large_n_d512_against_oracle():

@@ -26,4 +26,4 @@ for prec, name in ((ops.TF32X3, "x3"), (ops.TF32X1, "x1")):
     b.record()
     torch.cuda.synchronize()
     ms = a.elapsed_time(b) / reps
-    print(f"{name} n=2^{log2n} d={d} {ms:.3f} ms  {n * d * 4 / ms / 1e6:.0f} GB/s  dbg={os.environ.get('RLVI_TF32_PAIR_DEBUG', '0')}", flush=True)
+    print(f"{name} n=2^{log2n} d={d} {ms:.3f} ms  {n * d * 4 / ms / 1e6:.0f} GB/s", flush=True)
