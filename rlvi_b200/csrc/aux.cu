@@ -49,15 +49,7 @@ __global__ void __launch_bounds__(256) rrm_sum_kernel(const double* __restrict__
   }
   double v[1] = {acc};
   block_sum<1>(v, s_red);
-  if (threadIdx.x == 0) partials[blockIdx.x] = v[0];
-  if (last_block_ticket(ticket, gridDim.x)) {
-    if (threadIdx.x < 32) {
-      double a = 0.0;
-      for (unsigned int j = threadIdx.x; j < gridDim.x; j += 32) a += partials[j];
-      a = warp_sum(a);
-      if (threadIdx.x == 0) out_sum[0] = a;
-    }
-  }
+  if (grid_total<1>(v, partials, ticket)) out_sum[0] = v[0];
 }
 
 
@@ -108,12 +100,6 @@ __global__ void __launch_bounds__(256) sever_pass_kernel(const double* __restric
   }
 }
 
-int grid_for(const rlvi_ctx* ctx, int64_t n, int per_thread) {
-  int64_t want = (n + 256 * per_thread - 1) / (256 * per_thread);
-  const int64_t cap = int64_t(ctx->sm_count) * 8;
-  return int(want < 1 ? 1 : (want > cap ? cap : want));
-}
-
 }  // namespace
 
 extern "C" int rlvi_sigmoid_f64(rlvi_ctx* ctx, const double* x, int64_t n, double* out, void* stream) {
@@ -151,12 +137,11 @@ extern "C" int rlvi_rrm_sum_f64(rlvi_ctx* ctx, const double* losses, int64_t n, 
   RLVI_REQUIRE(n > 0, "n must be positive");
   RlviDeviceGuard guard(ctx->device);
   const int grid = grid_for(ctx, n, 4);
-  void* scratch = nullptr;
-  int rc = rlvi_scratch(ctx, 4096 + size_t(grid) * sizeof(double), &scratch);
+  RlviScratch s;
+  const int rc = rlvi_scratch_header(ctx, size_t(grid) * sizeof(double), &s);
   if (rc != RLVI_OK) return rc;
-  rrm_sum_kernel<<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(
-      losses, n, inv_alpha, cutoff, norm, w_out, reinterpret_cast<double*>(static_cast<char*>(scratch) + 4096),
-      reinterpret_cast<unsigned int*>(static_cast<char*>(scratch) + 128), out_sum);
+  rrm_sum_kernel<<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(losses, n, inv_alpha, cutoff, norm, w_out,
+                                                                      s.partials, s.ticket, out_sum);
   RLVI_LAUNCH_CHECK(ctx);
   return RLVI_OK;
 }

@@ -31,6 +31,52 @@ struct rlvi_ctx {
 
 void rlvi_set_error(const char* fmt, ...);
 int rlvi_scratch(rlvi_ctx* ctx, size_t bytes, void** out);   // grows ctx->scratch if needed
+
+// Scratch header: the first kScratchHeaderBytes of ctx->scratch, zero when allocated.  Byte offsets:
+//   [0, 64)       control words.  The fixed point uses [1] as its failure flag; stats_allreduce (dist.cu) uses [0] as
+//                 its ticket and [1] as its failure flag.  Each launcher clears them before its launch.
+//   [128, 132)    the ticket of grid_total.  Left at zero by every kernel that takes it (the last block resets it).
+//   [256, 448)    the fixed point's local LL window when world == 1 (4 slots x 6 LL words), cleared by its launcher.
+//   [2048, 2064)  the TF32 Gram's error flag (u32) and, at 2056, the weight maximum (u64), cleared by its launcher.
+//   [4096, ...)   per-launch partials.
+constexpr size_t kScratchControlBytes = 64;
+constexpr size_t kScratchTicket = 128;
+constexpr size_t kScratchFpWindow = 256;
+constexpr size_t kScratchTf32Err = 2048;
+constexpr size_t kScratchTf32Wmax = 2056;
+constexpr size_t kScratchHeaderBytes = 4096;
+
+struct RlviScratch {
+  unsigned int* control;
+  unsigned int* ticket;
+  double* fp_window;
+  unsigned int* tf32_err;
+  unsigned long long* tf32_wmax;
+  double* partials;
+};
+
+// Scratch for the header plus `partial_bytes` of partials, as typed pointers (valid until the next rlvi_scratch call).
+static inline int rlvi_scratch_header(rlvi_ctx* ctx, size_t partial_bytes, RlviScratch* out) {
+  void* scratch = nullptr;
+  const int rc = rlvi_scratch(ctx, kScratchHeaderBytes + partial_bytes, &scratch);
+  if (rc != RLVI_OK) return rc;
+  char* base = static_cast<char*>(scratch);
+  out->control = reinterpret_cast<unsigned int*>(base);
+  out->ticket = reinterpret_cast<unsigned int*>(base + kScratchTicket);
+  out->fp_window = reinterpret_cast<double*>(base + kScratchFpWindow);
+  out->tf32_err = reinterpret_cast<unsigned int*>(base + kScratchTf32Err);
+  out->tf32_wmax = reinterpret_cast<unsigned long long*>(base + kScratchTf32Wmax);
+  out->partials = reinterpret_cast<double*>(base + kScratchHeaderBytes);
+  return RLVI_OK;
+}
+
+// Grid for a 256-thread grid-stride pass of about `per_thread` elements per thread, capped at 8 CTAs per SM.
+static inline int grid_for(const rlvi_ctx* ctx, int64_t n, int per_thread) {
+  int64_t want = (n + 256 * per_thread - 1) / (256 * per_thread);
+  const int64_t cap = int64_t(ctx->sm_count) * 8;
+  return int(want < 1 ? 1 : (want > cap ? cap : want));
+}
+
 // gram_tma.cu: general-d Gram on the FP64 tensor pipe; RLVI_ERR_UNSUPPORTED = shape not covered (fall back)
 int rlvi_gram_tma_f64(rlvi_ctx* ctx, const double* X, const double* y, const double* weights, const double* center,
                       int64_t n, int d, int power, int want_gram, double* out, cudaStream_t st);
@@ -160,6 +206,29 @@ __device__ __forceinline__ bool last_block_ticket(unsigned int* counter, unsigne
   __syncthreads();
   if (s_last) __threadfence();
   return s_last != 0u;
+}
+
+// Deterministic cross-block sum of NV values, called by every thread of the grid.  Thread 0 holds the block's totals
+// in `v`; they are stored as partials[block][NV].  Returns true in lane 0 of warp 0 of the block that arrives last,
+// with `v` holding the grid totals.  Fixed order: lane j adds partials j, j + 32, ... in increasing order, then the
+// warp_sum xor tree.  `ticket` is the scratch header's ticket.
+template <int NV>
+__device__ __forceinline__ bool grid_total(double (&v)[NV], double* partials, unsigned int* ticket) {
+  if (threadIdx.x == 0) {
+#pragma unroll
+    for (int i = 0; i < NV; ++i) partials[NV * blockIdx.x + i] = v[i];
+  }
+  if (!last_block_ticket(ticket, gridDim.x) || threadIdx.x >= 32) return false;
+  double a[NV];
+#pragma unroll
+  for (int i = 0; i < NV; ++i) a[i] = 0.0;
+  for (unsigned int j = threadIdx.x; j < gridDim.x; j += 32) {
+#pragma unroll
+    for (int i = 0; i < NV; ++i) a[i] += partials[NV * j + i];
+  }
+#pragma unroll
+  for (int i = 0; i < NV; ++i) v[i] = warp_sum(a[i]);
+  return threadIdx.x == 0;
 }
 
 #endif  // __CUDACC__

@@ -77,8 +77,8 @@ extern "C" int rlvi_ctx_destroy(rlvi_ctx* ctx) {
 extern "C" int rlvi_ctx_sm_count(const rlvi_ctx* ctx) { return ctx ? ctx->sm_count : 0; }
 extern "C" int64_t rlvi_ctx_launch_count(const rlvi_ctx* ctx) { return ctx ? ctx->launches : 0; }
 
-// Scratch layout contract: the first 4 KiB are zero-initialised control words (barrier counters,
-// tickets) that every kernel leaves zeroed again; the rest is per-launch partials.
+// New scratch is zeroed.  Its layout (a header of control words, then per-launch partials) and which words must be
+// left at zero are stated once, next to rlvi_scratch_header in common.cuh.
 int rlvi_scratch(rlvi_ctx* ctx, size_t bytes, void** out) {
   if (bytes > ctx->scratch_bytes) {
     // Growing is rare (only for d > 64 shapes); it synchronises the device so that no in-flight

@@ -103,26 +103,18 @@ __global__ void __launch_bounds__(kWceThreads) wce_kernel(const WceParams p) {
       }
     }
   }
-  // block partial of the weighted loss: warps in order
-  if (lane == 0) s_red[warp] = wl_sum;
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    double s = 0.0;
-    for (int w = 0; w < nwarp; ++w) s += s_red[w];
-    p.partials[blockIdx.x] = s;
-  }
   if (p.out_correct && lane == 0 && (top1 | top5)) {
     atomicAdd(p.out_correct, top1);        // integer atomics: order-independent
     atomicAdd(p.out_correct + 1, top5);
   }
-  if (last_block_ticket(p.ticket, gridDim.x)) {
-    if (threadIdx.x < 32) {
-      double a = 0.0;
-      for (unsigned int j = lane; j < gridDim.x; j += 32) a += p.partials[j];
-      a = warp_sum(a);
-      if (lane == 0) p.out_loss[0] = float(a / double(p.batch));   // .mean() (line 94)
-    }
+  // block partial of the weighted loss: warps in order
+  if (lane == 0) s_red[warp] = wl_sum;
+  __syncthreads();
+  double v[1] = {0.0};
+  if (threadIdx.x == 0) {
+    for (int w = 0; w < nwarp; ++w) v[0] += s_red[w];
   }
+  if (grid_total<1>(v, p.partials, p.ticket)) p.out_loss[0] = float(v[0] / double(p.batch));   // .mean() (line 94)
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -281,15 +273,7 @@ __global__ void __launch_bounds__(256) shift_sum_kernel(const double* __restrict
   }
   double v[1] = {acc};
   block_sum<1>(v, s_red);
-  if (threadIdx.x == 0) partials[blockIdx.x] = v[0];
-  if (last_block_ticket(ticket, gridDim.x)) {
-    if (threadIdx.x < 32) {
-      double a = 0.0;
-      for (unsigned int j = threadIdx.x; j < gridDim.x; j += 32) a += partials[j];
-      a = warp_sum(a);
-      if (threadIdx.x == 0) out_sum[0] = a;
-    }
-  }
+  if (grid_total<1>(v, partials, ticket)) out_sum[0] = v[0];
 }
 
 // Same objective from the precomputed e_i = exp(-l_i) the fixed point leaves behind:  t_i = e_i * exp(shift).
@@ -351,15 +335,7 @@ __global__ void __launch_bounds__(256) shift_sum_e_kernel(const double* __restri
   }
   double v[1] = {acc0 + acc1};
   block_sum<1>(v, s_red);
-  if (threadIdx.x == 0) partials[blockIdx.x] = v[0];
-  if (last_block_ticket(ticket, gridDim.x)) {
-    if (threadIdx.x < 32) {
-      double a = 0.0;
-      for (unsigned int j = threadIdx.x; j < gridDim.x; j += 32) a += partials[j];
-      a = warp_sum(a);
-      if (threadIdx.x == 0) out_sum[0] = a;
-    }
-  }
+  if (grid_total<1>(v, partials, ticket)) out_sum[0] = v[0];
 }
 
 }  // namespace
@@ -380,8 +356,8 @@ extern "C" int rlvi_wce_fwd_bwd_f32(rlvi_ctx* ctx, const float* logits, const in
   int64_t want = (batch + nwarp - 1) / nwarp;
   const int64_t cap = int64_t(ctx->sm_count) * 8;
   const int grid = int(want > cap ? cap : want);
-  void* scratch = nullptr;
-  int rc = rlvi_scratch(ctx, 4096 + size_t(grid) * sizeof(double), &scratch);
+  RlviScratch s;
+  const int rc = rlvi_scratch_header(ctx, size_t(grid) * sizeof(double), &s);
   if (rc != RLVI_OK) return rc;
   WceParams p;
   p.logits = logits;
@@ -396,8 +372,8 @@ extern "C" int rlvi_wce_fwd_bwd_f32(rlvi_ctx* ctx, const float* logits, const in
   p.batch = batch;
   p.classes = classes;
   p.n_train = n_train;
-  p.ticket = reinterpret_cast<unsigned int*>(static_cast<char*>(scratch) + 128);
-  p.partials = reinterpret_cast<double*>(static_cast<char*>(scratch) + 4096);
+  p.ticket = s.ticket;
+  p.partials = s.partials;
   if (out_correct) RLVI_CUDA(cudaMemsetAsync(out_correct, 0, 2 * sizeof(int32_t), st));
   if (classes <= 128)
     wce_kernel<4><<<grid, kWceThreads, 0, st>>>(p);
@@ -435,15 +411,12 @@ extern "C" int rlvi_shift_sum_f64(rlvi_ctx* ctx, const double* losses, int64_t n
   RLVI_REQUIRE(ctx && losses && out_sum, "null pointer");
   RLVI_REQUIRE(n > 0, "n must be positive");
   RlviDeviceGuard guard(ctx->device);
-  int64_t want = (n + 256 * 4 - 1) / (256 * 4);
-  const int64_t cap = int64_t(ctx->sm_count) * 8;
-  const int grid = int(want < 1 ? 1 : (want > cap ? cap : want));
-  void* scratch = nullptr;
-  int rc = rlvi_scratch(ctx, 4096 + size_t(grid) * sizeof(double), &scratch);
+  const int grid = grid_for(ctx, n, 4);
+  RlviScratch s;
+  const int rc = rlvi_scratch_header(ctx, size_t(grid) * sizeof(double), &s);
   if (rc != RLVI_OK) return rc;
-  shift_sum_kernel<<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(
-      losses, n, shift, c, pi_out, reinterpret_cast<double*>(static_cast<char*>(scratch) + 4096),
-      reinterpret_cast<unsigned int*>(static_cast<char*>(scratch) + 128), out_sum);
+  shift_sum_kernel<<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(losses, n, shift, c, pi_out, s.partials, s.ticket,
+                                                                        out_sum);
   RLVI_LAUNCH_CHECK(ctx);
   return RLVI_OK;
 }
@@ -454,15 +427,12 @@ extern "C" int rlvi_shift_sum_e_f64(rlvi_ctx* ctx, const double* e, int64_t n, d
   RLVI_REQUIRE(n > 0, "n must be positive");
   RLVI_REQUIRE(scale_t >= 0.0 && scale_t < 1e300, "scale_t = exp(shift) must be finite and non-negative");
   RlviDeviceGuard guard(ctx->device);
-  int64_t want = (n + 256 * 8 - 1) / (256 * 8);
-  const int64_t cap = int64_t(ctx->sm_count) * 8;
-  const int grid = int(want < 1 ? 1 : (want > cap ? cap : want));
-  void* scratch = nullptr;
-  int rc = rlvi_scratch(ctx, 4096 + size_t(grid) * sizeof(double), &scratch);
+  const int grid = grid_for(ctx, n, 8);
+  RlviScratch s;
+  const int rc = rlvi_scratch_header(ctx, size_t(grid) * sizeof(double), &s);
   if (rc != RLVI_OK) return rc;
-  shift_sum_e_kernel<<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(
-      e, n, scale_t, c, pi_out, reinterpret_cast<double*>(static_cast<char*>(scratch) + 4096),
-      reinterpret_cast<unsigned int*>(static_cast<char*>(scratch) + 128), out_sum);
+  shift_sum_e_kernel<<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(e, n, scale_t, c, pi_out, s.partials, s.ticket,
+                                                                          out_sum);
   RLVI_LAUNCH_CHECK(ctx);
   return RLVI_OK;
 }

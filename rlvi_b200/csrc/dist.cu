@@ -159,8 +159,8 @@ extern "C" int rlvi_stats_allreduce_f64(rlvi_ctx* ctx, double* buf, int count, c
   RLVI_REQUIRE(dist->inbox && dist->peer_inbox && dist->call_index > 0, "incomplete rlvi_fp_dist");
   RlviDeviceGuard guard(ctx->device);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  void* scratch = nullptr;
-  int rc = rlvi_scratch(ctx, 4096, &scratch);
+  RlviScratch s;
+  const int rc = rlvi_scratch_header(ctx, 0, &s);
   if (rc != RLVI_OK) return rc;
   StatsParams p;
   p.buf = buf;
@@ -170,8 +170,8 @@ extern "C" int rlvi_stats_allreduce_f64(rlvi_ctx* ctx, double* buf, int count, c
   p.inbox = dist->inbox;
   p.peer_inbox = dist->peer_inbox;
   p.call_index = dist->call_index;
-  p.control = reinterpret_cast<unsigned int*>(scratch);
-  RLVI_CUDA(cudaMemsetAsync(p.control, 0, 64, st));
+  p.control = s.control;
+  RLVI_CUDA(cudaMemsetAsync(p.control, 0, kScratchControlBytes, st));
   const int grid = (count + 255) / 256;     // <= 32 CTAs: always co-resident
   stats_allreduce_kernel<<<grid, 256, 0, st>>>(p);
   RLVI_LAUNCH_CHECK(ctx);

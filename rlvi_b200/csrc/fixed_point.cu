@@ -1449,17 +1449,16 @@ int launch_fp(rlvi_ctx* ctx, K kernel, FpParams<T>& p, int64_t n_chunks, cudaStr
   int64_t max_grid = int64_t(ctx->sm_count) * per_sm;
   int64_t want = (n_chunks + int64_t(kFpThreads) * kFpUnroll - 1) / (int64_t(kFpThreads) * kFpUnroll);
   int grid = int(want < 1 ? 1 : (want > max_grid ? max_grid : want));
-  void* scratch = nullptr;
-  const size_t ctrl = 4096;
+  RlviScratch s;
   const size_t part_bytes = size_t(2) * grid * 6 * sizeof(unsigned long long);   // [2 round parities][grid][3 doubles as LL words]
-  int rc = rlvi_scratch(ctx, ctrl + part_bytes, &scratch);
+  int rc = rlvi_scratch_header(ctx, part_bytes, &s);
   if (rc != RLVI_OK) return rc;
-  p.control = reinterpret_cast<unsigned int*>(scratch);
-  p.partials = reinterpret_cast<double*>(static_cast<char*>(scratch) + ctrl);
-  // [0,64): failure flag; [256, 256 + 192): the local window used when world == 1 (4 slots x 6 LL words); then the block
-  // partials.  All zeroed: LL tags start at 1, so a zeroed (or any earlier call's) word never matches.
-  RLVI_CUDA(cudaMemsetAsync(p.control, 0, ctrl + part_bytes, stream));
-  if (p.world == 1) p.inbox = reinterpret_cast<double*>(static_cast<char*>(scratch) + 256);
+  p.control = s.control;
+  p.partials = s.partials;
+  // The whole header (failure flag, local LL window) and the block partials are zeroed: LL tags start at 1, so a zeroed
+  // (or any earlier call's) word never matches.
+  RLVI_CUDA(cudaMemsetAsync(p.control, 0, kScratchHeaderBytes + part_bytes, stream));
+  if (p.world == 1) p.inbox = s.fp_window;
   p.trace = nullptr;
   static const char* trace_env = getenv("RLVI_FP_TRACE");
   const size_t trace_bytes = size_t(kFpTraceRounds) * grid * 4 * sizeof(unsigned long long);

@@ -565,25 +565,19 @@ extern "C" int rlvi_weighted_moments_f32(rlvi_ctx* ctx, const float* X, const do
   p.power = power;
   p.chunks_per_flush = 256;     // 32 Ki rows per register accumulation
 
-  void* scratch = nullptr;
-  const int rc = rlvi_scratch(ctx, 4096 + part_bytes, &scratch);
+  RlviScratch s;
+  const int rc = rlvi_scratch_header(ctx, part_bytes, &s);
   if (rc != RLVI_OK) return rc;
-  char* base = static_cast<char*>(scratch);
-  char* part = base + 4096;
-  p.err = reinterpret_cast<unsigned int*>(base + 2048);
-  unsigned long long* wmax = reinterpret_cast<unsigned long long*>(base + 2048 + 8);
-  p.wmax = wmax;
+  p.err = s.tf32_err;
+  p.wmax = s.tf32_wmax;
   RLVI_CUDA(cudaMemsetAsync(p.err, 0, 16, st));          // error flag + the weight maximum
-  {
-    int64_t want = (n + 256 * 8 - 1) / (256 * 8);
-    const int64_t cap = int64_t(ctx->sm_count) * 8;
-    wmax_kernel<<<int(want < 1 ? 1 : (want > cap ? cap : want)), 256, 0, st>>>(weights, n, wmax);
-    RLVI_LAUNCH_CHECK(ctx);
-  }
-  if (pairs) return rlvi_tf32_pair_moments(ctx, tmap, tmap3, p, plan, part, want_gram, out, st);
+  wmax_kernel<<<grid_for(ctx, n, 8), 256, 0, st>>>(weights, n, s.tf32_wmax);
+  RLVI_LAUNCH_CHECK(ctx);
+  if (pairs)
+    return rlvi_tf32_pair_moments(ctx, tmap, tmap3, p, plan, reinterpret_cast<char*>(s.partials), want_gram, out, st);
 
   const int grid = cp.nslots;
-  p.gpart64 = reinterpret_cast<double*>(part);
+  p.gpart64 = s.partials;
   p.spart = p.gpart64 + size_t(grid) * kMB * kMB;
   cp.s0part = p.spart + size_t(grid) * kTeams * 2 * 128;
 #define RLVI_TF32_LAUNCH(NS, HY)                                                                                   \

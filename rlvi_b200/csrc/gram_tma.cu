@@ -453,10 +453,10 @@ int rlvi_gram_tma_f64(rlvi_ctx* ctx, const double* X, const double* y, const dou
   p.rows_per_chunk = ((n + nchunks - 1) / nchunks + kRows - 1) / kRows * kRows;
   nchunks = (n + p.rows_per_chunk - 1) / p.rows_per_chunk;
   const int64_t units = nchunks * p.npairs;
-  void* scratch = nullptr;
-  int rc = rlvi_scratch(ctx, 4096 + size_t(units) * kUnitStride * sizeof(double), &scratch);
+  RlviScratch s;
+  const int rc = rlvi_scratch_header(ctx, size_t(units) * kUnitStride * sizeof(double), &s);
   if (rc != RLVI_OK) return rc;
-  p.partials = reinterpret_cast<double*>(static_cast<char*>(scratch) + 4096);
+  p.partials = s.partials;
 #define RLVI_GRAM_TMA_LAUNCH(HY, CE)                                                                          \
   {                                                                                                           \
     RLVI_CUDA(cudaFuncSetAttribute(gram_tma_kernel<HY, CE>, cudaFuncAttributeMaxDynamicSharedMemorySize, kGSmem)); \

@@ -20,21 +20,48 @@ namespace {
 
 constexpr int kLossThreads = 256;
 
-struct LossParams {
-  const double* X;
-  const double* y;
-  const double* params;
+// What every loss kernel writes: l, exp(-l), and with weights the grid totals (sum w l, sum w) into wsum_out.
+struct LossOut {
   const double* w;
   double* losses;
   double* e_out;
   double* wsum_out;
+  double* partials;       // [grid][2]
+  unsigned int* ticket;
+};
+
+// One row's outputs; wi is only read when o.w is set.
+__device__ __forceinline__ void loss_row(const LossOut& o, int64_t row, double loss, double wi, double& s_wl,
+                                         double& s_w) {
+  if (o.losses) o.losses[row] = loss;
+  if (o.e_out) o.e_out[row] = exp(-loss);
+  if (o.w) {
+    s_wl = fma(wi, loss, s_wl);
+    s_w += wi;
+  }
+}
+
+// End of a loss kernel: block then grid totals of (sum w l, sum w).  `red` holds 2 * nwarps doubles.
+__device__ __forceinline__ void loss_sums(const LossOut& o, double s_wl, double s_w, double* red) {
+  if (!o.w) return;   // uniform across the grid
+  double v[2] = {s_wl, s_w};
+  block_sum<2>(v, red);
+  if (grid_total<2>(v, o.partials, o.ticket)) {
+    o.wsum_out[0] = v[0];
+    o.wsum_out[1] = v[1];
+  }
+}
+
+struct LossParams {
+  const double* X;
+  const double* y;
+  const double* params;
+  LossOut o;
   int64_t n;
   int d;
   int kind;
   int intercept;
   int L;
-  double* partials;       // [grid][2]
-  unsigned int* ticket;
 };
 
 // a = x.theta (or ||theta - x||^2 for SQDIST), b = x.x (PCA only), b0 = intercept, yi = label / target.
@@ -106,40 +133,10 @@ __global__ void __launch_bounds__(kLossThreads) loss_kernel(const LossParams p) 
     if (DOTK == 1) b = group_sum(b, L);
     if (q == 0 && valid) {
       const double loss = finish_loss(p.kind, a, b, b0, (p.kind == RLVI_LOSS_LOGISTIC_CE || p.kind == RLVI_LOSS_SQRES) ? p.y[row] : 0.0);
-      if (p.losses) p.losses[row] = loss;
-      if (p.e_out) p.e_out[row] = exp(-loss);
-      if (p.w) {
-        const double wi = p.w[row];
-        s_wl = fma(wi, loss, s_wl);
-        s_w += wi;
-      }
+      loss_row(p.o, row, loss, p.o.w ? p.o.w[row] : 0.0, s_wl, s_w);
     }
   }
-
-  if (p.w) {   // uniform across the grid
-    double v[2] = {s_wl, s_w};
-    block_sum<2>(v, sm_red);
-    if (threadIdx.x == 0) {
-      p.partials[2 * blockIdx.x] = v[0];
-      p.partials[2 * blockIdx.x + 1] = v[1];
-    }
-    if (last_block_ticket(p.ticket, gridDim.x)) {
-      // fixed-order final sum by warp 0 of the last block
-      if (threadIdx.x < 32) {
-        double a0 = 0.0, a1 = 0.0;
-        for (unsigned int j = lane; j < gridDim.x; j += 32) {
-          a0 += p.partials[2 * j];
-          a1 += p.partials[2 * j + 1];
-        }
-        a0 = warp_sum(a0);
-        a1 = warp_sum(a1);
-        if (lane == 0) {
-          p.wsum_out[0] = a0;
-          p.wsum_out[1] = a1;
-        }
-      }
-    }
-  }
+  loss_sums(p.o, s_wl, s_w, sm_red);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -156,17 +153,12 @@ struct LossTmaParams {
   const double* X;
   const double* y;
   const double* params;
-  const double* w;
-  double* losses;
-  double* e_out;
-  double* wsum_out;
+  LossOut o;
   int64_t n;
   int d;
   int kind;
   int intercept;
   RingGeom geom;
-  double* partials;   // [grid][2]
-  unsigned int* ticket;
 };
 
 // shared-memory tail after the ring: theta (d doubles, padded), the barriers, the block-reduction scratch
@@ -195,7 +187,7 @@ __global__ void __launch_bounds__(kRingThreads, 1) loss_tma_kernel(const LossTma
   double s_wl = 0.0, s_w = 0.0;
 
   if (warp == kRingConsumers) {
-    ring_produce(ring, p.X, need_y ? p.y : nullptr, p.w, p.n, my_tiles, false);
+    ring_produce(ring, p.X, need_y ? p.y : nullptr, p.o.w, p.n, my_tiles, false);
   } else if (warp < p.geom.ncons) {
     const double2* th2 = reinterpret_cast<const double2*>(sTheta);
     const int npair = d >> 1;                      // 16-byte units per row, a multiple of 8
@@ -237,41 +229,10 @@ __global__ void __launch_bounds__(kRingThreads, 1) loss_tma_kernel(const LossTma
       const double wi = st.w[lane];
       ring_release(ring, st);                        // the stage can be refilled while we do the tail
       const int64_t row = ring_row0(t) + lane;
-      if (row < p.n) {
-        const double loss = finish_loss(p.kind, a, b, b0, need_y ? yi : 0.0);
-        if (p.losses) p.losses[row] = loss;
-        if (p.e_out) p.e_out[row] = exp(-loss);
-        if (p.w) {
-          s_wl = fma(wi, loss, s_wl);
-          s_w += wi;
-        }
-      }
+      if (row < p.n) loss_row(p.o, row, finish_loss(p.kind, a, b, b0, need_y ? yi : 0.0), wi, s_wl, s_w);
     }
   }
-
-  if (p.w) {   // uniform across the grid
-    double v[2] = {s_wl, s_w};
-    block_sum<2>(v, sRed);
-    if (threadIdx.x == 0) {
-      p.partials[2 * blockIdx.x] = v[0];
-      p.partials[2 * blockIdx.x + 1] = v[1];
-    }
-    if (last_block_ticket(p.ticket, gridDim.x)) {
-      if (threadIdx.x < 32) {
-        double a0 = 0.0, a1 = 0.0;
-        for (unsigned int j = lane; j < gridDim.x; j += 32) {
-          a0 += p.partials[2 * j];
-          a1 += p.partials[2 * j + 1];
-        }
-        a0 = warp_sum(a0);
-        a1 = warp_sum(a1);
-        if (lane == 0) {
-          p.wsum_out[0] = a0;
-          p.wsum_out[1] = a1;
-        }
-      }
-    }
-  }
+  loss_sums(p.o, s_wl, s_w, sRed);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -287,14 +248,9 @@ __global__ void __launch_bounds__(kRingThreads, 1) loss_tma_kernel(const LossTma
 struct GaussParams {
   const double* X;
   const double* params;   // [c, mu(d), U(d*d) row-major upper triangular]
-  const double* w;
-  double* losses;
-  double* e_out;
-  double* wsum_out;
+  LossOut o;
   int64_t n;
   int d;
-  double* partials;
-  unsigned int* ticket;
 };
 
 template <int NB_MAX, bool VEC>
@@ -367,38 +323,10 @@ __global__ void __launch_bounds__(kLossThreads) gaussian_loss_kernel(const Gauss
     quad += __shfl_xor_sync(0xffffffffu, quad, 2);
     if (t == 0 && valid) {
       const double loss = 0.5 * (quad + cst);                    // utils.py:101
-      if (p.losses) p.losses[row] = loss;
-      if (p.e_out) p.e_out[row] = exp(-loss);
-      if (p.w) {
-        const double wi = p.w[row];
-        s_wl = fma(wi, loss, s_wl);
-        s_w += wi;
-      }
+      loss_row(p.o, row, loss, p.o.w ? p.o.w[row] : 0.0, s_wl, s_w);
     }
   }
-  if (p.w) {
-    double v[2] = {s_wl, s_w};
-    block_sum<2>(v, sRed);
-    if (threadIdx.x == 0) {
-      p.partials[2 * blockIdx.x] = v[0];
-      p.partials[2 * blockIdx.x + 1] = v[1];
-    }
-    if (last_block_ticket(p.ticket, gridDim.x)) {
-      if (threadIdx.x < 32) {
-        double a0 = 0.0, a1 = 0.0;
-        for (unsigned int j = lane; j < gridDim.x; j += 32) {
-          a0 += p.partials[2 * j];
-          a1 += p.partials[2 * j + 1];
-        }
-        a0 = warp_sum(a0);
-        a1 = warp_sum(a1);
-        if (lane == 0) {
-          p.wsum_out[0] = a0;
-          p.wsum_out[1] = a1;
-        }
-      }
-    }
-  }
+  loss_sums(p.o, s_wl, s_w, sRed);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -411,15 +339,10 @@ __global__ void __launch_bounds__(kLossThreads) gaussian_loss_kernel(const Gauss
 struct GaussTmaParams {
   const double* X;
   const double* params;   // [c, mu(d), U(d*d) row-major upper triangular]
-  const double* w;
-  double* losses;
-  double* e_out;
-  double* wsum_out;
+  LossOut o;
   int64_t n;
   int d;
   RingGeom geom;
-  double* partials;
-  unsigned int* ticket;
 };
 
 static inline size_t gauss_tma_tail(int d) {
@@ -452,7 +375,7 @@ __global__ void __launch_bounds__(kRingThreads, 1) gaussian_tma_kernel(const Gau
   double s_wl = 0.0, s_w = 0.0;
 
   if (warp == kRingConsumers) {
-    ring_produce(ring, p.X, nullptr, p.w, p.n, my_tiles, false);
+    ring_produce(ring, p.X, nullptr, p.o.w, p.n, my_tiles, false);
   } else if (warp < p.geom.ncons) {
     const int g = lane >> 2, t = lane & 3;
     for (int64_t tl = warp; tl < my_tiles; tl += p.geom.ncons) {
@@ -494,41 +417,10 @@ __global__ void __launch_bounds__(kRingThreads, 1) gaussian_tma_kernel(const Gau
       const double wi = st.w[lane];
       ring_release(ring, st);
       const int64_t row = ring_row0(tl) + lane;
-      if (row < p.n) {
-        const double loss = 0.5 * (myquad + cst);                    // utils.py:101
-        if (p.losses) p.losses[row] = loss;
-        if (p.e_out) p.e_out[row] = exp(-loss);
-        if (p.w) {
-          s_wl = fma(wi, loss, s_wl);
-          s_w += wi;
-        }
-      }
+      if (row < p.n) loss_row(p.o, row, 0.5 * (myquad + cst), wi, s_wl, s_w);   // utils.py:101
     }
   }
-
-  if (p.w) {
-    double v[2] = {s_wl, s_w};
-    block_sum<2>(v, sRed);
-    if (threadIdx.x == 0) {
-      p.partials[2 * blockIdx.x] = v[0];
-      p.partials[2 * blockIdx.x + 1] = v[1];
-    }
-    if (last_block_ticket(p.ticket, gridDim.x)) {
-      if (threadIdx.x < 32) {
-        double a0 = 0.0, a1 = 0.0;
-        for (unsigned int j = lane; j < gridDim.x; j += 32) {
-          a0 += p.partials[2 * j];
-          a1 += p.partials[2 * j + 1];
-        }
-        a0 = warp_sum(a0);
-        a1 = warp_sum(a1);
-        if (lane == 0) {
-          p.wsum_out[0] = a0;
-          p.wsum_out[1] = a1;
-        }
-      }
-    }
-  }
+  loss_sums(p.o, s_wl, s_w, sRed);
 }
 
 template <int DOTK>
@@ -550,6 +442,15 @@ int launch_loss(rlvi_ctx* ctx, const RowMapCfg& cfg, LossParams& p, int grid, si
   return RLVI_ERR_UNSUPPORTED;
 }
 
+// The grid's (sum w l, sum w) partials and the ticket, from the scratch header.
+int loss_scratch(rlvi_ctx* ctx, int grid, LossOut& o) {
+  RlviScratch s;
+  const int rc = rlvi_scratch_header(ctx, size_t(grid) * 2 * sizeof(double), &s);
+  o.partials = s.partials;
+  o.ticket = s.ticket;
+  return rc;
+}
+
 
 // ---------------------------------------------------------------------------------------------
 // FP32-STORED X (the FP32 mode of SURVEY.md section 8d, config C3): the same losses from float32 samples.
@@ -562,17 +463,12 @@ struct LossF32Params {
   const float* X;
   const double* y;
   const double* params;
-  const double* w;
-  double* losses;
-  double* e_out;
-  double* wsum_out;
+  LossOut o;
   int64_t n;
   int d;
   int kind;
   int intercept;
   int vec;                // X 16-byte aligned and d % 4 == 0
-  double* partials;       // [grid][2]
-  unsigned int* ticket;
 };
 
 // float -> double on the integer pipe: F2F.F64.F32 issues at ~4 lanes / clk / SM on B200 (measured: the conversion, not
@@ -661,39 +557,10 @@ __global__ void __launch_bounds__(kLossThreads) loss_f32_kernel(const LossF32Par
     if (DOTK == 1) b = warp_sum(b);
     if (lane == 0) {
       const double loss = finish_loss(p.kind, a, b, b0, (p.kind == RLVI_LOSS_LOGISTIC_CE || p.kind == RLVI_LOSS_SQRES) ? p.y[row] : 0.0);
-      if (p.losses) p.losses[row] = loss;
-      if (p.e_out) p.e_out[row] = exp(-loss);
-      if (p.w) {
-        const double wi = p.w[row];
-        s_wl = fma(wi, loss, s_wl);
-        s_w += wi;
-      }
+      loss_row(p.o, row, loss, p.o.w ? p.o.w[row] : 0.0, s_wl, s_w);
     }
   }
-
-  if (p.w) {   // uniform across the grid
-    double v[2] = {s_wl, s_w};
-    block_sum<2>(v, sm_red);
-    if (threadIdx.x == 0) {
-      p.partials[2 * blockIdx.x] = v[0];
-      p.partials[2 * blockIdx.x + 1] = v[1];
-    }
-    if (last_block_ticket(p.ticket, gridDim.x)) {
-      if (threadIdx.x < 32) {
-        double a0 = 0.0, a1 = 0.0;
-        for (unsigned int j = lane; j < gridDim.x; j += 32) {
-          a0 += p.partials[2 * j];
-          a1 += p.partials[2 * j + 1];
-        }
-        a0 = warp_sum(a0);
-        a1 = warp_sum(a1);
-        if (lane == 0) {
-          p.wsum_out[0] = a0;
-          p.wsum_out[1] = a1;
-        }
-      }
-    }
-  }
+  loss_sums(p.o, s_wl, s_w, sm_red);
 }
 
 }  // namespace
@@ -710,7 +577,7 @@ extern "C" int rlvi_loss_f64(rlvi_ctx* ctx, int kind, int intercept, const doubl
   RlviDeviceGuard guard(ctx->device);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   const int warps_per_block = kLossThreads / 32;
-  void* scratch = nullptr;
+  const LossOut o = {weights, losses_out, e_out, wsum_out, nullptr, nullptr};
 
   if (kind == RLVI_LOSS_GAUSSIAN) {
     if (d > 128) {
@@ -722,19 +589,14 @@ extern "C" int rlvi_loss_f64(rlvi_ctx* ctx, int kind, int intercept, const doubl
       GaussTmaParams q;
       q.X = X;
       q.params = params;
-      q.w = weights;
-      q.losses = losses_out;
-      q.e_out = e_out;
-      q.wsum_out = wsum_out;
+      q.o = o;
       q.n = n;
       q.d = d;
       const size_t tail = gauss_tma_tail(d);
       if (!ring_geometry(d, tail, &q.geom)) return RLVI_ERR_UNSUPPORTED;
       const int grid = ring_grid(q.geom, n, ctx->sm_count);
-      int rc = rlvi_scratch(ctx, 4096 + size_t(grid) * 2 * sizeof(double), &scratch);
+      const int rc = loss_scratch(ctx, grid, q.o);
       if (rc != RLVI_OK) return rc;
-      q.ticket = reinterpret_cast<unsigned int*>(static_cast<char*>(scratch) + 128);
-      q.partials = reinterpret_cast<double*>(static_cast<char*>(scratch) + 4096);
       const size_t smem = ring_bytes(q.geom) + tail;
 #define RLVI_GTMA_CASE(NB)                                                                                    \
   if (d == 8 * NB) {                                                                                          \
@@ -755,19 +617,14 @@ extern "C" int rlvi_loss_f64(rlvi_ctx* ctx, int kind, int intercept, const doubl
     int64_t steps = (n + 7) / 8;
     int64_t want = (steps + warps_per_block - 1) / warps_per_block;
     int grid = int(want < 1 ? 1 : (want > int64_t(ctx->sm_count) * 2 ? int64_t(ctx->sm_count) * 2 : want));
-    int rc = rlvi_scratch(ctx, 4096 + size_t(grid) * 2 * sizeof(double), &scratch);
-    if (rc != RLVI_OK) return rc;
     GaussParams p;
     p.X = X;
     p.params = params;
-    p.w = weights;
-    p.losses = losses_out;
-    p.e_out = e_out;
-    p.wsum_out = wsum_out;
+    p.o = o;
     p.n = n;
     p.d = d;
-    p.ticket = reinterpret_cast<unsigned int*>(static_cast<char*>(scratch) + 128);
-    p.partials = reinterpret_cast<double*>(static_cast<char*>(scratch) + 4096);
+    const int rc = loss_scratch(ctx, grid, p.o);
+    if (rc != RLVI_OK) return rc;
 #define RLVI_GAUSS_CASE(NB, V)                                                                             \
   if (nb <= NB && vec == V) {                                                                              \
     RLVI_CUDA(cudaFuncSetAttribute(gaussian_loss_kernel<NB, V>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
@@ -791,10 +648,7 @@ extern "C" int rlvi_loss_f64(rlvi_ctx* ctx, int kind, int intercept, const doubl
     q.X = X;
     q.y = y;
     q.params = params;
-    q.w = weights;
-    q.losses = losses_out;
-    q.e_out = e_out;
-    q.wsum_out = wsum_out;
+    q.o = o;
     q.n = n;
     q.d = d;
     q.kind = kind;
@@ -802,10 +656,8 @@ extern "C" int rlvi_loss_f64(rlvi_ctx* ctx, int kind, int intercept, const doubl
     const size_t tail = loss_tma_tail(d);
     if (ring_geometry(d, tail, &q.geom)) {
       const int grid = ring_grid(q.geom, n, ctx->sm_count);
-      int rc = rlvi_scratch(ctx, 4096 + size_t(grid) * 2 * sizeof(double), &scratch);
+      const int rc = loss_scratch(ctx, grid, q.o);
       if (rc != RLVI_OK) return rc;
-      q.ticket = reinterpret_cast<unsigned int*>(static_cast<char*>(scratch) + 128);
-      q.partials = reinterpret_cast<double*>(static_cast<char*>(scratch) + 4096);
       const size_t smem = ring_bytes(q.geom) + tail;
 #define RLVI_TMA_CASE(K)                                                                                   \
   {                                                                                                        \
@@ -831,23 +683,18 @@ extern "C" int rlvi_loss_f64(rlvi_ctx* ctx, int kind, int intercept, const doubl
   int64_t want = (steps + warps_per_block - 1) / warps_per_block;
   int64_t cap = int64_t(ctx->sm_count) * 8;    // 8 resident 256-thread CTAs per SM at <= 32 registers/thread... grid-stride covers the rest
   int grid = int(want < 1 ? 1 : (want > cap ? cap : want));
-  int rc = rlvi_scratch(ctx, 4096 + size_t(grid) * 2 * sizeof(double), &scratch);
-  if (rc != RLVI_OK) return rc;
   LossParams p;
   p.X = X;
   p.y = y;
   p.params = params;
-  p.w = weights;
-  p.losses = losses_out;
-  p.e_out = e_out;
-  p.wsum_out = wsum_out;
+  p.o = o;
   p.n = n;
   p.d = d;
   p.kind = kind;
   p.intercept = intercept ? 1 : 0;
   p.L = cfg.L;
-  p.ticket = reinterpret_cast<unsigned int*>(static_cast<char*>(scratch) + 128);
-  p.partials = reinterpret_cast<double*>(static_cast<char*>(scratch) + 4096);
+  const int rc = loss_scratch(ctx, grid, p.o);
+  if (rc != RLVI_OK) return rc;
   const size_t smem = (size_t(d) + 2 + 2 * warps_per_block) * sizeof(double);
   if (kind == RLVI_LOSS_PCA) return launch_loss<1>(ctx, cfg, p, grid, smem, st);
   if (kind == RLVI_LOSS_SQDIST) return launch_loss<2>(ctx, cfg, p, grid, smem, st);
@@ -873,24 +720,18 @@ extern "C" int rlvi_loss_f32(rlvi_ctx* ctx, int kind, int intercept, const float
   int64_t want = (n + warps_per_block - 1) / warps_per_block;
   const int64_t cap = int64_t(ctx->sm_count) * 8;
   const int grid = int(want < 1 ? 1 : (want > cap ? cap : want));
-  void* scratch = nullptr;
-  int rc = rlvi_scratch(ctx, 4096 + size_t(grid) * 2 * sizeof(double), &scratch);
-  if (rc != RLVI_OK) return rc;
   LossF32Params p;
   p.X = X;
   p.y = y;
   p.params = params;
-  p.w = weights;
-  p.losses = losses_out;
-  p.e_out = e_out;
-  p.wsum_out = wsum_out;
+  p.o = {weights, losses_out, e_out, wsum_out, nullptr, nullptr};
   p.n = n;
   p.d = d;
   p.kind = kind;
   p.intercept = intercept ? 1 : 0;
   p.vec = (rlvi_aligned16(X) && d % 4 == 0) ? 1 : 0;
-  p.ticket = reinterpret_cast<unsigned int*>(static_cast<char*>(scratch) + 128);
-  p.partials = reinterpret_cast<double*>(static_cast<char*>(scratch) + 4096);
+  const int rc = loss_scratch(ctx, grid, p.o);
+  if (rc != RLVI_OK) return rc;
   const size_t smem = (size_t((d + 127) & ~127) + 2 + 2 * warps_per_block) * sizeof(double);
   if (kind == RLVI_LOSS_PCA) loss_f32_kernel<1><<<grid, kLossThreads, smem, st>>>(p);
   else if (kind == RLVI_LOSS_SQDIST) loss_f32_kernel<2><<<grid, kLossThreads, smem, st>>>(p);

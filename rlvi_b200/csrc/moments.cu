@@ -736,10 +736,10 @@ int run_colsum(rlvi_ctx* ctx, const double* X, const double* y, const double* w,
     const size_t tail = colsum_tma_tail(d);
     if (ring_geometry(d, tail, &q.geom)) {
       const int grid = ring_grid(q.geom, n, ctx->sm_count);
-      void* scratch = nullptr;
-      int rc = rlvi_scratch(ctx, 4096 + size_t(grid) * stride * sizeof(double), &scratch);
+      RlviScratch s;
+      const int rc = rlvi_scratch_header(ctx, size_t(grid) * stride * sizeof(double), &s);
       if (rc != RLVI_OK) return rc;
-      q.partials = reinterpret_cast<double*>(static_cast<char*>(scratch) + 4096);
+      q.partials = s.partials;
       const size_t smem = ring_bytes(q.geom) + tail;
       RLVI_CUDA(cudaFuncSetAttribute(colsum_tma_kernel<MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
       colsum_tma_kernel<MODE><<<grid, kRingThreads, smem, st>>>(q);
@@ -763,8 +763,8 @@ int run_colsum(rlvi_ctx* ctx, const double* X, const double* y, const double* w,
   const int64_t cap = int64_t(ctx->sm_count) * 2;
   const int grid = int(want < 1 ? 1 : (want > cap ? cap : want));
   const int stride = 2 + 2 * d;
-  void* scratch = nullptr;
-  int rc = rlvi_scratch(ctx, 4096 + size_t(grid) * stride * sizeof(double), &scratch);
+  RlviScratch s;
+  int rc = rlvi_scratch_header(ctx, size_t(grid) * stride * sizeof(double), &s);
   if (rc != RLVI_OK) return rc;
   ColParams p;
   p.X = X;
@@ -776,7 +776,7 @@ int run_colsum(rlvi_ctx* ctx, const double* X, const double* y, const double* w,
   p.d = d;
   p.power = power;
   p.L = cfg.L;
-  p.partials = reinterpret_cast<double*>(static_cast<char*>(scratch) + 4096);
+  p.partials = s.partials;
   size_t smem = size_t(nwarp) * stride * sizeof(double);
   if (smem < size_t(d + 1) * sizeof(double)) smem = size_t(d + 1) * sizeof(double);
   rc = launch_colsum<MODE>(ctx, cfg, p, grid, smem, st);
@@ -820,8 +820,8 @@ static int weighted_moments_impl(rlvi_ctx* ctx, const double* X, const double* y
   if (fast) {
     const int64_t ntiles = (n + kTileRows - 1) / kTileRows;
     const int grid = int(ntiles < ctx->sm_count ? ntiles : ctx->sm_count);
-    void* scratch = nullptr;
-    int rc = rlvi_scratch(ctx, 4096 + size_t(grid) * kPartialStride * sizeof(double), &scratch);
+    RlviScratch s;
+    const int rc = rlvi_scratch_header(ctx, size_t(grid) * kPartialStride * sizeof(double), &s);
     if (rc != RLVI_OK) return rc;
     GramParams p;
     p.X = X;
@@ -829,7 +829,7 @@ static int weighted_moments_impl(rlvi_ctx* ctx, const double* X, const double* y
     p.w = weights;
     p.n = n;
     p.power = power;
-    p.partials = reinterpret_cast<double*>(static_cast<char*>(scratch) + 4096);
+    p.partials = s.partials;
     p.center = center;
 #define RLVI_GRAM64_LAUNCH(HY, CE)                                                                              \
   {                                                                                                             \
@@ -878,10 +878,10 @@ static int weighted_moments_impl(rlvi_ctx* ctx, const double* X, const double* y
   g.rows_per_chunk = ((n + nchunks - 1) / nchunks + kGR - 1) / kGR * kGR;
   nchunks = (n + g.rows_per_chunk - 1) / g.rows_per_chunk;
   g.nchunks = int(nchunks);
-  void* scratch = nullptr;
-  rc = rlvi_scratch(ctx, 4096 + size_t(nchunks) * npairs * kGT * kGT * sizeof(double), &scratch);
+  RlviScratch s;
+  rc = rlvi_scratch_header(ctx, size_t(nchunks) * npairs * kGT * kGT * sizeof(double), &s);
   if (rc != RLVI_OK) return rc;
-  g.partials = reinterpret_cast<double*>(static_cast<char*>(scratch) + 4096);
+  g.partials = s.partials;
   gen_gram_kernel<<<dim3(npairs, g.nchunks), 256, 0, st>>>(g);
   RLVI_LAUNCH_CHECK(ctx);
   const int64_t total = int64_t(npairs) * kGT * kGT;
