@@ -322,6 +322,33 @@ int rlvi_batched_em_f64(rlvi_ctx* ctx, int model, const double* X, const double*
                         int64_t n_rows, int d, double tol, int maxiter, double* theta_out, int32_t* iters_out,
                         int32_t* status_out, void* stream);
 
+enum rlvi_batched_logreg_mstep {
+  RLVI_BATCHED_LOGREG_NEWTON = 0,  /* standard-learning/utils.py:61-73 via the drop-in's Newton solve */
+  RLVI_BATCHED_LOGREG_MM = 1       /* standard-learning/utils.py:32-58                              */
+};
+
+/* Rows one problem of rlvi_batched_logistic_f64 may have at `d` features (1 <= d <= 63; 0 outside): the shared-memory
+ * budget of one warp.  At least 1024 at every d and at least 2000 at d <= 8. */
+int rlvi_batched_logistic_max_rows(int d);
+
+/* The whole EM loop of standard-learning/rlvi.py:92-108 per problem, following the drop-in rlvi_b200/rlvi.py
+ * logistic_regression: pi = 1; M-step; then up to `maxiter` times the E-step (the update_weights fixed point, tol 1e-3,
+ * maxiter 100, on the M-step's unscaled losses) and the M-step, stopping at the first theta with
+ * ||theta - prev|| / ||prev|| <= tol.  The design is [1, X]: theta has d + 1 entries, intercept first.  M-steps:
+ *   NEWTON  the minimiser of 1/2 |theta|^2 + 100 sum_i w_i CE_i, w = pi / max pi, by the drop-in's damped Newton
+ *           iteration (Hessian I + 100 [1,X]^T diag(w e (1 - e)) [1,X] by Cholesky, Armijo backtracking, stop when a full
+ *           step has |step| <= 1e-9 (1 + |theta|), at most 60 steps), warm-started from the previous EM iterate (0 first);
+ *           E-step losses softplus(b + x.w), whatever the label;
+ *   MM      theta <- theta - Q^-1 [1,X]^T (pi (sigmoid - y)) from theta = 0 while |delta theta| > 1e-2, with
+ *           Q = 1/4 [1,X]^T Pi [1,X] factored once per M-step; E-step losses the cross-entropy with y.
+ * Outputs: theta_out [nprob][d + 1], iters_out [nprob] (EM iterations), status_out [nprob]: 0 stop test met, 1 maxiter
+ * reached, 2 the problem needs the single-problem drop-in (theta NaN): Newton did not converge in 60 steps (a non-finite
+ * objective included), or MM's Q failed rlvi_batched_em_f64's pivot test (min L_ii^2 / Q_ii > 2^-52 (d + 1 + sqrt(n))),
+ * or MM took 10000 steps; -1 rejected segment.  RLVI_ERR_UNSUPPORTED for d outside 1..63. */
+int rlvi_batched_logistic_f64(rlvi_ctx* ctx, int mstep, const double* X, const double* y, const int64_t* offsets,
+                              int nprob, int64_t n_rows, int d, double tol, int maxiter, double* theta_out,
+                              int32_t* iters_out, int32_t* status_out, void* stream);
+
 /* ---- host-buffer convenience (the drop-in's NumPy route; bench.py's `e2e`) ------------------- */
 /* One E+M step of the logistic model on HOST buffers (pinned or pageable): chunks of X/y are copied
  * H2D on a copy stream while the loss kernel consumes the previous chunk; then the fixed point and

@@ -20,13 +20,15 @@ SYMBOLS = (
     "rlvi_weighted_moments_f64", "rlvi_weighted_moments_centered_f64", "rlvi_logistic_grad_f64", "rlvi_wce_fwd_bwd_f32", "rlvi_fn_threshold_f32",
     "rlvi_em_step_logistic_host", "rlvi_dist_window_create", "rlvi_dist_window_open", "rlvi_dist_window_close",
     "rlvi_stats_allreduce_f64", "rlvi_em_step_logistic_host_sharded", "rlvi_weighted_moments_f32", "rlvi_loss_f32", "rlvi_sigmoid_f64", "rlvi_online_ce_f64", "rlvi_irls_weights_f64", "rlvi_rrm_sum_f64", "rlvi_sever_pass_f64",
-    "rlvi_batched_max_rows", "rlvi_batched_fixed_point_f64", "rlvi_batched_em_f64",
+    "rlvi_batched_max_rows", "rlvi_batched_fixed_point_f64", "rlvi_batched_em_f64", "rlvi_batched_logistic_max_rows",
+    "rlvi_batched_logistic_f64",
 )
 
 FP_STANDARD, FP_ONLINE, FP_DEEP = 0, 1, 2
 LOSS_LOGISTIC_CE, LOSS_SOFTPLUS, LOSS_SQRES, LOSS_SQDIST, LOSS_PCA, LOSS_GAUSSIAN = range(6)
 TF32X3, TF32X1 = 0, 1
 BATCHED_MEAN, BATCHED_LINREG = 0, 1
+BATCHED_LOGREG_NEWTON, BATCHED_LOGREG_MM = 0, 1
 
 
 class FpResult(C.Structure):
@@ -92,6 +94,8 @@ def load():
         lib.rlvi_batched_max_rows.argtypes = [i32]
         lib.rlvi_batched_fixed_point_f64.argtypes = [vp, vp, vp, i32, i64, f64, i32, vp, vp, vp]
         lib.rlvi_batched_em_f64.argtypes = [vp, i32, vp, vp, vp, i32, i64, i32, f64, i32, vp, vp, vp, vp]
+        lib.rlvi_batched_logistic_max_rows.argtypes = [i32]
+        lib.rlvi_batched_logistic_f64.argtypes = [vp, i32, vp, vp, vp, i32, i64, i32, f64, i32, vp, vp, vp, vp]
         lib.rlvi_dist_window_create.argtypes = [vp, i32, C.POINTER(vp), C.c_char_p]
         lib.rlvi_dist_window_open.argtypes = [vp, i32, i32, vp, C.c_char_p, C.POINTER(vp)]
         lib.rlvi_dist_window_close.argtypes = [vp, i32, i32, vp, vp]

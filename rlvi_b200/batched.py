@@ -3,20 +3,26 @@
     update_weights(losses, tol=1e-3, maxiter=100)       rlvi.py:8-20   [B, n] -> [B, n];  list of 1-D -> list
     mean(samples, maxiter=100, tol=1e-3)                rlvi.py:46-65  [B, n, d] or list of [n_b, d] -> theta [B, d]
     linear_regression(X, y, maxiter=100, tol=1e-3)      rlvi.py:68-89  [B, n, d], [B, n] or lists -> theta [B, d]
+    logistic_regression(X, y, maxiter=100, tol=1e-2, mstep="sklearn")
+                                                        rlvi.py:92-108 [B, n, d], [B, n] or lists -> theta [B, d + 1]
 
 The reference's experiment driver (standard-learning/main.py) fits thousands of tiny problems -- Monte-Carlo runs over a
 grid of corruption rates at N = 40..100 -- and so do bootstrap replicates and per-group fits.  One call per problem through
 rlvi_b200.rlvi costs about ten launches and two host synchronisations per EM iteration; here every problem runs its whole
 EM loop inside one warp of one kernel (rlvi_batched_em_f64), so a sweep is one launch.  Each problem gets the result the
-single-problem drop-in computes, to rounding: the same fixed point, the same M-step through the normal equations, the same
-stop test.
+single-problem drop-in computes, to rounding: the same fixed point, the same M-step (the normal equations; for logistic
+regression the drop-in's Newton solve of utils.sklearn_log_reg or the MM iteration of utils.mm_log_reg, both in the
+warp, rlvi_batched_logistic_f64), the same stop test.
 
 A batch is a stacked array ([B, n, ...], every problem the same size) or a list of per-problem arrays (ragged).  NumPy in
 gives NumPy out (the problems are packed on the host and copied to the GPU once); CUDA float64 tensors in gives tensors out.
 A problem may have at most `rlvi_b200.ops.batched_max_rows(d)` rows (at least 1024 at every d <= 64); larger ones raise
 ValueError and belong to the single-problem functions.  Linear-regression problems whose normal equations fail the
 drop-in's pivot test (rank-deficient or ill-conditioned designs, n_b < d) are re-solved one by one with
-rlvi_b200.rlvi.linear_regression, whose eigen-decomposition route gives the minimum-norm answer.  There is no CPU fallback.
+rlvi_b200.rlvi.linear_regression, whose eigen-decomposition route gives the minimum-norm answer.  Logistic problems take
+at most `rlvi_b200.ops.batched_logistic_max_rows(d)` rows (at least 1024 at every d <= 63, 2000 at d <= 8); those whose
+Newton solve does not converge in 60 steps, or whose MM majoriser fails the pivot test, are re-solved one by one with
+rlvi_b200.rlvi.logistic_regression (an exception it raises names the problem).  There is no CPU fallback.
 """
 from __future__ import annotations
 
@@ -27,9 +33,10 @@ from . import ops
 from . import rlvi as _rlvi
 from ._host import default_device
 
-__all__ = ["update_weights", "mean", "linear_regression"]
+__all__ = ["update_weights", "mean", "linear_regression", "logistic_regression"]
 
-HOST_SOLVE = 2       # status of rlvi_batched_em_f64: the problem needs rlvi.linear_regression
+HOST_SOLVE = 2       # status of rlvi_batched_em_f64 / _logistic_f64: the problem needs the single-problem drop-in
+_LOGREG_MSTEP = {"sklearn": ops.BATCHED_LOGREG_NEWTON, "mm": ops.BATCHED_LOGREG_MM}
 
 
 def _gather(a, pdim, name):
@@ -60,10 +67,10 @@ def _offsets(lengths):
     return np.concatenate([[0], np.cumsum(lengths)]).astype(np.int64)
 
 
-def _check_cap(lengths, d, fn):
-    cap = ops.batched_max_rows(d)
+def _check_cap(lengths, d, fn, cap=None, d_max=64):
+    cap = ops.batched_max_rows(d) if cap is None else cap
     if cap == 0:
-        raise ValueError(f"batched.{fn} supports 1 <= d <= 64 (got d = {d}); use rlvi_b200.rlvi.{fn} per problem")
+        raise ValueError(f"batched.{fn} supports 1 <= d <= {d_max} (got d = {d}); use rlvi_b200.rlvi.{fn} per problem")
     if lengths.size and int(lengths.max()) > cap:
         raise ValueError(f"batched.{fn}: a problem has {int(lengths.max())} rows, the batched kernels admit at most {cap} "
                          f"rows per problem at d = {d}; fit larger problems with rlvi_b200.rlvi.{fn}")
@@ -124,4 +131,28 @@ def linear_regression(X, y, maxiter=100, tol=1e-3):
         # fresh copies: the drop-in's kernels choose their load path by alignment, and a copy gives the bits of the
         # problem fitted on its own
         theta[b] = _rlvi.linear_regression(Xd[s:e].clone(), yd[s:e].clone(), maxiter=maxiter, tol=tol)
+    return theta if is_t else theta.cpu().numpy()
+
+
+def logistic_regression(X, y, maxiter=100, tol=1e-2, mstep="sklearn"):
+    """rlvi.py:92-108 on every problem: X [B, n, d] or a list of [n_b, d], y [B, n] or a list of [n_b] -> theta [B, d + 1]
+    (intercept first).  `mstep` as in rlvi.logistic_regression: "sklearn" (the reference's default) or "mm"."""
+    if mstep not in _LOGREG_MSTEP:
+        raise ValueError(f'mstep must be "sklearn" or "mm" (got {mstep!r})')
+    fx, lengths, _, is_t = _gather(X, 2, "X")
+    fy, ly, _, _ = _gather(y, 1, "y")
+    if not np.array_equal(lengths, ly):
+        raise ValueError("X and y must describe the same problems with the same numbers of rows")
+    d = fx.shape[1]
+    _check_cap(lengths, d, "logistic_regression", ops.batched_logistic_max_rows(d), 63)
+    Xd, yd = _to_device(fx, fy.to(fx.device) if is_t else fy)
+    off = _offsets(lengths)
+    theta, _, status = ops.batched_logistic(Xd, yd, off, mstep=_LOGREG_MSTEP[mstep], tol=tol, maxiter=maxiter)
+    for b in np.flatnonzero(status.cpu().numpy() == HOST_SOLVE):
+        s, e = int(off[b]), int(off[b + 1])
+        try:     # fresh copies, as in linear_regression
+            theta[b] = _rlvi.logistic_regression(Xd[s:e].clone(), yd[s:e].clone(), maxiter=maxiter, tol=tol, mstep=mstep)
+        except Exception as exc:
+            exc.args = (f"batched.logistic_regression, problem {b}: {exc.args[0] if exc.args else exc}",) + exc.args[1:]
+            raise
     return theta if is_t else theta.cpu().numpy()

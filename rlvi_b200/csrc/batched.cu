@@ -5,6 +5,7 @@
 //   standard-learning/rlvi.py:8-20    update_weights     -> batched_fp_kernel
 //   standard-learning/rlvi.py:46-65   mean               -> batched_em_kernel<MODEL_MEAN>
 //   standard-learning/rlvi.py:68-89   linear_regression  -> batched_em_kernel<MODEL_LINREG>
+//   standard-learning/rlvi.py:92-108  logistic_regression -> batched_logreg_kernel<LOGREG_NEWTON / LOGREG_MM>
 // At that size a drop-in EM iteration is ~10 launches and two host synchronisations; here a problem's EM loop, its
 // fixed points, the d x d Cholesky and the stop tests run inside one warp, with no host round trip.
 //
@@ -40,8 +41,8 @@ __host__ __device__ inline int warp_doubles(int d) {
   return need > kMinWarpDoubles ? need : kMinWarpDoubles;
 }
 __host__ __device__ inline int max_rows(int d) { return warp_doubles(d) - d * g_ld(d) - 4 * d; }
-inline int warps_per_cta(int d) {
-  const int w = int(kSmemBudget / (size_t(warp_doubles(d)) * sizeof(double)));
+inline int warps_per_cta(size_t warp_bytes) {
+  const int w = int(kSmemBudget / warp_bytes);
   return w > kMaxWarpsPerCta ? kMaxWarpsPerCta : w;
 }
 
@@ -291,15 +292,316 @@ __global__ void batched_em_kernel(const double* __restrict__ X, const double* __
   }
 }
 
+// ---- logistic regression ---------------------------------------------------------------------------------------------
+// rlvi_b200/rlvi.py logistic_regression per problem, with either M-step of the drop-in:
+//   LOGREG_NEWTON  utils.sklearn_log_reg: F = 1/2 |theta|^2 + C sum_i w_i CE_i, w = pi / max pi, C = 100, damped Newton
+//                  with Armijo backtracking, warm-started from the previous EM iterate; E-step losses softplus(phi)
+//   LOGREG_MM      utils.mm_log_reg: theta <- theta - Q^-1 [1,X]^T (pi (sigmoid - y)), Q = 1/4 [1,X]^T Pi [1,X], from 0
+//                  while |delta theta| > 1e-2; E-step losses the cross-entropy with y
+// D = d + 1 parameters, intercept first; the design is [1, X].  The M-step's matrices are summed one lane per entry over
+// the rows in order, its vectors lane-strided plus the xor-shuffle tree, exactly as batched_em_kernel does; every branch
+// decision comes from such a warp-uniform value.  Every loop is bounded, so no problem can hold its warp forever.
+enum { LOGREG_NEWTON = RLVI_BATCHED_LOGREG_NEWTON, LOGREG_MM = RLVI_BATCHED_LOGREG_MM };
+
+constexpr int kLgMinRows = 1024;                      // the cap admits n = 1024 at every d in 1..63
+constexpr int kLgMinWarpDoubles = 4160;               // ... and n = 2008 at d <= 8
+constexpr int kLgMaxD = 63;
+constexpr double kLgC = 100.0;                        // utils.py:61 reg_coeff, which no caller varies
+constexpr int kNewtonMaxSteps = 60;                   // utils.sklearn_log_reg max_newton
+constexpr int kArmijoMaxHalvings = 27;                // t = 2^-27 is the first t < 1e-8
+constexpr int kMmMaxSteps = 10000;                    // the drop-in's MM loop has no bound; past this one the host solves
+
+// Per-warp shared memory, in doubles: w [cap] (pi, or Newton's pi / max pi) | v [cap] (e, curvature weights, gradient
+// coefficients or losses) | M [D][D + 1] | g [D] | theta [D] | theta_prev [D] | step [D] | theta_c [D] | diag(L) [D].
+__host__ __device__ inline int lg_fixed_doubles(int d) { return (d + 1) * (d + 2) + 6 * (d + 1); }
+__host__ __device__ inline int lg_warp_doubles(int d) {
+  const int need = 2 * kLgMinRows + lg_fixed_doubles(d);
+  return need > kLgMinWarpDoubles ? need : kLgMinWarpDoubles;
+}
+__host__ __device__ inline int lg_max_rows(int d) { return (lg_warp_doubles(d) - lg_fixed_doubles(d)) / 2; }
+
+// phi = theta_0 + x . theta_{1..d}, the row arithmetic of loss.cu and of the colsum gradient
+__device__ __forceinline__ double lg_phi(const double* xi, const double* th, int d) {
+  double a = 0.0;
+  for (int k = 0; k < d; ++k) a = fma(xi[k], th[k + 1], a);
+  return th[0] + a;
+}
+
+__device__ __forceinline__ double lg_sigmoid(double phi) {      // utils.py:7-16, overflow-free
+  const double z = exp(-fabs(phi));
+  return (phi >= 0.0 ? 1.0 : z) / (1.0 + z);
+}
+
+__device__ __forceinline__ double lg_ce(double phi, double yi) {   // loss.cu LOGISTIC_CE, utils.py:21
+  return (-yi * phi + phi) + log1p(exp(-phi));
+}
+
+__device__ __forceinline__ double lg_dot(const double* a, const double* b, int D) {
+  double s = 0.0;
+  for (int j = threadIdx.x & 31; j < D; j += kWarp) s = fma(a[j], b[j], s);
+  return warp_sum(s);
+}
+
+// M[j][k] = diag (j == k) + scale * sum_i v_i xt_ij xt_ik for k <= j < D, xt_i = [1, x_i]: one lane per entry, rows in order.
+__device__ void lg_gram(const double* __restrict__ X, int n, int d, const double* v, double scale, double diag, double* M) {
+  const int lane = threadIdx.x & 31;
+  const int D = d + 1, ld = D + 1, T = D * (D + 1) / 2;
+  for (int t = lane; t < T; t += kWarp) {
+    int j = int((sqrt(8.0 * t + 1.0) - 1.0) * 0.5);
+    while (j * (j + 1) / 2 > t) --j;
+    while ((j + 1) * (j + 2) / 2 <= t) ++j;
+    const int k = t - j * (j + 1) / 2;
+    double acc = 0.0;
+    for (int i = 0; i < n; ++i) {
+      const double* xi = X + int64_t(i) * d;
+      const double a = j ? xi[j - 1] : 1.0, b = k ? xi[k - 1] : 1.0;
+      acc = fma(v[i] * a, b, acc);
+    }
+    M[j * ld + k] = (j == k ? diag : 0.0) + scale * acc;
+  }
+  __syncwarp();
+}
+
+// out_j = sum_i v_i xt_ij: one lane per entry, rows in order
+__device__ void lg_xtv(const double* __restrict__ X, int n, int d, const double* v, double* out) {
+  for (int j = threadIdx.x & 31; j <= d; j += kWarp) {
+    double acc = 0.0;
+    for (int i = 0; i < n; ++i) acc = fma(v[i], j ? X[int64_t(i) * d + j - 1] : 1.0, acc);
+    out[j] = acc;
+  }
+  __syncwarp();
+}
+
+// Left-looking Cholesky of the lower triangle of M in place, diag(L) in dl; false unless every pivot L_jj^2 / M_jj
+// exceeds rtol (batched_em_kernel's test; rtol = 0 asks for positive, finite pivots only).
+__device__ bool lg_cholesky(double* M, int D, double* dl, double rtol) {
+  const int lane = threadIdx.x & 31, ld = D + 1;
+  for (int j = 0; j < D; ++j) {
+    const double mjj = M[j * ld + j];
+    double s = mjj;
+    for (int k = 0; k < j; ++k) s = fma(-M[j * ld + k], M[j * ld + k], s);
+    const double ljj = sqrt(s);
+    if (!(s > 0.0) || !(ljj * ljj / mjj > rtol) || !isfinite(ljj)) return false;   // warp-uniform
+    for (int i = j + 1 + lane; i < D; i += kWarp) {
+      double t = M[i * ld + j];
+      for (int k = 0; k < j; ++k) t = fma(-M[i * ld + k], M[j * ld + k], t);
+      M[i * ld + j] = t / ljj;
+    }
+    if (lane == 0) dl[j] = ljj;
+    __syncwarp();
+  }
+  return true;
+}
+
+// L L^T x = b in place (column sweeps)
+__device__ void lg_chol_solve(const double* M, int D, const double* dl, double* b) {
+  const int lane = threadIdx.x & 31, ld = D + 1;
+  for (int k = 0; k < D; ++k) {
+    const double zk = b[k] / dl[k];
+    __syncwarp();
+    for (int i = k + 1 + lane; i < D; i += kWarp) b[i] = fma(-M[i * ld + k], zk, b[i]);
+    if (lane == 0) b[k] = zk;
+    __syncwarp();
+  }
+  for (int k = D - 1; k >= 0; --k) {
+    const double tk = b[k] / dl[k];
+    __syncwarp();
+    for (int i = lane; i < k; i += kWarp) b[i] = fma(-M[k * ld + i], tk, b[i]);
+    if (lane == 0) b[k] = tk;
+    __syncwarp();
+  }
+}
+
+struct LgWarp {
+  const double* X;
+  const double* y;
+  int n, d;
+  double *w, *v, *M, *g, *th, *thp, *st, *tc, *dl;
+};
+
+// F(th) = 1/2 |th|^2 + C sum_i w_i CE_i (utils.sklearn_log_reg's objective); leaves e_i = exp(-CE_i) in v.
+__device__ double lg_objective(const LgWarp& p, const double* th) {
+  double s = 0.0;
+  for (int i = threadIdx.x & 31; i < p.n; i += kWarp) {
+    const double l = lg_ce(lg_phi(p.X + int64_t(i) * p.d, th, p.d), p.y[i]);
+    p.v[i] = exp(-l);
+    s = fma(p.w[i], l, s);
+  }
+  const double wl = warp_sum(s);
+  const double F = 0.5 * lg_dot(th, th, p.d + 1) + kLgC * wl;
+  __syncwarp();
+  return F;
+}
+
+// v_i = w_i (sigmoid(phi_i(th)) - y_i), the rows of rlvi_logistic_grad_f64
+__device__ void lg_grad_coeffs(const LgWarp& p, const double* th) {
+  for (int i = threadIdx.x & 31; i < p.n; i += kWarp)
+    p.v[i] = p.w[i] * (lg_sigmoid(lg_phi(p.X + int64_t(i) * p.d, th, p.d)) - p.y[i]);
+  __syncwarp();
+}
+
+// utils.sklearn_log_reg as the drop-in solves it.  On entry w = pi and th the warm start; on success th is the minimiser
+// and v its E-step losses softplus(phi); false when Newton does not converge in 60 steps or its matrix is not finite.
+__device__ bool lg_newton(const LgWarp& p) {
+  const int lane = threadIdx.x & 31, D = p.d + 1;
+  double m = -INFINITY;
+  for (int i = lane; i < p.n; i += kWarp) m = fmax(m, p.w[i]);
+  m = warp_max(m);
+  for (int i = lane; i < p.n; i += kWarp) p.w[i] = p.w[i] / m;              // utils.py:66
+  __syncwarp();
+  double F = lg_objective(p, p.th);
+  bool converged = false;
+  for (int it = 0; it < kNewtonMaxSteps && !converged; ++it) {
+    for (int i = lane; i < p.n; i += kWarp) {                                // rlvi_irls_weights_f64
+      const double s = p.v[i];
+      p.v[i] = p.w[i] * s * (1.0 - s);
+    }
+    __syncwarp();
+    lg_gram(p.X, p.n, p.d, p.v, kLgC, 1.0, p.M);                             // I + C [1,X]^T diag(h) [1,X]
+    lg_grad_coeffs(p, p.th);
+    lg_xtv(p.X, p.n, p.d, p.v, p.g);
+    for (int j = lane; j < D; j += kWarp) {
+      p.g[j] = p.th[j] + kLgC * p.g[j];                                      // grad = theta + C g
+      p.st[j] = p.g[j];
+    }
+    __syncwarp();
+    if (!lg_cholesky(p.M, D, p.dl, 0.0)) return false;
+    lg_chol_solve(p.M, D, p.dl, p.st);
+    const double slope = lg_dot(p.g, p.st, D);
+    const bool small = sqrt(lg_dot(p.st, p.st, D)) <= 1e-9 * (1.0 + sqrt(lg_dot(p.th, p.th, D)));
+    double t = 1.0, Fc = F;
+    for (int h = 0; h <= kArmijoMaxHalvings; ++h) {
+      for (int j = lane; j < D; j += kWarp) p.tc[j] = p.th[j] - t * p.st[j];
+      __syncwarp();
+      Fc = lg_objective(p, p.tc);
+      if (Fc <= F - 1e-4 * t * slope) break;                                 // Armijo
+      if (small && Fc <= F + 1e-12 * fabs(F)) break;                         // at the rounding floor of F
+      if (t < 1e-8) break;
+      t *= 0.5;
+    }
+    for (int j = lane; j < D; j += kWarp) p.th[j] = p.tc[j];
+    __syncwarp();
+    F = Fc;
+    converged = small && t == 1.0;
+  }
+  if (!converged) return false;
+  for (int i = lane; i < p.n; i += kWarp) {                                  // utils.py:70-71, label-independent
+    const double phi = lg_phi(p.X + int64_t(i) * p.d, p.th, p.d);
+    p.v[i] = fmax(phi, 0.0) + log1p(exp(-fabs(phi)));
+  }
+  __syncwarp();
+  return true;
+}
+
+// utils.mm_log_reg.  On entry w = pi; on success th is the MM iterate the drop-in returns and v its cross-entropy losses;
+// false when Q fails the pivot test or the step bound is reached.
+__device__ bool lg_mm(const LgWarp& p) {
+  const int lane = threadIdx.x & 31, D = p.d + 1;
+  lg_gram(p.X, p.n, p.d, p.w, 0.25, 0.0, p.M);                                // utils.py:36-38
+  if (!lg_cholesky(p.M, D, p.dl, kEps52 * (double(D) + sqrt(double(p.n))))) return false;
+  for (int j = lane; j < D; j += kWarp) p.th[j] = 0.0;                       // utils.py:35
+  __syncwarp();
+  bool done = false;
+  for (int it = 0; it < kMmMaxSteps && !done; ++it) {
+    for (int j = lane; j < D; j += kWarp) p.tc[j] = p.th[j];
+    __syncwarp();
+    lg_grad_coeffs(p, p.tc);
+    lg_xtv(p.X, p.n, p.d, p.v, p.st);
+    lg_chol_solve(p.M, D, p.dl, p.st);
+    double s = 0.0;
+    for (int j = lane; j < D; j += kWarp) {
+      p.th[j] = p.tc[j] - p.st[j];
+      const double t = p.th[j] - p.tc[j];
+      s = fma(t, t, s);
+    }
+    done = !(sqrt(warp_sum(s)) > 1e-2);                                       // utils.py:47; NaN stops too
+    __syncwarp();
+  }
+  if (!done) return false;
+  for (int i = lane; i < p.n; i += kWarp)                                     // utils.py:56
+    p.v[i] = lg_ce(lg_phi(p.X + int64_t(i) * p.d, p.th, p.d), p.y[i]);
+  __syncwarp();
+  return true;
+}
+
+template <int MSTEP>
+__device__ __forceinline__ bool lg_fit(const LgWarp& p) {
+  return MSTEP == LOGREG_NEWTON ? lg_newton(p) : lg_mm(p);
+}
+
+template <int MSTEP>
+__global__ void batched_logreg_kernel(const double* __restrict__ X, const double* __restrict__ y,
+                                      const int64_t* __restrict__ offsets, int nprob, int64_t n_rows, int d, double tol,
+                                      int maxiter, double* __restrict__ theta_out, int32_t* __restrict__ iters_out,
+                                      int32_t* __restrict__ status_out) {
+  extern __shared__ double batched_smem[];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int b = blockIdx.x * (blockDim.x >> 5) + warp;
+  if (b >= nprob) return;
+  const int D = d + 1, cap = lg_max_rows(d);
+  LgWarp p;
+  p.d = d;
+  p.w = batched_smem + size_t(warp) * lg_warp_doubles(d);
+  p.v = p.w + cap;
+  p.M = p.v + cap;
+  p.g = p.M + D * (D + 1);
+  p.th = p.g + D;
+  p.thp = p.th + D;
+  p.st = p.thp + D;
+  p.tc = p.st + D;
+  p.dl = p.tc + D;
+  double* out = theta_out + int64_t(b) * D;
+  int64_t start;
+  if (!segment(offsets, b, n_rows, cap, start, p.n)) {
+    for (int j = lane; j < D; j += kWarp) out[j] = NAN;
+    if (lane == 0) {
+      iters_out[b] = 0;
+      status_out[b] = ST_BAD_SEGMENT;
+    }
+    return;
+  }
+  p.X = X + start * d;
+  p.y = y + start;
+  for (int i = lane; i < p.n; i += kWarp) p.w[i] = 1.0;                      // rlvi.py:97  pi = 1
+  for (int j = lane; j < D; j += kWarp) p.th[j] = 0.0;                       // the first Newton fit starts from 0
+  __syncwarp();
+  int it = 0, status = lg_fit<MSTEP>(p) ? ST_MAXITER : ST_HOST_SOLVE;
+  while (status == ST_MAXITER && it < maxiter) {
+    const FpOut r = warp_fixed_point(p.v, p.n, 1.0, 1e-3, 100);             // rlvi.py:100, unscaled losses
+    for (int i = lane; i < p.n; i += kWarp) {
+      const double ev = p.v[i];
+      p.w[i] = ev / (r.rho + ev);
+    }
+    for (int j = lane; j < D; j += kWarp) p.thp[j] = p.th[j];               // also Newton's warm start
+    __syncwarp();
+    ++it;
+    if (!lg_fit<MSTEP>(p)) {
+      status = ST_HOST_SOLVE;
+      break;
+    }
+    double num = 0.0, den = 0.0;                                             // _rel_change
+    for (int j = lane; j < D; j += kWarp) {
+      const double t = p.th[j] - p.thp[j];
+      num = fma(t, t, num);
+      den = fma(p.thp[j], p.thp[j], den);
+    }
+    if (sqrt(warp_sum(num)) / sqrt(warp_sum(den)) <= tol) status = ST_CONVERGED;   // a NaN never stops the loop
+  }
+  for (int j = lane; j < D; j += kWarp) out[j] = (status == ST_HOST_SOLVE) ? NAN : p.th[j];
+  if (lane == 0) {
+    iters_out[b] = it;
+    status_out[b] = status;
+  }
+}
+
 struct LaunchShape {
   int grid, threads;
   size_t smem;
 };
 
-// warps_per_cta(d) problems per CTA, `per_warp_bytes` of dynamic shared memory each
+// `wpc` problems per CTA, `per_warp_bytes` of dynamic shared memory each
 template <typename K>
-int launch_shape(K kernel, int nprob, int d, size_t per_warp_bytes, LaunchShape& ls) {
-  const int wpc = warps_per_cta(d);
+int launch_shape(K kernel, int nprob, int wpc, size_t per_warp_bytes, LaunchShape& ls) {
   ls.grid = (nprob + wpc - 1) / wpc;
   ls.threads = wpc * kWarp;
   ls.smem = size_t(wpc) * per_warp_bytes;
@@ -324,7 +626,8 @@ extern "C" int rlvi_batched_fixed_point_f64(rlvi_ctx* ctx, const double* losses,
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   const int cap = max_rows(1);
   LaunchShape ls;
-  const int rc = launch_shape(batched_fp_kernel, nprob, 1, size_t(cap) * sizeof(double), ls);
+  const int rc = launch_shape(batched_fp_kernel, nprob, warps_per_cta(size_t(warp_doubles(1)) * sizeof(double)),
+                              size_t(cap) * sizeof(double), ls);
   if (rc != RLVI_OK) return rc;
   batched_fp_kernel<<<ls.grid, ls.threads, ls.smem, st>>>(losses, offsets, nprob, n_rows, cap, tol, maxiter, pi_out, results);
   RLVI_LAUNCH_CHECK(ctx);
@@ -349,15 +652,53 @@ extern "C" int rlvi_batched_em_f64(rlvi_ctx* ctx, int model, const double* X, co
   LaunchShape ls;
   int rc;
   if (model == RLVI_BATCHED_MEAN) {
-    rc = launch_shape(batched_em_kernel<MODEL_MEAN>, nprob, d, per_warp, ls);
+    rc = launch_shape(batched_em_kernel<MODEL_MEAN>, nprob, warps_per_cta(per_warp), per_warp, ls);
     if (rc != RLVI_OK) return rc;
     batched_em_kernel<MODEL_MEAN><<<ls.grid, ls.threads, ls.smem, st>>>(X, nullptr, offsets, nprob, n_rows, d, tol, maxiter,
                                                                theta_out, iters_out, status_out);
   } else {
-    rc = launch_shape(batched_em_kernel<MODEL_LINREG>, nprob, d, per_warp, ls);
+    rc = launch_shape(batched_em_kernel<MODEL_LINREG>, nprob, warps_per_cta(per_warp), per_warp, ls);
     if (rc != RLVI_OK) return rc;
     batched_em_kernel<MODEL_LINREG><<<ls.grid, ls.threads, ls.smem, st>>>(X, y, offsets, nprob, n_rows, d, tol, maxiter,
                                                                  theta_out, iters_out, status_out);
+  }
+  RLVI_LAUNCH_CHECK(ctx);
+  return RLVI_OK;
+}
+
+extern "C" int rlvi_batched_logistic_max_rows(int d) {
+  if (d < 1 || d > kLgMaxD) return 0;
+  return lg_max_rows(d);
+}
+
+extern "C" int rlvi_batched_logistic_f64(rlvi_ctx* ctx, int mstep, const double* X, const double* y,
+                                         const int64_t* offsets, int nprob, int64_t n_rows, int d, double tol,
+                                         int maxiter, double* theta_out, int32_t* iters_out, int32_t* status_out,
+                                         void* stream) {
+  RLVI_REQUIRE(ctx && X && y && offsets && theta_out && iters_out && status_out, "null pointer");
+  RLVI_REQUIRE(mstep == RLVI_BATCHED_LOGREG_NEWTON || mstep == RLVI_BATCHED_LOGREG_MM,
+               "mstep: RLVI_BATCHED_LOGREG_NEWTON, RLVI_BATCHED_LOGREG_MM");
+  RLVI_REQUIRE(nprob >= 1 && n_rows >= 1, "need at least one problem and one row");
+  RLVI_REQUIRE(maxiter >= 0, "maxiter must be >= 0");
+  if (d < 1 || d > kLgMaxD) {
+    rlvi_set_error("rlvi_batched_logistic_f64: d = %d outside 1..%d", d, kLgMaxD);
+    return RLVI_ERR_UNSUPPORTED;
+  }
+  RlviDeviceGuard guard(ctx->device);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const size_t per_warp = size_t(lg_warp_doubles(d)) * sizeof(double);
+  LaunchShape ls;
+  int rc;
+  if (mstep == RLVI_BATCHED_LOGREG_NEWTON) {
+    rc = launch_shape(batched_logreg_kernel<LOGREG_NEWTON>, nprob, warps_per_cta(per_warp), per_warp, ls);
+    if (rc != RLVI_OK) return rc;
+    batched_logreg_kernel<LOGREG_NEWTON><<<ls.grid, ls.threads, ls.smem, st>>>(X, y, offsets, nprob, n_rows, d, tol,
+                                                                               maxiter, theta_out, iters_out, status_out);
+  } else {
+    rc = launch_shape(batched_logreg_kernel<LOGREG_MM>, nprob, warps_per_cta(per_warp), per_warp, ls);
+    if (rc != RLVI_OK) return rc;
+    batched_logreg_kernel<LOGREG_MM><<<ls.grid, ls.threads, ls.smem, st>>>(X, y, offsets, nprob, n_rows, d, tol, maxiter,
+                                                                           theta_out, iters_out, status_out);
   }
   RLVI_LAUNCH_CHECK(ctx);
   return RLVI_OK;

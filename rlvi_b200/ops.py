@@ -12,14 +12,15 @@ import numpy as np
 import torch
 
 from . import _lib
-from ._lib import (BATCHED_LINREG, BATCHED_MEAN, FP_DEEP, FP_ONLINE, FP_STANDARD, LOSS_GAUSSIAN, LOSS_LOGISTIC_CE,
+from ._lib import (BATCHED_LINREG, BATCHED_LOGREG_MM, BATCHED_LOGREG_NEWTON, BATCHED_MEAN, FP_DEEP, FP_ONLINE, FP_STANDARD, LOSS_GAUSSIAN, LOSS_LOGISTIC_CE,
                    LOSS_PCA, LOSS_SOFTPLUS, LOSS_SQDIST, LOSS_SQRES, TF32X1, TF32X3)
 
 __all__ = ["FP_STANDARD", "FP_ONLINE", "FP_DEEP", "LOSS_LOGISTIC_CE", "LOSS_SOFTPLUS", "LOSS_SQRES",
            "LOSS_SQDIST", "LOSS_PCA", "LOSS_GAUSSIAN", "fixed_point", "fixed_point_deep", "shift_sum", "shift_sum_e", "loss",
            "weighted_moments", "split_moments", "logistic_grad", "wce_fwd_bwd", "fn_threshold", "read_result",
            "em_step_logistic_host", "launch_count", "TF32X3", "TF32X1", "sigmoid", "online_ce", "irls_weights", "rrm_sum",
-           "BATCHED_MEAN", "BATCHED_LINREG", "batched_max_rows", "batched_fixed_point", "batched_results", "batched_em"]
+           "BATCHED_MEAN", "BATCHED_LINREG", "batched_max_rows", "batched_fixed_point", "batched_results", "batched_em",
+           "BATCHED_LOGREG_NEWTON", "BATCHED_LOGREG_MM", "batched_logistic_max_rows", "batched_logistic"]
 
 _RESULT_DTYPE = np.dtype([("eps", "<f8"), ("rho", "<f8"), ("sum_pi", "<f8"), ("err", "<f8"), ("iters", "<i4"),
                           ("converged", "<i4")])
@@ -440,6 +441,44 @@ def batched_em(model, X, y, offsets, *, tol=1e-3, maxiter=100):
     rc = ctx.lib.rlvi_batched_em_f64(ctx.handle, int(model), _p(X), _p(y), _p(offs), nprob, rows, d, float(tol),
                                      int(maxiter), _p(theta), _p(iters), _p(status), _stream(dev))
     _lib.check(rc, "rlvi_batched_em_f64")
+    return theta, iters, status
+
+
+def batched_logistic_max_rows(d) -> int:
+    """rlvi_batched_logistic_max_rows: rows one problem of batched_logistic may have at `d` features (0 outside 1..63)."""
+    return int(_lib.load().rlvi_batched_logistic_max_rows(int(d)))
+
+
+def batched_logistic(X, y, offsets, *, mstep, tol=1e-2, maxiter=100):
+    """rlvi_batched_logistic_f64: the EM loop of rlvi.logistic_regression on every segment of the rows of X [rows, d] and
+    y [rows], with the Newton M-step of utils.sklearn_log_reg (mstep BATCHED_LOGREG_NEWTON) or utils.mm_log_reg
+    (BATCHED_LOGREG_MM).  `offsets` is a host integer array.  Returns device tensors (theta [nprob, d + 1] float64,
+    intercept first; iters [nprob] int32; status [nprob] int32): status 0 = stop test met, 1 = maxiter reached, 2 = theta
+    is NaN, solve that problem with rlvi.logistic_regression."""
+    dev = _dev(X)
+    f64 = torch.float64
+    _chk(X, f64, "X")
+    if mstep not in (BATCHED_LOGREG_NEWTON, BATCHED_LOGREG_MM):
+        raise ValueError("mstep must be BATCHED_LOGREG_NEWTON or BATCHED_LOGREG_MM")
+    if X.dim() != 2:
+        raise ValueError("X must be [rows, d]")
+    rows, d = X.shape
+    if not 1 <= d <= 63:
+        raise ValueError(f"batched logistic regression supports 1 <= d <= 63 (got d = {d})")
+    if y is None:
+        raise ValueError("logistic regression needs y")
+    _len(_chk(y, f64, "y"), rows, "y")
+    _same_device(X, y)
+    if int(maxiter) < 0:
+        raise ValueError("maxiter must be >= 0")
+    ctx = _ctx(dev)
+    offs, nprob = _batched_offsets(offsets, rows, ctx.lib.rlvi_batched_logistic_max_rows(d), X)
+    theta = torch.empty(nprob, d + 1, dtype=f64, device=X.device)
+    iters = torch.empty(nprob, dtype=torch.int32, device=X.device)
+    status = torch.empty(nprob, dtype=torch.int32, device=X.device)
+    rc = ctx.lib.rlvi_batched_logistic_f64(ctx.handle, int(mstep), _p(X), _p(y), _p(offs), nprob, rows, d, float(tol),
+                                           int(maxiter), _p(theta), _p(iters), _p(status), _stream(dev))
+    _lib.check(rc, "rlvi_batched_logistic_f64")
     return theta, iters, status
 
 
