@@ -428,9 +428,11 @@ __device__ __forceinline__ double2 ld_e2c(const ECache& ec, int slot, const doub
 
 // Branch-free fast evaluation of one trip (kFpUnroll chunks of two samples).  The issue slots are what bounds
 // the hot pass (ncu: 27 warp-instructions per sample and pass, 11 of them FP64 at half issue rate), so:
-//   * no per-sample range test -- an operand outside rcp_fast's domain (rho = inf, e = inf or 0/0, a denormal
-//     product) surfaces as a NaN / inf in the trip's sums, which the caller tests ONCE per trip and then redoes
-//     the trip with the IEEE divisions;
+//   * no per-sample range test -- an operand at the low end of rcp_fast's domain (0, a denormal product) or an
+//     infinite one (rho = inf, an overflowed product) surfaces as a NaN / inf in the trip's sums, which the caller
+//     tests ONCE per trip and then redoes the trip with the IEEE divisions.  The high end does not: .ftz flushes
+//     1/x to a finite 0 for x in [2^1022, 2^1024), so fp_kernel_f64 tests the largest argument of a pass once
+//     (rcp_fast_in_range) and takes the IEEE path for the whole pass when it is that large;
 //   * STANDARD accumulates sum t^2 and the caller multiplies by (rho_old - rho_new)^2 once per pass
 //     (pi' - pi = t (rho_old - rho_new)): one DMUL per sample less.
 // q2 = sum t^2 (STANDARD) or sum (pi' - pi)^2 (ONLINE).
@@ -469,6 +471,19 @@ __device__ __forceinline__ void trip_sum_only(const double2 (&v)[kFpUnroll], dou
 }
 __device__ __forceinline__ bool finite_f64(double x) {
   return (((unsigned int)__double2hiint(x) >> 20) & 0x7ffu) != 0x7ffu;
+}
+
+// false when some sample of a pass would hand rcp_fast an argument at or above 2^1022, where rcp.approx.ftz.f64 returns 0 (1/x
+// is subnormal and flushed) and the sample would drop out of the sums without a trace.  trip_fast's argument grows with e
+// (rho, rho' >= 0; rounding is monotone), so the largest of a pass is the one at max e; inf and NaN count as out of range.
+// It also bounds trip_sum_only's rho' + e: rho' + e > (rho' + e)(rho + e) needs rho + e < 1, and then rho' + e >= 2^1022
+// needs rho' = inf (rho' = eps / (1 - eps) or avg / (1 - avg) is below 2^54 when finite), which makes the product inf too.
+// emax and rho are the grid's (and the ranks') reduced values, so every block takes the same branch.
+template <int VARIANT>
+__device__ __forceinline__ bool rcp_fast_in_range(double emax, double rho_new, double rho_old) {
+  const double x = (VARIANT == RLVI_FP_STANDARD) ? (rho_new + emax) * (rho_old + emax)
+                                                 : (1.0 + rho_new * emax) * (1.0 + rho_old * emax);
+  return x < 0x1p1022;
 }
 
 // ---- series passes (STANDARD; DESIGN.md section 4, "Series passes") ------------------------------------------------
@@ -897,8 +912,11 @@ __device__ __forceinline__ void build_power_sums(const FpParams<double>& p, FpSh
 // =================================================================================================
 // FP64 kernel: STANDARD and ONLINE
 // =================================================================================================
+// VEC: two CTAs per SM, which the shared-memory budget (kFpCacheSlots, the ring) is sized for.  Left to itself ptxas gave
+// the STANDARD instantiation 174 registers (one CTA per SM, hence another grid and summation order) once the per-pass range
+// test was added; at 128 it spills what it spilled before.
 template <int VARIANT, bool VEC>
-__global__ void __launch_bounds__(kFpThreads) fp_kernel_f64(const FpParams<double> p) {
+__global__ void __launch_bounds__(kFpThreads, VEC ? 2 : 0) fp_kernel_f64(const FpParams<double> p) {
   __shared__ FpShared sh;
   unsigned int round = 0;
   const double n_glob = double(p.n_global);
@@ -995,7 +1013,7 @@ __global__ void __launch_bounds__(kFpThreads) fp_kernel_f64(const FpParams<doubl
           }
         }
       });
-    } else if (VEC) {
+    } else if (VEC && rcp_fast_in_range<VARIANT>(emax, rho_new, rho_old)) {
       // Which trip?  By Cauchy-Schwarz  ||pi' - pi||_2 >= |sum pi' - sum pi| / sqrt(N): when that lower bound is above tol
       // the stop test `err < tol` (rlvi.py:18) is decided WITHOUT the sum of squared differences, and the pass needs
       // half the FP64 instructions.  The bound is predicted from the last two (it decays geometrically: in the
@@ -1018,6 +1036,7 @@ __global__ void __launch_bounds__(kFpThreads) fp_kernel_f64(const FpParams<doubl
         else stream_pass_vec<VARIANT, false>(e, ec, p.n, rho_new, rho_old, s1, s2);
       }
     } else {
+      // the scalar path, and a pass of the aligned one that is out of rcp_fast's range (leaves the ring's armed copies alone)
       for_each_chunk<double, VEC>(p.n, [&](int64_t c, int) {
         const int64_t i = c * W;
         double ev[W];
