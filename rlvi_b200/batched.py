@@ -22,7 +22,7 @@ drop-in's pivot test (rank-deficient or ill-conditioned designs, n_b < d) are re
 rlvi_b200.rlvi.linear_regression, whose eigen-decomposition route gives the minimum-norm answer.  Logistic problems take
 at most `rlvi_b200.ops.batched_logistic_max_rows(d)` rows (at least 1024 at every d <= 63, 2000 at d <= 8); those whose
 Newton solve does not converge in 60 steps, or whose MM majoriser fails the pivot test, are re-solved one by one with
-rlvi_b200.rlvi.logistic_regression (an exception it raises names the problem).  There is no CPU fallback.
+rlvi_b200.rlvi.logistic_regression.  An exception a re-solve raises names the problem.  There is no CPU fallback.
 """
 from __future__ import annotations
 
@@ -115,23 +115,36 @@ def mean(samples, maxiter=100, tol=1e-3):
     return theta if is_t else theta.cpu().numpy()
 
 
-def linear_regression(X, y, maxiter=100, tol=1e-3):
-    """rlvi.py:68-89 on every problem: X [B, n, d] or a list of [n_b, d], y [B, n] or a list of [n_b] -> theta [B, d]."""
+def _fit_xy(fn, X, y, fit, cap, d_max, **dropin_kw):
+    """The body of linear_regression and logistic_regression: packs X and y, checks them against `cap(d)`, runs
+    `fit(X, y, offsets)` (one batched call) and re-fits the HOST_SOLVE problems with rlvi.<fn>(..., **dropin_kw); an
+    exception the drop-in raises names the problem."""
     fx, lengths, _, is_t = _gather(X, 2, "X")
     fy, ly, _, _ = _gather(y, 1, "y")
     if not np.array_equal(lengths, ly):
         raise ValueError("X and y must describe the same problems with the same numbers of rows")
     d = fx.shape[1]
-    _check_cap(lengths, d, "linear_regression")
+    _check_cap(lengths, d, fn, cap(d), d_max)
     Xd, yd = _to_device(fx, fy.to(fx.device) if is_t else fy)
     off = _offsets(lengths)
-    theta, _, status = ops.batched_em(ops.BATCHED_LINREG, Xd, yd, off, tol=tol, maxiter=maxiter)
+    theta, _, status = fit(Xd, yd, off)
     for b in np.flatnonzero(status.cpu().numpy() == HOST_SOLVE):
         s, e = int(off[b]), int(off[b + 1])
         # fresh copies: the drop-in's kernels choose their load path by alignment, and a copy gives the bits of the
         # problem fitted on its own
-        theta[b] = _rlvi.linear_regression(Xd[s:e].clone(), yd[s:e].clone(), maxiter=maxiter, tol=tol)
+        try:
+            theta[b] = getattr(_rlvi, fn)(Xd[s:e].clone(), yd[s:e].clone(), **dropin_kw)
+        except Exception as exc:
+            exc.args = (f"batched.{fn}, problem {b}: {exc.args[0] if exc.args else exc}",) + exc.args[1:]
+            raise
     return theta if is_t else theta.cpu().numpy()
+
+
+def linear_regression(X, y, maxiter=100, tol=1e-3):
+    """rlvi.py:68-89 on every problem: X [B, n, d] or a list of [n_b, d], y [B, n] or a list of [n_b] -> theta [B, d]."""
+    return _fit_xy("linear_regression", X, y,
+                   lambda Xd, yd, off: ops.batched_em(ops.BATCHED_LINREG, Xd, yd, off, tol=tol, maxiter=maxiter),
+                   ops.batched_max_rows, 64, maxiter=maxiter, tol=tol)
 
 
 def logistic_regression(X, y, maxiter=100, tol=1e-2, mstep="sklearn"):
@@ -139,20 +152,7 @@ def logistic_regression(X, y, maxiter=100, tol=1e-2, mstep="sklearn"):
     (intercept first).  `mstep` as in rlvi.logistic_regression: "sklearn" (the reference's default) or "mm"."""
     if mstep not in _LOGREG_MSTEP:
         raise ValueError(f'mstep must be "sklearn" or "mm" (got {mstep!r})')
-    fx, lengths, _, is_t = _gather(X, 2, "X")
-    fy, ly, _, _ = _gather(y, 1, "y")
-    if not np.array_equal(lengths, ly):
-        raise ValueError("X and y must describe the same problems with the same numbers of rows")
-    d = fx.shape[1]
-    _check_cap(lengths, d, "logistic_regression", ops.batched_logistic_max_rows(d), 63)
-    Xd, yd = _to_device(fx, fy.to(fx.device) if is_t else fy)
-    off = _offsets(lengths)
-    theta, _, status = ops.batched_logistic(Xd, yd, off, mstep=_LOGREG_MSTEP[mstep], tol=tol, maxiter=maxiter)
-    for b in np.flatnonzero(status.cpu().numpy() == HOST_SOLVE):
-        s, e = int(off[b]), int(off[b + 1])
-        try:     # fresh copies, as in linear_regression
-            theta[b] = _rlvi.logistic_regression(Xd[s:e].clone(), yd[s:e].clone(), maxiter=maxiter, tol=tol, mstep=mstep)
-        except Exception as exc:
-            exc.args = (f"batched.logistic_regression, problem {b}: {exc.args[0] if exc.args else exc}",) + exc.args[1:]
-            raise
-    return theta if is_t else theta.cpu().numpy()
+    return _fit_xy("logistic_regression", X, y,
+                   lambda Xd, yd, off: ops.batched_logistic(Xd, yd, off, mstep=_LOGREG_MSTEP[mstep], tol=tol,
+                                                            maxiter=maxiter),
+                   ops.batched_logistic_max_rows, 63, maxiter=maxiter, tol=tol, mstep=mstep)

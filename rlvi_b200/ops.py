@@ -408,40 +408,48 @@ def batched_results(results):
     return results.cpu().numpy().reshape(-1).view(_RESULT_DTYPE).copy()
 
 
+def _batched_xy(entry, max_rows, X, y, offsets, code, D_extra, d_max, d_what, tol, maxiter):
+    """The body of batched_em and batched_logistic: checks X [rows, d] (1 <= d <= d_max) and y [rows] (when given),
+    uploads the offsets against the cap `max_rows` at d, allocates (theta [nprob, d + D_extra], iters, status) and calls
+    the C entry point `entry` with model / mstep `code`."""
+    dev = _dev(X)
+    f64 = torch.float64
+    _chk(X, f64, "X")
+    if X.dim() != 2:
+        raise ValueError("X must be [rows, d]")
+    rows, d = X.shape
+    if not 1 <= d <= d_max:
+        raise ValueError(f"{d_what} 1 <= d <= {d_max} (got d = {d})")
+    if y is not None:
+        _len(_chk(y, f64, "y"), rows, "y")
+    _same_device(X, y)
+    if int(maxiter) < 0:
+        raise ValueError("maxiter must be >= 0")
+    ctx = _ctx(dev)
+    offs, nprob = _batched_offsets(offsets, rows, getattr(ctx.lib, max_rows)(d), X)
+    theta = torch.empty(nprob, d + D_extra, dtype=f64, device=X.device)
+    iters = torch.empty(nprob, dtype=torch.int32, device=X.device)
+    status = torch.empty(nprob, dtype=torch.int32, device=X.device)
+    rc = getattr(ctx.lib, entry)(ctx.handle, int(code), _p(X), _p(y), _p(offs), nprob, rows, d, float(tol), int(maxiter),
+                                 _p(theta), _p(iters), _p(status), _stream(dev))
+    _lib.check(rc, entry)
+    return theta, iters, status
+
+
 def batched_em(model, X, y, offsets, *, tol=1e-3, maxiter=100):
     """rlvi_batched_em_f64: the EM loop of rlvi.mean (model BATCHED_MEAN, y None) or rlvi.linear_regression
     (BATCHED_LINREG) on every segment of the rows of X [rows, d] (and y [rows]).  `offsets` is a host integer array.
     Returns device tensors (theta [nprob, d] float64, iters [nprob] int32, status [nprob] int32); status 0 = stop test met,
     1 = maxiter reached, 2 = the normal equations failed the pivot test: theta is NaN, solve that problem with
     rlvi.linear_regression."""
-    dev = _dev(X)
-    f64 = torch.float64
-    _chk(X, f64, "X")
     if model not in (BATCHED_MEAN, BATCHED_LINREG):
         raise ValueError("model must be BATCHED_MEAN or BATCHED_LINREG")
-    if X.dim() != 2:
-        raise ValueError("X must be [rows, d]")
-    rows, d = X.shape
-    if not 1 <= d <= 64:
-        raise ValueError(f"batched calls support 1 <= d <= 64 (got d = {d})")
     if model == BATCHED_MEAN and y is not None:
         raise ValueError("the mean model takes no y")
-    if model == BATCHED_LINREG:
-        if y is None:
-            raise ValueError("linear regression needs y")
-        _len(_chk(y, f64, "y"), rows, "y")
-    _same_device(X, y)
-    if int(maxiter) < 0:
-        raise ValueError("maxiter must be >= 0")
-    ctx = _ctx(dev)
-    offs, nprob = _batched_offsets(offsets, rows, ctx.lib.rlvi_batched_max_rows(d), X)
-    theta = torch.empty(nprob, d, dtype=f64, device=X.device)
-    iters = torch.empty(nprob, dtype=torch.int32, device=X.device)
-    status = torch.empty(nprob, dtype=torch.int32, device=X.device)
-    rc = ctx.lib.rlvi_batched_em_f64(ctx.handle, int(model), _p(X), _p(y), _p(offs), nprob, rows, d, float(tol),
-                                     int(maxiter), _p(theta), _p(iters), _p(status), _stream(dev))
-    _lib.check(rc, "rlvi_batched_em_f64")
-    return theta, iters, status
+    if model == BATCHED_LINREG and y is None:
+        raise ValueError("linear regression needs y")
+    return _batched_xy("rlvi_batched_em_f64", "rlvi_batched_max_rows", X, y, offsets, model, 0, 64,
+                       "batched calls support", tol, maxiter)
 
 
 def batched_logistic_max_rows(d) -> int:
@@ -455,31 +463,12 @@ def batched_logistic(X, y, offsets, *, mstep, tol=1e-2, maxiter=100):
     (BATCHED_LOGREG_MM).  `offsets` is a host integer array.  Returns device tensors (theta [nprob, d + 1] float64,
     intercept first; iters [nprob] int32; status [nprob] int32): status 0 = stop test met, 1 = maxiter reached, 2 = theta
     is NaN, solve that problem with rlvi.logistic_regression."""
-    dev = _dev(X)
-    f64 = torch.float64
-    _chk(X, f64, "X")
     if mstep not in (BATCHED_LOGREG_NEWTON, BATCHED_LOGREG_MM):
         raise ValueError("mstep must be BATCHED_LOGREG_NEWTON or BATCHED_LOGREG_MM")
-    if X.dim() != 2:
-        raise ValueError("X must be [rows, d]")
-    rows, d = X.shape
-    if not 1 <= d <= 63:
-        raise ValueError(f"batched logistic regression supports 1 <= d <= 63 (got d = {d})")
     if y is None:
         raise ValueError("logistic regression needs y")
-    _len(_chk(y, f64, "y"), rows, "y")
-    _same_device(X, y)
-    if int(maxiter) < 0:
-        raise ValueError("maxiter must be >= 0")
-    ctx = _ctx(dev)
-    offs, nprob = _batched_offsets(offsets, rows, ctx.lib.rlvi_batched_logistic_max_rows(d), X)
-    theta = torch.empty(nprob, d + 1, dtype=f64, device=X.device)
-    iters = torch.empty(nprob, dtype=torch.int32, device=X.device)
-    status = torch.empty(nprob, dtype=torch.int32, device=X.device)
-    rc = ctx.lib.rlvi_batched_logistic_f64(ctx.handle, int(mstep), _p(X), _p(y), _p(offs), nprob, rows, d, float(tol),
-                                           int(maxiter), _p(theta), _p(iters), _p(status), _stream(dev))
-    _lib.check(rc, "rlvi_batched_logistic_f64")
-    return theta, iters, status
+    return _batched_xy("rlvi_batched_logistic_f64", "rlvi_batched_logistic_max_rows", X, y, offsets, mstep, 1, 63,
+                       "batched logistic regression supports", tol, maxiter)
 
 
 def sever_pass(X, u, op, scalar, *, a=None, b=None, active=None, out0=None, out1=None, out2=None):
