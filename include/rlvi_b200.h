@@ -207,10 +207,18 @@ int rlvi_weighted_moments_centered_f64(rlvi_ctx* ctx, const double* X, const dou
  * X is float32 [n][d] row-major; every per-sample vector (y, weights, losses, e) and every statistic stays FP64.
  * The Gram contraction runs on the 5th-generation tensor cores (tcgen05.mma kind::tf32, accumulators in TMEM):
  *   RLVI_TF32X3  three products per term (hi*hi + lo*hi + hi*lo; z = hi + lo with hi the TF32 rounding) with short FP32
- *                accumulation chains flushed into FP64: the statistics agree with an FP64 evaluation on the same float32
- *                samples to ~1e-6 (the 1e-5 FP32 tolerance of BASELINE.json's north_star); default.  On the CTA-pair
- *                kernel (d > 128) the two correction products run as BF16 (kind::f16), which keeps that accuracy at two
- *                thirds of the tensor time; RLVI_TF32_PURE3=1 in the environment keeps all three in TF32;
+ *                accumulation chains flushed into FP64; default.  Against an FP64 evaluation on the same float32 samples,
+ *                entry by entry: |G - G_ref| <= 1e-5 B with B = |X|^T diag(w) |X|, |S1 - S1_ref| <= 1e-5 |X|^T weights,
+ *                |Sy - Sy_ref| <= 1e-5 |X|^T |w y| (the 1e-5 FP32 tolerance of BASELINE.json's north_star; measured on
+ *                a B200 at 1000 W: <= 7e-7 B for d <= 128, <= 2.8e-6 B for d > 128, 2.3e-6 B with 32 Ki-row FP32
+ *                register sums of all-positive data).  Supported range: every scaled sample z = s_i x_ij, s_i =
+ *                (pi_i / 2^e)^(power / 2) with 2^e the even power of two at or above max pi, is 0 or has
+ *                2^-60 <= |z| < 2^56.  Below it the products leave the FP32 normal range and lose their corrections
+ *                (measured: 1.4e-6 B at 2^-66, 2.6e-5 B at 2^-68, 4e-4 B at 2^-70); from 2^56 on, a 32 Ki-row FP32
+ *                sum can overflow (non-finite G measured at 2^61 with 32 rows per CTA).  Rows outside the range, e.g.
+ *                weights far below max pi, lose at most their own share of B.  On the CTA-pair kernel (d > 128) the two
+ *                correction products run as BF16 (kind::f16), which keeps that accuracy at two thirds of the tensor
+ *                time; RLVI_TF32_PURE3=1 in the environment keeps all three in TF32;
  *   RLVI_TF32X1  one TF32 product per term (operands rounded to 11 bits, zero-mean error): 3x fewer tensor-core
  *                flops, ~1e-3 / sqrt(rows) relative accuracy.
  * Same output layout as rlvi_weighted_moments_f64.  Replaces utils.py:82-84 (power = 2), rlvi.py:70-71,79-80 and

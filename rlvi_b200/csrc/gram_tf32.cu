@@ -40,8 +40,12 @@
 // SURVEY.md H1) stays inside the FP32 range; the statistics are scaled back exactly.
 //
 // Accuracy: 3xTF32 keeps ~2^-21 per product, the three-level accumulation keeps the sums at FP32 level over
-// any N -> statistics agree with the FP64 oracle on the same float32 samples to ~1e-6 (tested at 1e-5);
-// single-pass TF32 (precision = RLVI_TF32X1) rounds operands to 11 bits (zero-mean error): ~1e-3/sqrt(rows).
+// any N -> entry by entry, |G - G_ref| <= 1e-5 B with B = |X|^T diag(w) |X| against FP64 on the same float32 samples
+// (measured <= 7e-7 B here, <= 2.8e-6 B on the CTA pairs, on inputs whose TF32 remainders all have one sign; B200,
+// 1000 W), for scaled samples 2^-60 <= |z| < 2^56 (or 0): below, the products leave the FP32 normal range and lose their
+// corrections first; from 2^56 on, a 32 Ki-row register sum of z^2 can overflow.  tests/test_gpu_fp32_mode.py checks
+// both ends.  Single-pass TF32 (precision = RLVI_TF32X1) rounds operands to 11 bits: ~1e-3/sqrt(rows) on zero-mean
+// remainders, up to ~5e-4 B when they share a sign.
 #include "tf32.cuh"
 
 namespace {
@@ -465,6 +469,8 @@ __global__ void __launch_bounds__(256) add_f64_kernel(double* __restrict__ dst, 
 static int moments_f32_via_f64(rlvi_ctx* ctx, const float* X, const double* y, const double* weights, int64_t n, int d,
                                int power, int want_gram, double* out, cudaStream_t st) {
   const int nm = rlvi_moments_out_doubles(d);
+  const int nsum = want_gram ? nm : 2 + 2 * d;             // want_gram == 0 leaves G in `out` untouched
+
   int64_t chunk = (int64_t(64) << 20) / (int64_t(d) * 8);   // 64 MiB of converted rows at a time
   if (chunk < 64) chunk = 64;
   if (chunk > n) chunk = n;
@@ -487,10 +493,10 @@ static int moments_f32_via_f64(rlvi_ctx* ctx, const float* X, const double* y, c
     const int64_t rows = (n - r0 < chunk) ? (n - r0) : chunk;
     f32_to_f64_kernel<<<ctx->sm_count * 4, 256, 0, st>>>(X + r0 * d, xd, rows * d);
     RLVI_LAUNCH_CHECK(ctx);
-    RLVI_CUDA(cudaMemsetAsync(tmp, 0, size_t(nm) * 8, st));
+    RLVI_CUDA(cudaMemsetAsync(tmp, 0, size_t(nsum) * 8, st));
     const int rc = rlvi_weighted_moments_f64(ctx, xd, y ? y + r0 : nullptr, weights + r0, rows, d, power, want_gram, tmp, st);
     if (rc != RLVI_OK) return rc;
-    add_f64_kernel<<<(nm + 255) / 256, 256, 0, st>>>(out, tmp, nm, first ? 1 : 0);
+    add_f64_kernel<<<(nsum + 255) / 256, 256, 0, st>>>(out, tmp, nsum, first ? 1 : 0);
     RLVI_LAUNCH_CHECK(ctx);
     first = false;
   }

@@ -1,12 +1,15 @@
 """FP32-stored-X mode (SURVEY.md section 8d, BASELINE.json config 3): rlvi_weighted_moments_f32 (tcgen05 TF32 Gram)
 and rlvi_loss_f32 against the NumPy oracle evaluated in FP64 on the SAME float32 samples.  Tolerance: north_star's
-1e-5 for FP32 quantities (3xTF32 is ~1e-6; single-pass TF32 is bounded at its own, looser, level)."""
+1e-5 for FP32 quantities, entry by entry: |G - G_ref| <= 1e-5 |X|^T diag(w) |X| (tests/tf32_bounds.py); single-pass TF32 is
+bounded at its own, looser, level.  The tests on `biased_inputs` make a missing correction product fail that check on
+every entry, which zero-mean rounding on random samples hides."""
 import os
 
 import numpy as np
 import pytest
 import torch
 
+import tf32_bounds as tb
 from oracle import rlvi_np
 
 pytestmark = pytest.mark.gpu
@@ -49,14 +52,7 @@ def test_moments_f32_tf32x3_matches_oracle(n, d, power, with_y):
     w = rng.random(n) ** 4
     y = rng.normal(size=n) if with_y else None
     m = gpu_moments(X, w, y, power)
-    r = oracle_moments(X, w, y, power)
-    assert rel(m["G"], r["G"]) < TOL32
-    assert rel(m["S1"], r["S1"]) < TOL32
-    assert abs(m["S0"] - r["S0"]) < 1e-9 * r["S0"]
-    assert np.array_equal(m["G"], m["G"].T)                      # exact symmetry
-    if with_y:
-        assert rel(m["Sy"], r["Sy"]) < TOL32
-        assert abs(m["Swy"] - r["Swy"]) < 1e-9 * abs(r["Swy"]) + 1e-12
+    tb.check_moments(m, tb.reference(X, w, y, power), TOL32, with_y)      # includes exact symmetry
 
 
 @pytest.mark.parametrize("scale", [1e-7, 1e-20, 1e-150, 1e40])
@@ -69,10 +65,7 @@ def test_moments_f32_collapse_regime_weights(scale):
     w = scale * rng.random(n) ** 3
     y = rng.normal(size=n)
     for power in (1, 2):
-        m = gpu_moments(X, w, y, power)
-        r = oracle_moments(X, w, y, power)
-        assert rel(m["G"], r["G"]) < TOL32 and rel(m["S1"], r["S1"]) < TOL32 and rel(m["Sy"], r["Sy"]) < TOL32
-        assert abs(m["S0"] - r["S0"]) < 1e-9 * r["S0"]
+        tb.check_moments(gpu_moments(X, w, y, power), tb.reference(X, w, y, power), TOL32, True)
 
 
 def test_moments_f32_fallback_shapes():
@@ -81,9 +74,7 @@ def test_moments_f32_fallback_shapes():
     for n, d in ((500, 10), (2000, 130), (300, 600)):
         X = rng.normal(size=(n, d)).astype(np.float32)
         w = rng.random(n)
-        m = gpu_moments(X, w, None, 1)
-        r = oracle_moments(X, w, None, 1)
-        assert rel(m["G"], r["G"]) < 1e-12 and rel(m["S1"], r["S1"]) < 1e-12
+        tb.check_moments(gpu_moments(X, w, None, 1), tb.reference(X, w, None, 1), tb.TAU_F64, False)
     from rlvi_b200 import ops
     dev = torch.device("cuda", 0)
     X = rng.normal(size=(1001, 64)).astype(np.float32)
@@ -91,8 +82,7 @@ def test_moments_f32_fallback_shapes():
     Xu = base[1:].view(1001, 64)                                 # 4-byte aligned only
     w = rng.random(1001)
     out = ops.weighted_moments(Xu, torch.from_numpy(w).to(dev))
-    G = ops.split_moments(out, 64)["G"].cpu().numpy()
-    assert rel(G, oracle_moments(X, w, None, 1)["G"]) < 1e-12
+    tb.check_moments(ops.split_moments(out, 64), tb.reference(X, w, None, 1), tb.TAU_F64, False)
 
 
 def test_moments_f32_single_pass_tf32_is_bounded():
@@ -115,16 +105,13 @@ def test_moments_f32_correction_modes_agree(n, d, power, with_y, monkeypatch):
     X[:, :3] += 2.0
     w = rng.random(n) ** 3
     y = rng.normal(size=n) if with_y else None
-    r = oracle_moments(X, w, y, power)
+    r = tb.reference(X, w, y, power)
     monkeypatch.delenv("RLVI_TF32_PURE3", raising=False)
     mixed = gpu_moments(X, w, y, power)
     monkeypatch.setenv("RLVI_TF32_PURE3", "1")
     pure = gpu_moments(X, w, y, power)
     for m in (mixed, pure):
-        assert rel(m["G"], r["G"]) < TOL32
-        assert rel(m["S1"], r["S1"]) < TOL32
-        if with_y:
-            assert rel(m["Sy"], r["Sy"]) < TOL32
+        tb.check_moments(m, r, TOL32, with_y)
     assert rel(mixed["G"], pure["G"]) < 3e-6
     # column sums do not go through the tensor core; the two modes split the row tiles over the pair types differently,
     # so their FP32 partial sums group differently
@@ -150,10 +137,144 @@ def test_moments_f32_large_n_d512_against_oracle():
     X = rng.standard_normal(size=(n, d), dtype=np.float32)
     w = rng.random(n) ** 2
     m = gpu_moments(X, w, None, 2)
-    X64 = X.astype(np.float64)
-    Gr = (X64 * (w * w)[:, None]).T @ X64
-    assert rel(m["G"], Gr) < TOL32
-    assert rel(m["S1"], X64.T @ w) < TOL32
+    tb.check_moments(m, tb.reference(torch.from_numpy(X).cuda(), torch.from_numpy(w), None, 2), TOL32, False)
+
+
+# ---- biased inputs (tests/tf32_bounds.py): every TF32 remainder of the same sign, so a missing product is a bias ----
+SINGLE_CTA_D = (4, 36, 64, 100, 128)             # d % 32 != 0: four 2-D boxes; d % 32 == 0: one 3-D box
+PAIR_D = (132, 256, 260, 384, 388, 448, 512)     # one pair type (d <= 256), three types; 257..384 run as 512
+DEV = "cuda"
+
+
+def dev_moments(X, w, y=None, power=1, precision=0, want_gram=True, out=None):
+    from rlvi_b200 import ops
+    o = ops.weighted_moments(X, w, y=y, power=power, precision=precision, want_gram=want_gram, out=out)
+    return ops.split_moments(o, X.shape[1])
+
+
+def report(what, q):
+    print(f"[tf32] {what}: max |G - G_ref| / B = {q:.3g}")
+
+
+@pytest.mark.parametrize("power,with_y", [(1, False), (1, True), (2, False), (2, True)])
+@pytest.mark.parametrize("d", SINGLE_CTA_D + PAIR_D)
+def test_moments_f32_biased_inputs_every_route(d, power, with_y, monkeypatch):
+    """Both kernels, both powers, with and without y, BF16 and TF32 corrections (RLVI_TF32_PURE3=1, pair kernel only):
+    entry-wise within 1e-5 B.  RLVI_TF32X1 on the same inputs -- the kernel without its corrections -- must miss by
+    more than 1e-4 B on every diagonal entry, which shows the check sees a missing correction."""
+    n = 3000 + 7 * d
+    X, w = tb.biased_inputs(n, d, seed=d * 4 + power * 2 + with_y, device=DEV)
+    y = torch.randn(n, dtype=torch.float64, device=DEV) if with_y else None
+    r = tb.reference(X, w, y, power)
+    modes = ("0", "1") if d > 128 else ("0",)
+    for pure in modes:
+        monkeypatch.setenv("RLVI_TF32_PURE3", pure)
+        q = tb.check_moments(dev_moments(X, w, y, power), r, TOL32, with_y)
+        report(f"d={d} p={power} y={with_y} {'pure TF32' if pure == '1' else 'default'} corrections", q)
+    monkeypatch.delenv("RLVI_TF32_PURE3")
+    G1 = dev_moments(X, w, y, power, precision=1)["G"].cpu().numpy()
+    q1 = np.abs(G1 - r["G"]) / r["BG"]
+    report(f"d={d} p={power} y={with_y} TF32X1", float(q1.max()))
+    assert np.diag(q1).min() > 1e-4
+
+
+@pytest.mark.parametrize("d", (64, 256, 512))
+@pytest.mark.parametrize("n", (1, 15, 16, 17, 127, 128, 129))
+def test_moments_f32_row_count_edges(n, d):
+    """Partial and single tiles, fewer tiles than CTAs and fewer than the pairs of one pair type."""
+    X, w = tb.biased_inputs(n, d, seed=n * 1000 + d, device=DEV)
+    y = torch.randn(n, dtype=torch.float64, device=DEV)
+    power = 1 + n % 2
+    tb.check_moments(dev_moments(X, w, y, power), tb.reference(X, w, y, power), TOL32, True)
+
+
+@pytest.mark.parametrize("d,power", [(128, 2), (256, 1), (512, 1)])
+def test_moments_f32_register_flush_depth(d, power):
+    """Every slot runs at least one full 32 Ki-row FP32 register accumulation (chunks_per_flush = 256 chunks of 128
+    rows) on all-positive data: the worst case for one-signed FP32 rounding.  The single-CTA kernel has one slot per SM;
+    the CTA-pair kernel has at most SMs / 2 pairs of one type, so these n reach a full flush in every slot whatever the
+    plan picks."""
+    sms = torch.cuda.get_device_properties(0).multi_processor_count
+    slots = sms if d <= 128 else sms // 2
+    n = slots * 32768 + 16 * slots + 5
+    X, w = tb.biased_inputs(n, d, seed=d, device=DEV)
+    y = torch.randn(n, dtype=torch.float64, device=DEV)
+    q = tb.check_moments(dev_moments(X, w, y, power), tb.reference(X, w, y, power), TOL32, True)
+    report(f"flush depth n={n} d={d} p={power} ({torch.cuda.get_device_name(0)})", q)
+
+
+@pytest.mark.parametrize("power", (1, 2))
+@pytest.mark.parametrize("d", (64, 256, 512))
+def test_moments_f32_weight_range(d, power):
+    """Weights from 1 down to 1e-300 in one call, with exact zeros and subnormal doubles: the kernels normalise by a
+    power of two and the rows whose scaled weight leaves the FP32 range contribute below the bound."""
+    n = 6000
+    X, _ = tb.biased_inputs(n, d, seed=7 + d, device=DEV)
+    g = torch.Generator(device=DEV).manual_seed(d + power)
+    w = torch.pow(10.0, -300.0 * torch.rand(n, dtype=torch.float64, device=DEV, generator=g))
+    w[::97] = 0.0
+    w[1:4] = torch.tensor([5e-324, 1e-310, 2.2e-308], dtype=torch.float64)
+    w[4] = 1.0
+    y = torch.randn(n, dtype=torch.float64, device=DEV, generator=g)
+    tb.check_moments(dev_moments(X, w, y, power), tb.reference(X, w, y, power), TOL32, True)
+
+
+@pytest.mark.parametrize("power", (1, 2))
+@pytest.mark.parametrize("d", (64, 256, 512))
+def test_moments_f32_column_magnitudes(d, power):
+    """Columns scaled from 2^-20 to 2^20 in one X: every entry meets its own bound."""
+    X, w = tb.biased_inputs(5000, d, seed=11 + d, device=DEV, col_exp=np.linspace(-20, 20, d).round().astype(int))
+    y = torch.randn(5000, dtype=torch.float64, device=DEV)
+    tb.check_moments(dev_moments(X, w, y, power), tb.reference(X, w, y, power), TOL32, True)
+
+
+# The supported range of the scaled samples z = s x (include/rlvi_b200.h, RLVI_TF32X3): 2^Z_LO <= |z| < 2^Z_HI.  Measured
+# on a B200: still within the bound at 2^-66, 2.6e-5 B at 2^-68; non-finite at 2^61 (32 rows per CTA).
+Z_LO, Z_HI = -60, 56
+
+
+@pytest.mark.parametrize("end", ("low", "high"))
+@pytest.mark.parametrize("power", (1, 2))
+@pytest.mark.parametrize("d", (64, 256))
+def test_moments_f32_supported_range_ends(d, power, end):
+    """All samples at one end of the supported range of |s x|: unit weights give s = 1/2 (power 1) or 1/4 (power 2)
+    after the kernels' normalisation, so x = 2^(E + 1) or 2^(E + 2) puts z in [2^E, 2^(E + 1))."""
+    e = (Z_LO if end == "low" else Z_HI - 1) + power
+    X, w = tb.biased_inputs(4096, d, seed=d + power, device=DEV, col_exp=[e] * d, max_k=0, zero_frac=0.0)
+    q = tb.check_moments(dev_moments(X, w, None, power), tb.reference(X, w, None, power), TOL32, False)
+    report(f"range end {end}: |z| in [2^{e - power}, 2^{e - power + 1}) d={d} p={power}", q)
+
+
+@pytest.mark.parametrize("n,d", [(5000, 64), (5000, 256), (5000, 512), (1_700_000, 10)])
+def test_moments_f32_want_gram_0_leaves_G_untouched(n, d):
+    """want_gram = 0 on the three routes (single CTA, CTA pairs, FP64 conversion over three chunks): the G region of
+    `out` comes back bit-identical, the vectors within their bounds."""
+    X, w = tb.biased_inputs(n, d, seed=n + d, device=DEV)
+    y = torch.randn(n, dtype=torch.float64, device=DEV)
+    out = torch.randn(2 + 2 * d + d * d, dtype=torch.float64, device=DEV) * 1e300      # sentinel
+    g0 = out[2 + 2 * d:].clone()
+    m = dev_moments(X, w, y, 2, want_gram=False, out=out)
+    assert torch.equal(out[2 + 2 * d:].view(torch.int64), g0.view(torch.int64))
+    tau = tb.TAU_F64 if d % 4 else TOL32
+    tb.check_moments(m, tb.reference(X, w, y, 2), tau, True, want_gram=False)
+
+
+@pytest.mark.parametrize("power", (1, 2))
+@pytest.mark.parametrize("n,d,aligned", [(2_100_000, 10, True), (40000, 516, True), (20561, 1020, True),
+                                         (300_001, 64, False)])
+def test_moments_f32_fp64_route_chunks(n, d, aligned, power):
+    """The FP64 conversion route (d % 4 != 0, d > 512, unaligned X) over three chunks of 64 MiB / (8 d) rows: the
+    chunk loop, its y / weights offsets and the accumulation of the chunk results, entry-wise at FP64 level."""
+    g = torch.Generator(device=DEV).manual_seed(n + power)
+    X = torch.randn((n, d), dtype=torch.float32, device=DEV, generator=g) + 0.5
+    if not aligned:
+        base = torch.zeros(n * d + 1, dtype=torch.float32, device=DEV)
+        base[1:].copy_(X.view(-1))
+        X = base[1:].view(n, d)                                       # 4-byte aligned only
+    assert n > 2 * (64 << 20) // (8 * d)
+    w = torch.rand(n, dtype=torch.float64, device=DEV, generator=g) ** 2
+    y = torch.randn(n, dtype=torch.float64, device=DEV, generator=g)
+    tb.check_moments(dev_moments(X, w, y, power), tb.reference(X, w, y, power), tb.TAU_F64, True)
 
 
 @pytest.mark.parametrize("kind_name", ["LOGISTIC_CE", "SOFTPLUS", "SQRES", "SQDIST", "PCA"])
